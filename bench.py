@@ -1,8 +1,12 @@
 #!/usr/bin/env python
 """bench.py -- SGC-LL train throughput (graphs/s) on N B200s, one JSON line on rank 0.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+The result line goes to stdout without the per-kernel tables and descriptions; the full record follows on stderr as
+one JSON line.  K is the number of timed steps of `value`.  --dump-outputs DIR writes what the last of them computed
+(loss, gradients, parameters after Adam) as DIR/*.npy.
 
 Headline workload (BASELINE.json configs[1], SURVEY.md section 8d "C2"): ToxCast-shape synthetic molecules,
 B = 1024 graphs per GPU (weak scaling), Nmax = 132, 75 atom features, 617 tasks, K = 3, through the SimpleAGCN
@@ -367,7 +371,8 @@ class Runner(object):
         return float(t)
 
     def resident_step(self):
-        return self.model.step(self.Xd, self.Ld, self.batch, self.tg_d, self.w_d)
+        self.loss = self.model.step(self.Xd, self.Ld, self.batch, self.tg_d, self.w_d)   # (a replayed graph rewrites it)
+        return self.loss
 
     def timed(self, fn, steps, warmup):
         torch = self.torch
@@ -745,6 +750,36 @@ def layer3_roofline(r, peaks, tf32_peak):
             "kernels_of_the_layer_forward": rows, "layer": layer_row}
 
 
+def dump_outputs(r, out_dir):
+    """What the last timed step hands its caller: the loss, every parameter's gradient and the parameters after Adam
+    (flat, in the model's parameter order), as float32 DIR/{loss,grads,params}.npy.  The inputs, the initial
+    parameters and the number of steps run before are fixed by the arguments, so two builds can be compared."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("loss", r.loss), ("grads", r.model.flat_grad), ("params", r.model.flat_params.flat)):
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
+# what only describes or breaks down a number: left out of the result line, kept in the full record on stderr
+DETAIL_KEYS = {"kernels", "kernels_of_the_layer_forward", "layer", "pipeline", "note", "how", "sample",
+               "traffic_source", "peak_source"}
+
+
+def result_line(rec):
+    """The record without its detail and with each secondary config cut to its rates, small enough (~4 KB) for a
+    reader that keeps only the end of the output to parse."""
+    def strip(o):
+        return {k: strip(v) for k, v in o.items() if k not in DETAIL_KEYS} if isinstance(o, dict) else o
+
+    def rates(res):
+        out = {k: res[k] for k in ("value", "ms_per_step", "error") if k in res}
+        out.update({k: res[k]["value"] for k in ("e2e", "cpu_baseline") if k in res})
+        if "roofline" in res:
+            out["roofline_frac"] = res["roofline"]["frac"]
+        return out
+    return strip(dict(rec, configs={k: rates(v) for k, v in rec["configs"].items()}))
+
+
 def measure_workload(cfg, dev, rank, world, args, peaks, tf32_peak, full):
     """graphs/s (resident, CUDA-graph replay), e2e (host buffers), kernel table, dominant-kernel roofline for one
     workload.  full=True adds the secondary e2e modes and the paper-semantics co-headline (the C2 headline)."""
@@ -771,6 +806,8 @@ def measure_workload(cfg, dev, rank, world, args, peaks, tf32_peak, full):
         sampler.start()
         sampler.wait_first(2.0)
     ms_step = r.timed(step_fn, steps, warmup)
+    if full and rank == 0 and args.dump_outputs:
+        dump_outputs(r, args.dump_outputs)
     if full:
         # the timed region is a few tens of milliseconds, shorter than nvidia-smi's sampling period: every rank keeps
         # the SAME step running (untimed, same count everywhere) for ~0.7 s so the clocks line describes this load
@@ -949,8 +986,10 @@ def run_ours(args):
                 "kernels": main.get("kernels"), "peaks": dict(peaks, **measured),
                 "cpu_baseline": {k: cpu_main.get(k) for k in ("value", "unit", "cores", "kind", "sample")},
                 "cpu_vectorised": cpu_vec, "configs": others}
-        print(json.dumps(line))
+        print(json.dumps(result_line(line)))
         sys.stdout.flush()
+        sys.stderr.write(json.dumps(line) + "\n")
+        sys.stderr.flush()
     mark("done")
     if world > 1:
         # every CUDA graph that captured a collective is released (Runner.release) before the process group goes;
@@ -981,6 +1020,8 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true", help="skip the CPU legs (quick experiments)")
     ap.add_argument("--no-overlap", action="store_true", help="N > 1: one all-reduce after backward instead of buckets")
     ap.add_argument("--ref-graphs", type=int, default=0, help="graphs per step of the reference arm (default: the batch)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the loss, gradients and parameters of the last timed step as DIR/*.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":

@@ -13,6 +13,16 @@ pytestmark = pytest.mark.gpu
 SIZES = [132, 4, 5, 18, 33, 64, 65, 17, 96, 31]
 
 
+@pytest.fixture(autouse=True)
+def _fixed_weights():
+    """The layers draw their glorot weights from torch's global generator, which every process seeds differently.
+    A ReLU output whose pre-activation lies within rounding of zero can fall on either side in the fp32 kernel and
+    the fp64 oracle, and that one flip moves a weight gradient by ~1e-2.  With seed 1 every pre-activation of these
+    tests stays >= 5e-6 of the output's magnitude away from zero, eight times the largest forward error of these
+    kernels (6e-7 relative on a B200)."""
+    torch.manual_seed(1)
+
+
 def _padded(n, F, Nmax, seed, relu=True):
     rng = np.random.default_rng(seed)
     X = np.zeros((len(n), Nmax, F), np.float32)
