@@ -85,11 +85,17 @@ _SIGNATURES = {
                             [_P] * 7 + [ctypes.c_size_t, _P]),
     "agcn_head_loss_grad_ex": (ctypes.c_int, [_P] * 8 + [ctypes.c_float, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
                                                      ctypes.c_int32] + [_P] * 7 + [ctypes.c_size_t, _P]),
+    "agcn_head_predict_workspace_bytes": (ctypes.c_int, [_P, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
+                                                          ctypes.POINTER(ctypes.c_size_t)]),
+    "agcn_head_predict": (ctypes.c_int, [_P] * 8 + [ctypes.c_float, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
+                                                ctypes.c_int32] + [_P] * 3 + [ctypes.c_size_t, _P]),
     "agcn_stack_create": (ctypes.c_int, [_P, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _P,
                                          ctypes.POINTER(_P)]),
     "agcn_stack_destroy": (ctypes.c_int, [_P]),
     "agcn_stack_workspace_bytes": (ctypes.c_int, [_P, _P, ctypes.POINTER(ctypes.c_size_t)]),
     "agcn_stack_loss_grad": (ctypes.c_int, [_P] * 6 + [ctypes.c_float] + [_P] * 4 + [ctypes.c_size_t, _P, _P, _P]),
+    "agcn_stack_predict_workspace_bytes": (ctypes.c_int, [_P, _P, ctypes.POINTER(ctypes.c_size_t)]),
+    "agcn_stack_predict": (ctypes.c_int, [_P] * 6 + [ctypes.c_float] + [_P] * 4 + [ctypes.c_size_t, _P]),
     "agcn_adam_step": (ctypes.c_int, [_P] * 5 + [ctypes.c_int64] + [ctypes.c_float] * 4 + [_P]),
     "agcn_sgcll_host_scratch_bytes": (ctypes.c_int, [ctypes.POINTER(Desc), _P, ctypes.POINTER(ctypes.c_size_t)]),
     "agcn_sgcll_forward_host": (ctypes.c_int, [ctypes.POINTER(Desc), _P] + [_P] * 8 + [ctypes.c_size_t, _P]),

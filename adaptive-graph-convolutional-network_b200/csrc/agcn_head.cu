@@ -153,6 +153,43 @@ __global__ void softmax_ce_kernel(float* __restrict__ logits, int ld, const floa
   if (lane == 0) part[b] = wb * (lse * sy - sxy) * scale;
 }
 
+// Prediction side of the same head (agcn_head_predict): probs[b, :] = softmax(x_b) = exp(x_b - logsumexp(x_b)), one warp
+// per sample.  With targets, part[b] receives the loss term of softmax_ce_kernel, evaluated by the same expressions in
+// the same order, so that the summed loss is bit-identical to the training step's.
+__global__ void softmax_predict_kernel(const float* __restrict__ logits, int ld, const float* __restrict__ y,
+                                       const float* __restrict__ w, int B, int C, float scale, float* __restrict__ probs,
+                                       float* __restrict__ part) {
+  const int b = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (b >= B) return;
+  const float* x = logits + (int64_t)b * ld;
+  float mx = -INFINITY;
+  for (int c = lane; c < C; c += 32) mx = fmaxf(mx, x[c]);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  float se = 0.f, sy = 0.f, sxy = 0.f;
+  for (int c = lane; c < C; c += 32) se += expf(x[c] - mx);
+  if (y) {
+    const float* yb = y + (int64_t)b * C;
+    for (int c = lane; c < C; c += 32) {
+      sy += yb[c];
+      sxy += yb[c] * x[c];
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    se += __shfl_xor_sync(0xffffffffu, se, o);
+    sy += __shfl_xor_sync(0xffffffffu, sy, o);
+    sxy += __shfl_xor_sync(0xffffffffu, sxy, o);
+  }
+  const float lse = mx + logf(se);
+  float* pb = probs + (int64_t)b * C;
+  for (int c = lane; c < C; c += 32) pb[c] = expf(x[c] - lse);
+  if (y && lane == 0) {
+    const float wb = w[b];
+    part[b] = wb * (lse * sy - sxy) * scale;
+  }
+}
+
 __global__ void sum_parts_kernel(const float* __restrict__ parts, int n, float* __restrict__ out) {
   __shared__ float red[256];
   float s = 0.f;
@@ -217,6 +254,35 @@ HeadWork carve_head(const agcn_plan* plan, int Fh, int Fm, int Nt, void* base) {
   tn = std::max(tn, tn_any_partial(t));
   w.tn_part = take(tn);
   w.splitk = take((size_t)8 * B * std::max(Fm, Fh));  // split-K partial sums of the two long contractions
+  w.bytes = off;
+  return w;
+}
+
+// agcn_head_predict's work area: the forward half of carve_head, plus the logits of the single-task head (the
+// multitask head's probabilities come straight out of the logits GEMM's epilogue)
+struct HeadPredictWork {
+  float *hsum, *pre, *mol, *logits, *loss_part, *tcB;
+  size_t bytes;
+};
+
+HeadPredictWork carve_head_predict(const agcn_plan* plan, int Fh, int Fm, int Nt, void* base) {
+  char* b = reinterpret_cast<char*>(base);
+  size_t off = 0;
+  auto take = [&](size_t floats) {
+    float* r = b ? reinterpret_cast<float*>(b + off) : nullptr;
+    off += al256(floats * sizeof(float));
+    return r;
+  };
+  const size_t B = plan->B;
+  HeadPredictWork w{};
+  w.hsum = take(B * Fh);
+  w.pre = take(B * Fm);
+  w.mol = take(B * Fm);
+  w.logits = take(B * pad4(Nt));
+  GemmArgs g;
+  g.M = (int)B; g.N = Nt; g.Z = 1; g.prob = 1;
+  w.loss_part = take(std::max((size_t)tc_gemm_loss_parts(g), B) + 64);
+  w.tcB = take(tc_gemm_scratch_floats(Nt, Fm, 1, 1));
   w.bytes = off;
   return w;
 }
@@ -391,6 +457,88 @@ int agcn_head_loss_grad_ex(const agcn_plan* plan, const float* d_H, const float*
   }
   AGCN_CUDA(cudaEventRecord(plan->ev_side_join, side));
   AGCN_CUDA(cudaStreamWaitEvent(st, plan->ev_side_join, 0));
+  return AGCN_OK;
+}
+
+int agcn_head_predict_workspace_bytes(const agcn_plan* plan, int32_t Fh, int32_t Fm, int32_t Nt, size_t* bytes) {
+  AGCN_REQUIRE(plan && bytes && Fh >= 1 && Fm >= 1 && Nt >= 1, "head_predict_workspace_bytes: bad arguments");
+  *bytes = carve_head_predict(plan, Fh, Fm, Nt, nullptr).bytes + 256;
+  return AGCN_OK;
+}
+
+int agcn_head_predict(const agcn_plan* plan, const float* d_H, const float* d_dense_W, const float* d_dense_b,
+                      const float* d_head_W, const float* d_head_b, const float* d_targets, const float* d_weights,
+                      float scale, int32_t loss_kind, int32_t Fh, int32_t Fm, int32_t Nt, float* d_probs, float* d_loss,
+                      void* d_work, size_t work_bytes, void* stream) {
+  AGCN_REQUIRE(!d_targets == !d_weights && !d_targets == !d_loss,
+               "head_predict: d_targets, d_weights and d_loss must be all NULL or all set");
+  AGCN_REQUIRE(plan && d_H && d_dense_W && d_dense_b && d_head_W && d_head_b && d_probs && d_work,
+               "head_predict: null pointer");
+  AGCN_REQUIRE(loss_kind == AGCN_LOSS_SIGMOID_CE || loss_kind == AGCN_LOSS_SOFTMAX_CE, "head_predict: unknown loss_kind");
+  AGCN_REQUIRE(Fh >= 1 && Fm >= 32 && Fm % 4 == 0 && Nt >= 1,
+               "head_predict: unsupported sizes (need Fm >= 32 and a multiple of 4)");
+  const bool sigmoid = loss_kind == AGCN_LOSS_SIGMOID_CE;
+  AGCN_REQUIRE(!sigmoid || Nt % 2 == 0, "head_predict: the multitask head needs two logits per task (Nt even)");
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc = plan_use(plan, st);
+  if (rc) return rc;
+  HeadPredictWork w = carve_head_predict(plan, Fh, Fm, Nt, d_work);
+  if (w.bytes > work_bytes) {
+    set_error("head_predict: workspace too small");
+    return AGCN_ERR_WORKSPACE;
+  }
+  const int B = plan->B, Ntp = pad4(Nt);
+  cudaStream_t side = plan->side;
+
+  // The products of agcn_head_loss_grad_ex with the same operands and the same tile configuration (the loss, when
+  // asked for, must be bit-identical to the training step's): `pre` on the CUDA cores, the logits on the tensor cores.
+  GemmArgs g_pre, g_log;
+  g_pre.M = B; g_pre.N = Fm; g_pre.Kd = Fh;
+  g_pre.A0 = w.hsum; g_pre.lda0 = Fh;
+  g_pre.B = d_dense_W; g_pre.ldb = Fm;
+  g_pre.C = w.pre; g_pre.ldc = Fm;
+  g_log.M = B; g_log.N = Nt; g_log.Kd = Fm;
+  g_log.A0 = w.mol; g_log.lda0 = Fm;
+  g_log.B = d_head_W; g_log.ldb = Nt;
+  g_log.bias = d_head_b;
+  if (sigmoid) {  // pairwise softmax epilogue: probabilities straight to d_probs
+    g_log.C = d_probs; g_log.ldc = Nt;
+    g_log.prob = 1;
+    if (d_targets) {
+      g_log.bce_y = d_targets; g_log.bce_w = d_weights; g_log.bce_ld = Nt; g_log.bce_scale = scale;
+      g_log.loss_part = w.loss_part;
+    }
+  } else {
+    g_log.C = w.logits; g_log.ldc = Ntp;
+  }
+  AGCN_REQUIRE(tc_gemm_supported(g_log), "head_predict: operands are not TMA-compatible (alignment)");
+  AGCN_CUDA(cudaEventRecord(plan->ev_side_fork, st));
+  AGCN_CUDA(cudaStreamWaitEvent(side, plan->ev_side_fork, 0));
+  if ((rc = tc_gemm_split_b(g_log, w.tcB, side))) return rc;
+  AGCN_CUDA(cudaEventRecord(plan->ev_side_join, side));
+
+  // GraphGatherMol + DenseMol (commuted) + tanh
+  segment_sum_kernel<<<(B + 7) / 8, 256, 0, st>>>(d_H, plan->d_node_off, B, Fh, w.hsum);
+  AGCN_LAUNCH_CHECK();
+  if ((rc = gemm_rows(g_pre, st))) return rc;
+  {
+    const int64_t total = (int64_t)B * Fm;
+    gather_tanh_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(w.pre, d_dense_b, plan->d_n, B, Fm, w.mol);
+    AGCN_LAUNCH_CHECK();
+  }
+  AGCN_CUDA(cudaStreamWaitEvent(st, plan->ev_side_join, 0));
+  if ((rc = tc_gemm(g_log, w.tcB, st))) return rc;
+  int n_parts = tc_gemm_loss_parts(g_log);
+  if (!sigmoid) {
+    softmax_predict_kernel<<<(B + 7) / 8, 256, 0, st>>>(w.logits, Ntp, d_targets, d_weights, B, Nt, scale, d_probs,
+                                                         w.loss_part);
+    AGCN_LAUNCH_CHECK();
+    n_parts = B;
+  }
+  if (d_loss) {
+    sum_parts_kernel<<<1, 256, 0, st>>>(w.loss_part, n_parts, d_loss);
+    AGCN_LAUNCH_CHECK();
+  }
   return AGCN_OK;
 }
 

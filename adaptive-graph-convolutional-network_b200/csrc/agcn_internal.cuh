@@ -200,6 +200,9 @@ struct GemmArgs {
   int bce_ld = 0;  // row pitch of bce_y / bce_w (0: same as ldc)
   float bce_scale = 1.f;
   float* loss_part = nullptr;
+  // tensor-core kernel only: prediction epilogue of the multitask head (agcn_head_predict): C receives the two-class
+  // softmax of every column pair (2t, 2t+1); with bce_y set, loss_part receives the same partial sums as above
+  int prob = 0;
   // tensor-core kernel only: scratch of 8 * M * N floats; when given, long contractions with few output tiles are
   // split along K (plain outputs only: no bias / activation / accumulate / loss epilogue, ldc == N, Z == 1)
   float* split_k_partial = nullptr;

@@ -1,4 +1,5 @@
-// A stack of SGC_LL layers + DenseMol + GraphGatherMol + logits + loss as ONE host call, and the Adam update.
+// A stack of SGC_LL layers + DenseMol + GraphGatherMol + logits + loss as ONE host call, its forward-only prediction
+// call, and the Adam update.
 //
 // The reference runs a training step as one `sess.run([train_op, loss, ...])`
 // (models/tf_modules/multitask_classifier.py:255-264): the TensorFlow runtime walks the whole graph of
@@ -96,6 +97,59 @@ int carve_stack(const agcn_stack* s, const agcn_plan* plan, void* base, StackWor
   return AGCN_OK;
 }
 
+// Forward-only arena of agcn_stack_predict: nothing outlives a layer call, so two ping-pong activation buffers and one
+// `saved` area (the layers run without AGCN_SAVE_FOR_BACKWARD; it is their forward scratch) serve every layer.
+struct PredictWork {
+  float* A = nullptr;  // activation ping-pong buffers [R, max Fo]
+  float* B = nullptr;
+  void* saved = nullptr;
+  void* layer_work = nullptr;
+  size_t layer_work_bytes = 0;
+  void* head_work = nullptr;
+  size_t head_work_bytes = 0;
+  size_t bytes = 0;
+};
+
+agcn_sgcll_desc forward_only(const agcn_sgcll_desc& d) {
+  agcn_sgcll_desc f = d;
+  f.flags = 0;
+  return f;
+}
+
+int carve_predict(const agcn_stack* s, const agcn_plan* plan, void* base, PredictWork* w) {
+  char* b = reinterpret_cast<char*>(base);
+  size_t off = 0;
+  auto take = [&](size_t bytes) {
+    void* r = b ? b + off : nullptr;
+    off += al256(bytes);
+    return r;
+  };
+  const size_t R = (size_t)plan->R;
+  int maxFo = 0;
+  size_t saved_max = 0, work_max = 0;
+  for (const agcn_sgcll_desc& d : s->layers) {
+    const agcn_sgcll_desc f = forward_only(d);
+    size_t saved = 0, work = 0;
+    int rc = agcn_sgcll_workspace_bytes(&f, plan, &saved, &work);
+    if (rc) return rc;
+    saved_max = std::max(saved_max, saved);
+    work_max = std::max(work_max, work);
+    maxFo = std::max(maxFo, d.Fo);
+  }
+  w->A = reinterpret_cast<float*>(take(R * maxFo * sizeof(float)));
+  w->B = reinterpret_cast<float*>(take(R * maxFo * sizeof(float)));
+  w->saved = take(saved_max);
+  w->layer_work_bytes = work_max;
+  w->layer_work = take(work_max);
+  size_t hb = 0;
+  int rc = agcn_head_predict_workspace_bytes(plan, s->layers.back().Fo, s->Fm, s->Nt, &hb);
+  if (rc) return rc;
+  w->head_work_bytes = hb;
+  w->head_work = take(hb);
+  w->bytes = off;
+  return AGCN_OK;
+}
+
 }  // namespace
 }  // namespace agcn
 
@@ -184,6 +238,46 @@ int agcn_stack_loss_grad(const agcn_stack* s, const agcn_plan* plan, const float
     std::swap(dcur, dnext);
   }
   return AGCN_OK;
+}
+
+int agcn_stack_predict_workspace_bytes(const agcn_stack* s, const agcn_plan* plan, size_t* bytes) {
+  AGCN_REQUIRE(s && plan && bytes, "stack_predict_workspace_bytes: null pointer");
+  PredictWork w;
+  int rc = carve_predict(s, plan, nullptr, &w);
+  if (rc) return rc;
+  *bytes = w.bytes + 256;
+  return AGCN_OK;
+}
+
+int agcn_stack_predict(const agcn_stack* s, const agcn_plan* plan, const float* d_X, const float* d_Lint,
+                       const float* d_targets, const float* d_weights, float scale, const float* d_params,
+                       float* d_probs, float* d_loss, void* d_work, size_t work_bytes, void* stream) {
+  AGCN_REQUIRE(!d_targets == !d_weights && !d_targets == !d_loss,
+               "stack_predict: d_targets, d_weights and d_loss must be all NULL or all set");
+  AGCN_REQUIRE(s && plan && d_X && d_Lint && d_params && d_probs && d_work, "stack_predict: null pointer");
+  PredictWork w;
+  int rc = carve_predict(s, plan, d_work, &w);
+  if (rc) return rc;
+  if (w.bytes > work_bytes) {
+    set_error("stack_predict: workspace too small");
+    return AGCN_ERR_WORKSPACE;
+  }
+  const int nl = (int)s->layers.size();
+  auto P = [&](int l, int k) { return s->off[5 * (size_t)l + k] >= 0 ? d_params + s->off[5 * (size_t)l + k] : nullptr; };
+  const int64_t* ho = &s->off[5 * (size_t)nl];
+  const float* x = d_X;
+  float* out = w.A;
+  for (int l = 0; l < nl; ++l) {
+    const agcn_sgcll_desc d = forward_only(s->layers[l]);
+    rc = agcn_sgcll_forward(&d, plan, x, d_Lint, nullptr, P(l, 2), P(l, 0), P(l, 1), P(l, 3), nullptr, out, nullptr,
+                            nullptr, nullptr, w.saved, w.layer_work, w.layer_work_bytes, stream);
+    if (rc) return rc;
+    x = out;
+    out = out == w.A ? w.B : w.A;
+  }
+  return agcn_head_predict(plan, x, d_params + ho[0], d_params + ho[1], d_params + ho[2], d_params + ho[3], d_targets,
+                           d_weights, scale, s->loss_kind, s->layers.back().Fo, s->Fm, s->Nt, d_probs, d_loss,
+                           w.head_work, w.head_work_bytes, stream);
 }
 
 int agcn_adam_step(float* d_params, const float* d_grads, float* d_m, float* d_v, int32_t* d_step, int64_t n, float lr,

@@ -107,7 +107,11 @@ struct Smem {
   static constexpr int TOTAL = STAGES * STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/;
 };
 
-template <int BN, int ST = 0>
+// PROB: the multitask head's prediction epilogue (agcn_head_predict): C receives the two-class softmax of every column
+// pair (2t, 2t+1) instead of the product, and with bce_y set the same pass adds up the weighted sigmoid cross-entropy
+// exactly as the training epilogue does.  A lane owns 4 consecutive columns starting at a multiple of 4, so a pair never
+// straddles lanes or tiles.
+template <int BN, int ST = 0, bool PROB = false>
 __global__ void __launch_bounds__(192, ST == 2 ? 2 : 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmA1,
                const __grid_constant__ CUtensorMap tmBhi, const __grid_constant__ CUtensorMap tmBlo, Args p) {
@@ -296,7 +300,24 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
           const long long off = (long long)m * p.ldc + cc;
           float* dst = Cz + off;
           o.x = o.x * sc + bv.x; o.y = o.y * sc + bv.y; o.z = o.z * sc + bv.z; o.w = o.w * sc + bv.w;
-          if (vec_ok && cc + 3 < p.N) {
+          if constexpr (PROB) {
+            // loss terms in the order of the training epilogue (the gradient finish() returns is dropped), then
+            // probs[2t + c] = 1 / (1 + exp(x[2t + 1 - c] - x[2t + c]))
+            const float ov[4] = {o.x, o.y, o.z, o.w};
+#pragma unroll
+            for (int e = 0; e < 4; ++e)
+              if (cc + e < p.N) (void)finish(ov[e], 0.f, yv[i][e], wv[i][e]);
+            const float4 pr = make_float4(1.f / (1.f + expf(o.y - o.x)), 1.f / (1.f + expf(o.x - o.y)),
+                                          1.f / (1.f + expf(o.w - o.z)), 1.f / (1.f + expf(o.z - o.w)));
+            if (vec_ok && cc + 3 < p.N) {
+              *reinterpret_cast<float4*>(dst) = pr;
+            } else {
+              const float pv[4] = {pr.x, pr.y, pr.z, pr.w};
+#pragma unroll
+              for (int e = 0; e < 4; ++e)
+                if (cc + e < p.N) dst[e] = pv[e];
+            }
+          } else if (vec_ok && cc + 3 < p.N) {
             float4 old = make_float4(0.f, 0.f, 0.f, 0.f);
             if (p.accumulate) old = *reinterpret_cast<const float4*>(dst);
             o.x = finish(o.x, old.x, yv[i][0], wv[i][0]); o.y = finish(o.y, old.y, yv[i][1], wv[i][1]);
@@ -656,7 +677,7 @@ bool tc_gemm_supported(const GemmArgs& a) {
 // (ToxCast head, 1024 x 1234 x 256: 55 us with 80 CTAs of 128 columns).
 static bool tc_gemm_narrow2(const GemmArgs& a) {
   const int Npad = tc_npad(a.N);
-  if (!a.bce_y || Npad <= 64) return false;
+  if (!(a.bce_y || a.prob) || Npad <= 64) return false;
   const int tiles128 = ((a.M + tc::BM - 1) / tc::BM) * a.Z * (Npad / 128);
   return tiles128 < 148;
 }
@@ -683,6 +704,29 @@ int tc_gemm_split_b(const GemmArgs& a, float* scratch, cudaStream_t st) {
   split_b_kernel<<<blocks, 256, 0, st>>>(a.B, sn, sk, ss, a.N, Npad, a.Kd, Kp, slices, Bhi, Blo);
   AGCN_LAUNCH_CHECK();
   return AGCN_OK;
+}
+
+template <int BN, int ST, bool PROB>
+static void launch_tc_gemm_kernel(dim3 grid, const CUtensorMap& mA0, const CUtensorMap& mA1, const CUtensorMap& mBhi,
+                                  const CUtensorMap& mBlo, const tc::Args& p, cudaStream_t st) {
+  using namespace tc;
+  static std::once_flag once;
+  std::call_once(once, [] {
+    cudaFuncSetAttribute(tc_gemm_kernel<BN, ST, PROB>, cudaFuncAttributeMaxDynamicSharedMemorySize, Smem<BN, ST>::TOTAL);
+  });
+  ProfScope prof(PROB ? "tc::tc_gemm_kernel<prob>" : "tc::tc_gemm_kernel", st);
+  tc_gemm_kernel<BN, ST, PROB><<<grid, 192, Smem<BN, ST>::TOTAL, st>>>(mA0, mA1, mBhi, mBlo, p);
+}
+
+template <bool PROB>
+static void launch_tc_gemm(bool narrow2, int BN, dim3 grid, const CUtensorMap& mA0, const CUtensorMap& mA1,
+                           const CUtensorMap& mBhi, const CUtensorMap& mBlo, const tc::Args& p, cudaStream_t st) {
+  if (narrow2)
+    launch_tc_gemm_kernel<64, 2, PROB>(grid, mA0, mA1, mBhi, mBlo, p, st);
+  else if (BN == 64)
+    launch_tc_gemm_kernel<64, 0, PROB>(grid, mA0, mA1, mBhi, mBlo, p, st);
+  else
+    launch_tc_gemm_kernel<128, 0, PROB>(grid, mA0, mA1, mBhi, mBlo, p, st);
 }
 
 // scratch holds the hi / lo copies of B written by tc_gemm_split_b (tc_gemm_scratch_floats floats).
@@ -713,8 +757,8 @@ int tc_gemm(const GemmArgs& a, const float* scratch, cudaStream_t st) {
   // split-K for long contractions with few output tiles (plain outputs only): partial sums + one reduction
   const int out_tiles = ((a.M + BM - 1) / BM) * a.Z * (Npad / BN);
   int ksplit = 1;
-  if (a.split_k_partial && !a.bias && !a.scale && a.act == AGCN_ACT_LINEAR && !a.accumulate && !a.bce_y && a.ldc == a.N && a.Z == 1 &&
-      total_kb >= 16 && out_tiles < 74)
+  if (a.split_k_partial && !a.bias && !a.scale && a.act == AGCN_ACT_LINEAR && !a.accumulate && !a.bce_y && !a.prob &&
+      a.ldc == a.N && a.Z == 1 && total_kb >= 16 && out_tiles < 74)
     ksplit = std::min(std::min(8, total_kb / 4), std::max(1, 148 / out_tiles));
   p.ksplit = ksplit;
   p.kb_per_split = (total_kb + ksplit - 1) / ksplit;
@@ -731,33 +775,10 @@ int tc_gemm(const GemmArgs& a, const float* scratch, cudaStream_t st) {
   p.bce_y = a.bce_y; p.bce_w = a.bce_w; p.bce_scale = a.bce_scale; p.loss_part = a.loss_part;
   p.bce_ld = a.bce_ld > 0 ? a.bce_ld : a.ldc;
   dim3 grid((a.M + BM - 1) / BM, a.Z * ksplit, Npad / BN);
-  static std::once_flag once64, once128;
-  if (narrow2) {
-    static std::once_flag once642;
-    std::call_once(once642, [] {
-      cudaFuncSetAttribute(tc_gemm_kernel<64, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, Smem<64, 2>::TOTAL);
-    });
-    {
-      ProfScope prof("tc::tc_gemm_kernel", st);
-      tc_gemm_kernel<64, 2><<<grid, 192, Smem<64, 2>::TOTAL, st>>>(mA0, mA1, mBhi, mBlo, p);
-    }
-  } else if (BN == 64) {
-    std::call_once(once64, [] {
-      cudaFuncSetAttribute(tc_gemm_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, Smem<64>::TOTAL);
-    });
-    {
-      ProfScope prof("tc::tc_gemm_kernel", st);
-      tc_gemm_kernel<64><<<grid, 192, Smem<64>::TOTAL, st>>>(mA0, mA1, mBhi, mBlo, p);
-    }
-  } else {
-    std::call_once(once128, [] {
-      cudaFuncSetAttribute(tc_gemm_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, Smem<128>::TOTAL);
-    });
-    {
-      ProfScope prof("tc::tc_gemm_kernel", st);
-      tc_gemm_kernel<128><<<grid, 192, Smem<128>::TOTAL, st>>>(mA0, mA1, mBhi, mBlo, p);
-    }
-  }
+  if (a.prob)
+    launch_tc_gemm<true>(narrow2, BN, grid, mA0, mA1, mBhi, mBlo, p, st);
+  else
+    launch_tc_gemm<false>(narrow2, BN, grid, mA0, mA1, mBhi, mBlo, p, st);
   AGCN_LAUNCH_CHECK();
   if (ksplit > 1) {
     const long long elems = (long long)a.M * a.ldc;

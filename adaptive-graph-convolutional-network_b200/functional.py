@@ -175,6 +175,39 @@ def head_loss(H, dense_W, dense_b, head_W, head_b, targets, weights, batch, scal
                                    loss_kind)
 
 
+def head_predict(H, dense_W, dense_b, head_W, head_b, batch, loss_kind, targets=None, weights=None, scale=None):
+    """Class probabilities of the SimpleAGCN head on the packed output of the last SGC-LL layer (agcn_head_predict),
+    with no autograd node.  Returns (probs [B, Nt], loss or None).
+    loss_kind "sigmoid_ce": probs[b, 2t+c] = softmax over task t's two logits; "softmax_ce": softmax over the Nt
+    class logits.  With targets and weights (laid out as for head_loss) the loss is also computed: the same weighted
+    cross-entropy x scale as head_loss, bit for bit; scale defaults to 1 / batch size."""
+    if (targets is None) != (weights is None):
+        raise ValueError("head_predict: pass both targets and weights, or neither")
+    H = H.detach().contiguous()
+    R, Fh = H.shape
+    Fm, Nt = head_W.shape
+    B = batch.batch_size
+    dev = H.device
+    assert dense_W.shape == (Fh, Fm) and R == batch.total_nodes
+    loss = None
+    if targets is not None:
+        targets, weights = targets.detach().contiguous(), weights.detach().contiguous()
+        assert targets.shape == (B, Nt)
+        assert weights.numel() == (B * Nt if loss_kind == "sigmoid_ce" else B)
+        scale = 1.0 / B if scale is None else scale
+        loss = torch.empty(1, device=dev, dtype=torch.float32)
+    nbytes = ctypes.c_size_t()
+    _lib.check(_lib.lib().agcn_head_predict_workspace_bytes(batch.handle, Fh, Fm, Nt, ctypes.byref(nbytes)))
+    work = _Workspace.get(dev, nbytes.value)
+    probs = torch.empty(B, Nt, device=dev, dtype=torch.float32)
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib().agcn_head_predict(
+            batch.handle, _ptr(H), _ptr(dense_W.detach()), _ptr(dense_b.detach()), _ptr(head_W.detach()),
+            _ptr(head_b.detach()), _ptr(targets), _ptr(weights), float(scale or 0.0), _lib.LOSS[loss_kind], Fh, Fm, Nt,
+            _ptr(probs), _ptr(loss), _ptr(work), work.numel(), _stream_ptr(dev)))
+    return probs, (loss.reshape(()) if loss is not None else None)
+
+
 class _UnpackNodes(torch.autograd.Function):
     @staticmethod
     def forward(ctx, packed, batch):

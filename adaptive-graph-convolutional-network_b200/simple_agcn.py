@@ -102,6 +102,7 @@ class SimpleAGCNStep(object):
         _lib.check(_lib.lib().agcn_stack_create(descs, len(self.layers), self.Fm, self.Nt, _lib.LOSS[loss], offs_c,
                                                 ctypes.byref(self._stack)))
         self._arena = None
+        self._pred_arena = None
         self._step_graph = ctypes.c_void_p()
         self._graph_stream = None
         # opt-in: capture the NCCL all-reduce of the multi-GPU step too (launched by torch.distributed on its own stream,
@@ -187,6 +188,63 @@ class SimpleAGCNStep(object):
         loss = self.forward_loss(X, Lint, batch, targets, weights)
         loss.backward()
         return loss.detach().reshape(1)
+
+    # ---- prediction (predict_proba / predict / evaluate of the reference's classifiers) -------------------------
+    def _predict_stack(self, X, Lint, batch, targets, weights, scale):
+        lib = _lib.lib()
+        nbytes = ctypes.c_size_t()
+        _lib.check(lib.agcn_stack_predict_workspace_bytes(self._stack, batch.handle, ctypes.byref(nbytes)))
+        if self._pred_arena is None or self._pred_arena.numel() < nbytes.value:
+            self._pred_arena = torch.empty(int(nbytes.value * 1.25) + 4096, dtype=torch.uint8, device=self.device)
+        probs = torch.empty(batch.batch_size, self.Nt, device=self.device, dtype=torch.float32)
+        loss = torch.empty(1, device=self.device, dtype=torch.float32) if targets is not None else None
+        with torch.cuda.device(self.device):
+            _lib.check(lib.agcn_stack_predict(
+                self._stack, batch.handle, _ptr(X), _ptr(Lint), _ptr(targets), _ptr(weights),
+                float(scale if scale is not None else 0.0), _ptr(self.flat_params.flat), _ptr(probs), _ptr(loss),
+                _ptr(self._pred_arena), self._pred_arena.numel(), _stream_ptr(self.device)))
+        return probs, (loss.reshape(()) if loss is not None else None)
+
+    def _predict(self, X, Lint, batch, targets=None, weights=None, scale=None):
+        """(probs [B, Nt], loss or None) of the current parameters; no gradient, no parameter or optimizer state
+        touched."""
+        X, Lint = X.contiguous(), Lint.contiguous()
+        assert X.shape[0] == batch.total_nodes and Lint.numel() == batch.total_lap
+        if targets is not None:
+            targets, weights = targets.contiguous(), weights.contiguous()
+            assert targets.shape == (batch.batch_size, self.Nt)
+            scale = 1.0 / batch.batch_size if scale is None else scale
+        if self.engine == "stack":
+            return self._predict_stack(X, Lint, batch, targets, weights, scale)
+        from .functional import head_predict
+        x = {'node_features': PackedNodes(X, batch), 'original_laplacian': PackedLaplacians(Lint, batch),
+             'data_slice': None, 'lap_slice': None, '_batch': batch}
+        with torch.no_grad():
+            for layer in self.layers:
+                out, _, _ = layer(x)
+                x = dict(x, node_features=out)
+            return head_predict(out.data, self.dense_W, self.dense_b, self.head_W, self.head_b, batch, self.loss_kind,
+                                targets, weights, scale)
+
+    def _shape_probs(self, probs):
+        return probs.reshape(probs.shape[0], -1, 2) if self.loss_kind == "sigmoid_ce" else probs
+
+    def predict_proba(self, X, Lint, batch):
+        """Class probabilities: [B, n_tasks, 2] for sigmoid_ce (softmax over each task's two logits), [B, n_classes]
+        for softmax_ce.  X [R, F] packed, Lint packed."""
+        return self._shape_probs(self._predict(X, Lint, batch)[0])
+
+    def predict(self, X, Lint, batch):
+        """Class labels (int64): [B, n_tasks] for sigmoid_ce, [B] for softmax_ce."""
+        return self.predict_proba(X, Lint, batch).argmax(-1)
+
+    def evaluate(self, X, Lint, batch, targets, weights, scale=None):
+        """(probabilities as predict_proba, loss): the loss is the training loss of this batch without its gradients,
+        bit for bit what loss_and_grads returns with the same scale (default 1 / batch size)."""
+        if targets is None or weights is None:
+            raise ValueError("evaluate needs targets and weights")
+        probs, loss = self._predict(X, Lint, batch, targets, weights, scale)
+        return self._shape_probs(probs), loss
 
     def apply_adam(self):
         with torch.cuda.device(self.device):

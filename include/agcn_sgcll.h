@@ -274,6 +274,23 @@ int agcn_head_loss_grad_ex(const agcn_plan* plan, const float* d_H, const float*
                            float* d_dH, float* d_ddense_W, float* d_ddense_b, float* d_dhead_W, float* d_dhead_b,
                            void* d_work, size_t work_bytes, void* stream);
 
+/* Prediction with the same head (the forward half of agcn_head_loss_grad_ex, no gradient): what predict_proba of
+ * MultitaskGraphClassifier / SingletaskGraphClassifier returns (models/tf_modules/multitask_classifier.py,
+ * singletask_classifier.py; parity unpinned, as the other TensorFlow ops of DESIGN.md section 7).
+ *   AGCN_LOSS_SIGMOID_CE: Nt = 2 n_tasks, column 2t+c = class c of task t; probs[b, 2t+c] is the softmax over that task's
+ *     two logits, 1 / (1 + exp(x[2t+1-c] - x[2t+c])) -- read as [B, n_tasks, 2], the layout of DeepChem's
+ *     MultitaskGraphClassifier.predict_proba (a softmax over every task's [B, 2] logits).  Nt must be even.  The
+ *     probabilities are the epilogue of the logits GEMM: the logits never reach memory.
+ *   AGCN_LOSS_SOFTMAX_CE: probs[b, :] = softmax over the Nt class logits.
+ *   d_probs [B,Nt] out.  d_targets / d_weights / d_loss are all NULL, or all set: then d_loss [1] also receives the
+ *   weighted loss x scale, bit-identical to the loss agcn_head_loss_grad_ex writes for the same inputs.
+ *   Same size rules as agcn_head_loss_grad_ex (Fm >= 32 and a multiple of 4). */
+int agcn_head_predict_workspace_bytes(const agcn_plan* plan, int32_t Fh, int32_t Fm, int32_t Nt, size_t* bytes);
+int agcn_head_predict(const agcn_plan* plan, const float* d_H, const float* d_dense_W, const float* d_dense_b,
+                      const float* d_head_W, const float* d_head_b, const float* d_targets, const float* d_weights,
+                      float scale, int32_t loss_kind, int32_t Fh, int32_t Fm, int32_t Nt, float* d_probs, float* d_loss,
+                      void* d_work, size_t work_bytes, void* stream);
+
 /* ---- one training step's loss and gradients as ONE call: the counterpart of `sess.run([train_op, loss, ...])`
  *      (models/tf_modules/multitask_classifier.py:255-264), which executes the whole graph of
  *      models/networks/basic_AGCN.py:35-47 inside the TensorFlow runtime.  A stack = n_layers SGC_LL layers (relu or
@@ -295,6 +312,16 @@ int agcn_stack_loss_grad(const agcn_stack* stack, const agcn_plan* plan, const f
                          const float* d_targets, const float* d_weights, float scale, const float* d_params,
                          float* d_grads, float* d_loss, void* d_work, size_t work_bytes, agcn_stack_notify_fn notify,
                          void* notify_user, void* stream);
+/* Forward-only counterpart of agcn_stack_loss_grad (predict_proba / evaluate of the reference's classifiers): the layers
+ * run without AGCN_SAVE_FOR_BACKWARD, then agcn_head_predict.  d_probs [B,Nt] as agcn_head_predict; d_targets /
+ * d_weights / d_loss all NULL or all set (then d_loss [1] is bit-identical to agcn_stack_loss_grad's loss for the same
+ * batch, parameters and scale).  Nothing outside d_probs, d_loss and d_work is written; no allocation, no
+ * synchronisation, no host callback (capturable).  The arena holds two [R, max Fo] activation buffers and ONE `saved`
+ * area that each layer reuses, so it is smaller than agcn_stack_workspace_bytes'. */
+int agcn_stack_predict_workspace_bytes(const agcn_stack* stack, const agcn_plan* plan, size_t* bytes);
+int agcn_stack_predict(const agcn_stack* stack, const agcn_plan* plan, const float* d_X, const float* d_Lint,
+                       const float* d_targets, const float* d_weights, float scale, const float* d_params,
+                       float* d_probs, float* d_loss, void* d_work, size_t work_bytes, void* stream);
 
 /* tf.train.AdamOptimizer's update (multitask_classifier.py:233-237) over a flat parameter buffer:
  *   t = *d_step + 1;  lr_t = lr sqrt(1 - beta2^t) / (1 - beta1^t);  m = beta1 m + (1 - beta1) g;
