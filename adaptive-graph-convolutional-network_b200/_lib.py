@@ -14,7 +14,7 @@ VARIANT = {"SGC_LL": 0, "SGC_LL_Reslap": 1}
 LAPLACIAN = {"reference_literal": 0, "paper": 1}
 METRIC_GRAD = {"reference": 0, "full": 1}
 ACT = {"linear": 0, "relu": 1}
-LOSS = {"sigmoid_ce": 0, "softmax_ce": 1}
+LOSS = {"sigmoid_ce": 0, "softmax_ce": 1, "weighted_l2": 2}
 ADJ_RULE = {"mean_distance": 0, "cutoff": 1}
 NOTIFY_FN = ctypes.CFUNCTYPE(None, ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p)
 OUT_RES_L, OUT_RES_W, OUT_L_ALL, SAVE_FOR_BACKWARD = 1, 2, 4, 8

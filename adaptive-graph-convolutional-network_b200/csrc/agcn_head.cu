@@ -5,11 +5,13 @@
 //   GraphGatherMol  per-graph sum over the real atoms, tanh      models/layers/graphgather.py:50-78
 //   logits          n_tasks independent [n_feature, 2] heads     models/operators/model_operatos.py:792-864
 //   loss            weighted sigmoid cross-entropy / batch size  models/tf_modules/multitask_classifier.py:41-44,187-209
+//   or, for regression, n_tasks [n_feature, 1] heads and the weighted L2 / batch size of DeepChem's
+//   MultitaskGraphRegressor (models/tf_modules/multitask_regressor.py, final_loss='weighted_L2'; parity unpinned)
 //
 // DenseMol is linear, so the gather commutes with it: sum_i (h_i W + b) = (sum_i h_i) W + n_g b.  The dense GEMM
 // then has B rows instead of R = sum n_g.  The n_tasks heads are one [n_feature, 2 n_tasks] matrix.  Every
-// contraction runs on the tcgen05 3xTF32 GEMMs of agcn_tc_gemm.cu; the cross-entropy and its gradient are the
-// epilogue of the logits GEMM, so the [B, 2 n_tasks] logits never reach HBM as logits.
+// contraction runs on the tcgen05 3xTF32 GEMMs of agcn_tc_gemm.cu; the cross-entropy (or the weighted L2) and its
+// gradient are the epilogue of the logits GEMM, so the [B, 2 n_tasks] logits never reach HBM as logits.
 #include <algorithm>
 
 #include "agcn_internal.cuh"
@@ -241,7 +243,7 @@ HeadWork carve_head(const agcn_plan* plan, int Fh, int Fm, int Nt, void* base) {
   w.dhsum = take(B * Fh);
   w.dWh_pad = take((size_t)Fm * Ntp);
   GemmArgs g;
-  g.M = (int)B; g.N = Nt; g.Z = 1;
+  g.M = (int)B; g.N = Nt; g.Z = 1; g.prob = 1;  // sized for the tiles of the fused-loss product
   w.loss_part = take(std::max((size_t)tc_gemm_loss_parts(g), B) + 64);
   w.tcA = take(tc_gemm_scratch_floats(Fm, Fh, 1, 1));   // dense_W            (pre   = hsum dense_W)
   w.tcB = take(tc_gemm_scratch_floats(Nt, Fm, 1, 1));   // head_W             (logits = mol head_W)
@@ -331,7 +333,9 @@ int agcn_head_loss_grad_ex(const agcn_plan* plan, const float* d_H, const float*
   AGCN_REQUIRE(plan && d_H && d_dense_W && d_dense_b && d_head_W && d_head_b && d_targets && d_weights && d_loss &&
                    d_dH && d_ddense_W && d_ddense_b && d_dhead_W && d_dhead_b && d_work,
                "head_loss_grad: null pointer");
-  AGCN_REQUIRE(loss_kind == AGCN_LOSS_SIGMOID_CE || loss_kind == AGCN_LOSS_SOFTMAX_CE, "head_loss_grad: unknown loss_kind");
+  AGCN_REQUIRE(loss_kind == AGCN_LOSS_SIGMOID_CE || loss_kind == AGCN_LOSS_SOFTMAX_CE ||
+                   loss_kind == AGCN_LOSS_WEIGHTED_L2,
+               "head_loss_grad: unknown loss_kind");
   // the logits GEMM carries the cross-entropy epilogue on the tensor cores: its contraction (Fm) must reach one
   // k-block with 16-byte operand pitches; every other contraction falls back to the CUDA-core kernels when its
   // shape is not TMA-compatible (e.g. 12 tasks: Nt = 24)
@@ -361,10 +365,11 @@ int agcn_head_loss_grad_ex(const agcn_plan* plan, const float* d_H, const float*
   g_log.B = d_head_W; g_log.ldb = Nt;
   g_log.C = w.dlog; g_log.ldc = Ntp;
   g_log.bias = d_head_b;
-  const bool sigmoid = loss_kind == AGCN_LOSS_SIGMOID_CE;
-  if (sigmoid) {
+  const bool softmax = loss_kind == AGCN_LOSS_SOFTMAX_CE;
+  if (!softmax) {  // sigmoid cross-entropy or weighted L2: the loss is the GEMM's epilogue
     g_log.bce_y = d_targets; g_log.bce_w = d_weights; g_log.bce_ld = Nt; g_log.bce_scale = scale;
     g_log.loss_part = w.loss_part;
+    g_log.l2 = loss_kind == AGCN_LOSS_WEIGHTED_L2;
   }
   g_dmol.M = B; g_dmol.N = Fm; g_dmol.Kd = Nt;
   g_dmol.A0 = w.dlog; g_dmol.lda0 = Ntp;
@@ -401,10 +406,10 @@ int agcn_head_loss_grad_ex(const agcn_plan* plan, const float* d_H, const float*
     gather_tanh_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(w.pre, d_dense_b, plan->d_n, B, Fm, w.mol);
     AGCN_LAUNCH_CHECK();
   }
-  // logits + weighted sigmoid cross-entropy: C receives d loss / d logits, the loss its per-warp partial sums
+  // logits + weighted sigmoid cross-entropy (weighted L2): C receives d loss / d logits, the loss its per-warp partial sums
   if ((rc = tc_gemm(g_log, w.tcB, st))) return rc;
   int n_parts = tc_gemm_loss_parts(g_log);
-  if (!sigmoid) {  // the GEMM wrote the logits; softmax cross-entropy and its gradient row by row
+  if (softmax) {  // the GEMM wrote the logits; softmax cross-entropy and its gradient row by row
     softmax_ce_kernel<<<(B + 7) / 8, 256, 0, st>>>(w.dlog, Ntp, d_targets, d_weights, B, Nt, scale, w.loss_part);
     AGCN_LAUNCH_CHECK();
     n_parts = B;
@@ -474,10 +479,12 @@ int agcn_head_predict(const agcn_plan* plan, const float* d_H, const float* d_de
                "head_predict: d_targets, d_weights and d_loss must be all NULL or all set");
   AGCN_REQUIRE(plan && d_H && d_dense_W && d_dense_b && d_head_W && d_head_b && d_probs && d_work,
                "head_predict: null pointer");
-  AGCN_REQUIRE(loss_kind == AGCN_LOSS_SIGMOID_CE || loss_kind == AGCN_LOSS_SOFTMAX_CE, "head_predict: unknown loss_kind");
+  AGCN_REQUIRE(loss_kind == AGCN_LOSS_SIGMOID_CE || loss_kind == AGCN_LOSS_SOFTMAX_CE ||
+                   loss_kind == AGCN_LOSS_WEIGHTED_L2,
+               "head_predict: unknown loss_kind");
   AGCN_REQUIRE(Fh >= 1 && Fm >= 32 && Fm % 4 == 0 && Nt >= 1,
                "head_predict: unsupported sizes (need Fm >= 32 and a multiple of 4)");
-  const bool sigmoid = loss_kind == AGCN_LOSS_SIGMOID_CE;
+  const bool sigmoid = loss_kind == AGCN_LOSS_SIGMOID_CE, softmax = loss_kind == AGCN_LOSS_SOFTMAX_CE;
   AGCN_REQUIRE(!sigmoid || Nt % 2 == 0, "head_predict: the multitask head needs two logits per task (Nt even)");
   cudaStream_t st = (cudaStream_t)stream;
   int rc = plan_use(plan, st);
@@ -501,9 +508,10 @@ int agcn_head_predict(const agcn_plan* plan, const float* d_H, const float* d_de
   g_log.A0 = w.mol; g_log.lda0 = Fm;
   g_log.B = d_head_W; g_log.ldb = Nt;
   g_log.bias = d_head_b;
-  if (sigmoid) {  // pairwise softmax epilogue: probabilities straight to d_probs
+  if (!softmax) {  // pairwise softmax epilogue: probabilities straight to d_probs (weighted L2: the values x)
     g_log.C = d_probs; g_log.ldc = Nt;
     g_log.prob = 1;
+    g_log.l2 = loss_kind == AGCN_LOSS_WEIGHTED_L2;
     if (d_targets) {
       g_log.bce_y = d_targets; g_log.bce_w = d_weights; g_log.bce_ld = Nt; g_log.bce_scale = scale;
       g_log.loss_part = w.loss_part;
@@ -529,7 +537,7 @@ int agcn_head_predict(const agcn_plan* plan, const float* d_H, const float* d_de
   AGCN_CUDA(cudaStreamWaitEvent(st, plan->ev_side_join, 0));
   if ((rc = tc_gemm(g_log, w.tcB, st))) return rc;
   int n_parts = tc_gemm_loss_parts(g_log);
-  if (!sigmoid) {
+  if (softmax) {
     softmax_predict_kernel<<<(B + 7) / 8, 256, 0, st>>>(w.logits, Ntp, d_targets, d_weights, B, Nt, scale, d_probs,
                                                          w.loss_part);
     AGCN_LAUNCH_CHECK();

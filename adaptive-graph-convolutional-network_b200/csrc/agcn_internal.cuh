@@ -193,7 +193,8 @@ struct GemmArgs {
   const float* scale = nullptr;  // optional device scalar: the product is multiplied by scale[0] before bias / accumulate
   int act = AGCN_ACT_LINEAR;
   int accumulate = 0;  // C += result
-  // tensor-core kernel only: fused weighted sigmoid cross-entropy epilogue (C = d loss / d logits, see agcn_head.cu);
+  // tensor-core kernel only: fused loss epilogue, weighted sigmoid cross-entropy unless l2 is set (C = d loss / d logits,
+  // see agcn_head.cu);
   // bce_y / bce_w are laid out like C, loss_part holds tc_gemm_loss_parts() floats
   const float* bce_y = nullptr;
   const float* bce_w = nullptr;
@@ -203,6 +204,9 @@ struct GemmArgs {
   // tensor-core kernel only: prediction epilogue of the multitask head (agcn_head_predict): C receives the two-class
   // softmax of every column pair (2t, 2t+1); with bce_y set, loss_part receives the same partial sums as above
   int prob = 0;
+  // tensor-core kernel only: the loss of the epilogues above is the weighted L2 of the regression head instead of the
+  // sigmoid cross-entropy (loss term (w (x - y))^2, C = 2 w^2 (x - y) bce_scale; with prob set C receives x itself)
+  int l2 = 0;
   // tensor-core kernel only: scratch of 8 * M * N floats; when given, long contractions with few output tiles are
   // split along K (plain outputs only: no bias / activation / accumulate / loss epilogue, ldc == N, Z == 1)
   float* split_k_partial = nullptr;

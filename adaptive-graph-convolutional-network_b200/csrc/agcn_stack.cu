@@ -161,7 +161,10 @@ int agcn_stack_create(const agcn_sgcll_desc* layer_descs, int32_t n_layers, int3
                       const int64_t* param_offsets, agcn_stack** out) {
   AGCN_REQUIRE(layer_descs && n_layers >= 1 && param_offsets && out, "stack_create: bad arguments");
   AGCN_REQUIRE(Fm >= 1 && Nt >= 1, "stack_create: Fm and Nt must be positive");
-  AGCN_REQUIRE(loss_kind == AGCN_LOSS_SIGMOID_CE || loss_kind == AGCN_LOSS_SOFTMAX_CE, "stack_create: unknown loss_kind");
+  // the head calls take loss_kind as it is: agcn_stack_loss_grad / agcn_stack_predict need nothing per kind
+  AGCN_REQUIRE(loss_kind == AGCN_LOSS_SIGMOID_CE || loss_kind == AGCN_LOSS_SOFTMAX_CE ||
+                   loss_kind == AGCN_LOSS_WEIGHTED_L2,
+               "stack_create: unknown loss_kind");
   for (int l = 0; l < n_layers; ++l) {
     AGCN_REQUIRE(layer_descs[l].variant == AGCN_VARIANT_SGC_LL, "stack_create: SGC_LL layers only (basic_AGCN.py:35-47)");
     AGCN_REQUIRE(l == 0 || layer_descs[l].F == layer_descs[l - 1].Fo, "stack_create: layer widths do not chain");

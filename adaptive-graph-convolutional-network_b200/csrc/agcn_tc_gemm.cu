@@ -111,7 +111,11 @@ struct Smem {
 // pair (2t, 2t+1) instead of the product, and with bce_y set the same pass adds up the weighted sigmoid cross-entropy
 // exactly as the training epilogue does.  A lane owns 4 consecutive columns starting at a multiple of 4, so a pair never
 // straddles lanes or tiles.
-template <int BN, int ST = 0, bool PROB = false>
+// L2: the regression head's weighted L2 takes the place of the sigmoid cross-entropy (DeepChem's
+// MultitaskGraphRegressor, final_loss='weighted_L2': the loss term is (w (x - y))^2, C receives 2 w^2 (x - y) bce_scale).
+// With PROB as well it is the regression head's prediction epilogue: C receives x itself, and with bce_y set the same
+// loss terms are added up in the order of the training epilogue.
+template <int BN, int ST = 0, bool PROB = false, bool L2 = false>
 __global__ void __launch_bounds__(192, ST == 2 ? 2 : 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmA1,
                const __grid_constant__ CUtensorMap tmBhi, const __grid_constant__ CUtensorMap tmBlo, Args p) {
@@ -240,9 +244,16 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
     auto finish = [&](float x, float old, float y, float w) -> float {
       if (p.accumulate) x += old;
       if (p.bce_y) {
-        // weighted sigmoid cross-entropy with logits (multitask_classifier.py:41-44): loss and its gradient
-        loss_acc += w * (fmaxf(x, 0.f) - x * y + log1pf(expf(-fabsf(x))));
-        return w * (1.f / (1.f + expf(-x)) - y) * p.bce_scale;
+        if constexpr (L2) {
+          // weighted L2, tf.square(tf.mul(tf.sub(x, t), w)): loss and its gradient
+          const float d = w * (x - y);
+          loss_acc += d * d;
+          return 2.f * w * d * p.bce_scale;
+        } else {
+          // weighted sigmoid cross-entropy with logits (multitask_classifier.py:41-44): loss and its gradient
+          loss_acc += w * (fmaxf(x, 0.f) - x * y + log1pf(expf(-fabsf(x))));
+          return w * (1.f / (1.f + expf(-x)) - y) * p.bce_scale;
+        }
       }
       return (p.act == AGCN_ACT_RELU) ? fmaxf(x, 0.f) : x;
     };
@@ -302,13 +313,14 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__
           o.x = o.x * sc + bv.x; o.y = o.y * sc + bv.y; o.z = o.z * sc + bv.z; o.w = o.w * sc + bv.w;
           if constexpr (PROB) {
             // loss terms in the order of the training epilogue (the gradient finish() returns is dropped), then
-            // probs[2t + c] = 1 / (1 + exp(x[2t + 1 - c] - x[2t + c]))
+            // probs[2t + c] = 1 / (1 + exp(x[2t + 1 - c] - x[2t + c]))  (L2: the values x)
             const float ov[4] = {o.x, o.y, o.z, o.w};
 #pragma unroll
             for (int e = 0; e < 4; ++e)
               if (cc + e < p.N) (void)finish(ov[e], 0.f, yv[i][e], wv[i][e]);
-            const float4 pr = make_float4(1.f / (1.f + expf(o.y - o.x)), 1.f / (1.f + expf(o.x - o.y)),
-                                          1.f / (1.f + expf(o.w - o.z)), 1.f / (1.f + expf(o.z - o.w)));
+            const float4 pr = L2 ? o
+                                 : make_float4(1.f / (1.f + expf(o.y - o.x)), 1.f / (1.f + expf(o.x - o.y)),
+                                               1.f / (1.f + expf(o.w - o.z)), 1.f / (1.f + expf(o.z - o.w)));
             if (vec_ok && cc + 3 < p.N) {
               *reinterpret_cast<float4*>(dst) = pr;
             } else {
@@ -674,7 +686,9 @@ bool tc_gemm_supported(const GemmArgs& a) {
 
 // The fused-loss logits product (M = batch, N = 2 n_tasks) has fewer 128-column tiles than SMs and a long epilogue per
 // tile: 64-column tiles, two stages, two CTAs per SM put twice as many CTAs to work at once
-// (ToxCast head, 1024 x 1234 x 256: 55 us with 80 CTAs of 128 columns).
+// (ToxCast head, 1024 x 1234 x 256: 55 us with 80 CTAs of 128 columns).  The decision depends on bce_y / prob only,
+// not on which loss (l2) they carry: a head's training and prediction products tile alike, so their loss terms are
+// added up in the same order.
 static bool tc_gemm_narrow2(const GemmArgs& a) {
   const int Npad = tc_npad(a.N);
   if (!(a.bce_y || a.prob) || Npad <= 64) return false;
@@ -706,27 +720,30 @@ int tc_gemm_split_b(const GemmArgs& a, float* scratch, cudaStream_t st) {
   return AGCN_OK;
 }
 
-template <int BN, int ST, bool PROB>
+template <int BN, int ST, bool PROB, bool L2>
 static void launch_tc_gemm_kernel(dim3 grid, const CUtensorMap& mA0, const CUtensorMap& mA1, const CUtensorMap& mBhi,
                                   const CUtensorMap& mBlo, const tc::Args& p, cudaStream_t st) {
   using namespace tc;
   static std::once_flag once;
   std::call_once(once, [] {
-    cudaFuncSetAttribute(tc_gemm_kernel<BN, ST, PROB>, cudaFuncAttributeMaxDynamicSharedMemorySize, Smem<BN, ST>::TOTAL);
+    cudaFuncSetAttribute(tc_gemm_kernel<BN, ST, PROB, L2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                         Smem<BN, ST>::TOTAL);
   });
-  ProfScope prof(PROB ? "tc::tc_gemm_kernel<prob>" : "tc::tc_gemm_kernel", st);
-  tc_gemm_kernel<BN, ST, PROB><<<grid, 192, Smem<BN, ST>::TOTAL, st>>>(mA0, mA1, mBhi, mBlo, p);
+  ProfScope prof(L2 ? (PROB ? "tc::tc_gemm_kernel<l2,prob>" : "tc::tc_gemm_kernel<l2>")
+                    : (PROB ? "tc::tc_gemm_kernel<prob>" : "tc::tc_gemm_kernel"),
+                 st);
+  tc_gemm_kernel<BN, ST, PROB, L2><<<grid, 192, Smem<BN, ST>::TOTAL, st>>>(mA0, mA1, mBhi, mBlo, p);
 }
 
-template <bool PROB>
+template <bool PROB, bool L2>
 static void launch_tc_gemm(bool narrow2, int BN, dim3 grid, const CUtensorMap& mA0, const CUtensorMap& mA1,
                            const CUtensorMap& mBhi, const CUtensorMap& mBlo, const tc::Args& p, cudaStream_t st) {
   if (narrow2)
-    launch_tc_gemm_kernel<64, 2, PROB>(grid, mA0, mA1, mBhi, mBlo, p, st);
+    launch_tc_gemm_kernel<64, 2, PROB, L2>(grid, mA0, mA1, mBhi, mBlo, p, st);
   else if (BN == 64)
-    launch_tc_gemm_kernel<64, 0, PROB>(grid, mA0, mA1, mBhi, mBlo, p, st);
+    launch_tc_gemm_kernel<64, 0, PROB, L2>(grid, mA0, mA1, mBhi, mBlo, p, st);
   else
-    launch_tc_gemm_kernel<128, 0, PROB>(grid, mA0, mA1, mBhi, mBlo, p, st);
+    launch_tc_gemm_kernel<128, 0, PROB, L2>(grid, mA0, mA1, mBhi, mBlo, p, st);
 }
 
 // scratch holds the hi / lo copies of B written by tc_gemm_split_b (tc_gemm_scratch_floats floats).
@@ -775,10 +792,14 @@ int tc_gemm(const GemmArgs& a, const float* scratch, cudaStream_t st) {
   p.bce_y = a.bce_y; p.bce_w = a.bce_w; p.bce_scale = a.bce_scale; p.loss_part = a.loss_part;
   p.bce_ld = a.bce_ld > 0 ? a.bce_ld : a.ldc;
   dim3 grid((a.M + BM - 1) / BM, a.Z * ksplit, Npad / BN);
-  if (a.prob)
-    launch_tc_gemm<true>(narrow2, BN, grid, mA0, mA1, mBhi, mBlo, p, st);
+  if (a.l2 && a.prob)
+    launch_tc_gemm<true, true>(narrow2, BN, grid, mA0, mA1, mBhi, mBlo, p, st);
+  else if (a.l2)
+    launch_tc_gemm<false, true>(narrow2, BN, grid, mA0, mA1, mBhi, mBlo, p, st);
+  else if (a.prob)
+    launch_tc_gemm<true, false>(narrow2, BN, grid, mA0, mA1, mBhi, mBlo, p, st);
   else
-    launch_tc_gemm<false>(narrow2, BN, grid, mA0, mA1, mBhi, mBlo, p, st);
+    launch_tc_gemm<false, false>(narrow2, BN, grid, mA0, mA1, mBhi, mBlo, p, st);
   AGCN_LAUNCH_CHECK();
   if (ksplit > 1) {
     const long long elems = (long long)a.M * a.ldc;

@@ -123,8 +123,8 @@ def sgc_ll_packed(X, Lint, Lprev, params, batch, cfg):
 
 class _HeadLossFunction(torch.autograd.Function):
     """DenseMol + GraphGatherMol(tanh) + multitask logits + weighted sigmoid cross-entropy * scale
-    (dense_layer.py:33-50, graphgather.py:50-78, model_operatos.py:792-864, multitask_classifier.py:41-44,187-209)
-    -> scalar loss.  The C call computes the loss AND every gradient; backward hands them out (scaled by the
+    (dense_layer.py:33-50, graphgather.py:50-78, model_operatos.py:792-864, multitask_classifier.py:41-44,187-209),
+    or the softmax / weighted-L2 heads (loss_kind) -> scalar loss.  The C call computes the loss AND every gradient; backward hands them out (scaled by the
     incoming gradient unless `unit_grad` says the loss is differentiated directly)."""
 
     @staticmethod
@@ -134,7 +134,7 @@ class _HeadLossFunction(torch.autograd.Function):
         Fm, Nt = head_W.shape
         dev = H.device
         assert dense_W.shape == (Fh, Fm) and targets.shape == (batch.batch_size, Nt) and R == batch.total_nodes
-        assert weights.numel() == (batch.batch_size * Nt if loss_kind == "sigmoid_ce" else batch.batch_size)
+        assert weights.numel() == (batch.batch_size if loss_kind == "softmax_ce" else batch.batch_size * Nt)
         nbytes = ctypes.c_size_t()
         _lib.check(_lib.lib().agcn_head_workspace_bytes(batch.handle, Fh, Fm, Nt, ctypes.byref(nbytes)))
         work = _Workspace.get(dev, nbytes.value)
@@ -169,7 +169,8 @@ def head_loss(H, dense_W, dense_b, head_W, head_b, targets, weights, batch, scal
               loss_kind="sigmoid_ce"):
     """Scalar loss of the SimpleAGCN head on the packed output of the last SGC-LL layer.
     loss_kind "sigmoid_ce": multitask two-class heads, weights [B, Nt]; "softmax_ce": one n_classes head,
-    weights [B].  unit_grad=True: the caller differentiates this loss directly (d loss / d loss = 1), which skips
+    weights [B]; "weighted_l2": n_tasks regression outputs (Nt = n_tasks), targets / weights [B, Nt] float,
+    loss = scale * sum (w (x - y))^2.  unit_grad=True: the caller differentiates this loss directly (d loss / d loss = 1), which skips
     the rescaling kernels; parameters registered with FlatGradBuffer(direct=...) require it."""
     return _HeadLossFunction.apply(H, dense_W, dense_b, head_W, head_b, targets, weights, batch, scale, unit_grad,
                                    loss_kind)
@@ -179,8 +180,9 @@ def head_predict(H, dense_W, dense_b, head_W, head_b, batch, loss_kind, targets=
     """Class probabilities of the SimpleAGCN head on the packed output of the last SGC-LL layer (agcn_head_predict),
     with no autograd node.  Returns (probs [B, Nt], loss or None).
     loss_kind "sigmoid_ce": probs[b, 2t+c] = softmax over task t's two logits; "softmax_ce": softmax over the Nt
-    class logits.  With targets and weights (laid out as for head_loss) the loss is also computed: the same weighted
-    cross-entropy x scale as head_loss, bit for bit; scale defaults to 1 / batch size."""
+    class logits; "weighted_l2": the regression values x [B, Nt] themselves, not probabilities.  With targets and
+    weights (laid out as for head_loss) the loss is also computed: the same weighted loss x scale as head_loss, bit for
+    bit; scale defaults to 1 / batch size."""
     if (targets is None) != (weights is None):
         raise ValueError("head_predict: pass both targets and weights, or neither")
     H = H.detach().contiguous()
@@ -193,7 +195,7 @@ def head_predict(H, dense_W, dense_b, head_W, head_b, batch, loss_kind, targets=
     if targets is not None:
         targets, weights = targets.detach().contiguous(), weights.detach().contiguous()
         assert targets.shape == (B, Nt)
-        assert weights.numel() == (B * Nt if loss_kind == "sigmoid_ce" else B)
+        assert weights.numel() == (B if loss_kind == "softmax_ce" else B * Nt)
         scale = 1.0 / B if scale is None else scale
         loss = torch.empty(1, device=dev, dtype=torch.float32)
     nbytes = ctypes.c_size_t()

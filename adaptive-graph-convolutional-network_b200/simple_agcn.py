@@ -4,8 +4,9 @@ The reference assembles the same stack in models/networks/basic_AGCN.py:35-47: f
 (l_n_filters = [64, 128, 128, 64], utils/hyper_parameters.py:14), DenseMol, GraphGatherMol(tanh), then either
 MultitaskGraphClassifier's per-task 2-class logits with weighted sigmoid cross-entropy divided by the batch size
 (models/tf_modules/multitask_classifier.py:41-44,187-209) or SingletaskGraphClassifier's n_classes logits with
-softmax cross-entropy (models/tf_modules/singletask_classifier.py:124-151), and tf.train.AdamOptimizer
-(multitask_classifier.py:233-237).  The reference executes one step as a single ``sess.run``; the counterpart
+softmax cross-entropy (models/tf_modules/singletask_classifier.py:124-151) or MultitaskGraphRegressor's one output per
+task with the weighted L2 divided by the batch size (models/tf_modules/multitask_regressor.py, DeepChem 1.x), and
+tf.train.AdamOptimizer (multitask_classifier.py:233-237).  The reference executes one step as a single ``sess.run``; the counterpart
 here is ONE library call, ``agcn_stack_loss_grad`` (engine="stack", the default and the path bench.py times),
 which chains the same C entry points the layer classes use.  engine="autograd" runs the same step through the
 layer classes and torch.autograd (the drop-in path of models/layers); tests pin both against the oracle and
@@ -34,7 +35,8 @@ class SimpleAGCNStep(object):
                  metric_grad="reference", seed=123, loss="sigmoid_ce", engine="stack", overlap_allreduce=False,
                  beta1=0.9, beta2=0.999, epsilon=1e-8):
         """loss="sigmoid_ce": n_tasks two-class heads (Nt = 2 n_tasks logits);  loss="softmax_ce": one head with
-        n_tasks classes (Nt = n_tasks logits)."""
+        n_tasks classes (Nt = n_tasks logits);  loss="weighted_l2": n_tasks regression outputs (Nt = n_tasks),
+        loss = sum (w (x - y))^2 / global batch."""
         if engine not in ("stack", "autograd"):
             raise ValueError("engine must be 'stack' or 'autograd'")
         if loss not in _lib.LOSS:
@@ -167,7 +169,7 @@ class SimpleAGCNStep(object):
 
     def forward_loss(self, X, Lint, batch, targets, weights):
         """The drop-in path: layer classes + torch.autograd.  X [R, F] packed, Lint packed, targets [B, Nt] float,
-        weights [B, Nt] (sigmoid_ce) or [B] (softmax_ce) -> scalar loss."""
+        weights [B, Nt] (sigmoid_ce, weighted_l2) or [B] (softmax_ce) -> scalar loss."""
         from .functional import head_loss
         x = {'node_features': PackedNodes(X, batch), 'original_laplacian': PackedLaplacians(Lint, batch),
              'data_slice': None, 'lap_slice': None, '_batch': batch}
@@ -189,7 +191,7 @@ class SimpleAGCNStep(object):
         loss.backward()
         return loss.detach().reshape(1)
 
-    # ---- prediction (predict_proba / predict / evaluate of the reference's classifiers) -------------------------
+    # ---- prediction (predict_proba / predict / evaluate of the reference's classifiers and regressor) ------------
     def _predict_stack(self, X, Lint, batch, targets, weights, scale):
         lib = _lib.lib()
         nbytes = ctypes.c_size_t()
@@ -206,8 +208,8 @@ class SimpleAGCNStep(object):
         return probs, (loss.reshape(()) if loss is not None else None)
 
     def _predict(self, X, Lint, batch, targets=None, weights=None, scale=None):
-        """(probs [B, Nt], loss or None) of the current parameters; no gradient, no parameter or optimizer state
-        touched."""
+        """(probs [B, Nt] -- the values for weighted_l2 --, loss or None) of the current parameters; no gradient, no
+        parameter or optimizer state touched."""
         X, Lint = X.contiguous(), Lint.contiguous()
         assert X.shape[0] == batch.total_nodes and Lint.numel() == batch.total_lap
         if targets is not None:
@@ -231,16 +233,22 @@ class SimpleAGCNStep(object):
 
     def predict_proba(self, X, Lint, batch):
         """Class probabilities: [B, n_tasks, 2] for sigmoid_ce (softmax over each task's two logits), [B, n_classes]
-        for softmax_ce.  X [R, F] packed, Lint packed."""
+        for softmax_ce.  X [R, F] packed, Lint packed.  A weighted_l2 regressor has none: ValueError (use predict)."""
+        if self.loss_kind == "weighted_l2":
+            raise ValueError("predict_proba: a regressor (loss='weighted_l2') has no class probabilities; use predict")
         return self._shape_probs(self._predict(X, Lint, batch)[0])
 
     def predict(self, X, Lint, batch):
-        """Class labels (int64): [B, n_tasks] for sigmoid_ce, [B] for softmax_ce."""
+        """Class labels (int64): [B, n_tasks] for sigmoid_ce, [B] for softmax_ce.  weighted_l2: the regression values
+        (float32) [B, n_tasks]."""
+        if self.loss_kind == "weighted_l2":
+            return self._predict(X, Lint, batch)[0]
         return self.predict_proba(X, Lint, batch).argmax(-1)
 
     def evaluate(self, X, Lint, batch, targets, weights, scale=None):
-        """(probabilities as predict_proba, loss): the loss is the training loss of this batch without its gradients,
-        bit for bit what loss_and_grads returns with the same scale (default 1 / batch size)."""
+        """(probabilities as predict_proba -- the values as predict for weighted_l2 --, loss): the loss is the training
+        loss of this batch without its gradients, bit for bit what loss_and_grads returns with the same scale (default
+        1 / batch size)."""
         if targets is None or weights is None:
             raise ValueError("evaluate needs targets and weights")
         probs, loss = self._predict(X, Lint, batch, targets, weights, scale)
@@ -340,8 +348,13 @@ def expand_labels(y, w, targets, weights, stream=None):
 
 def synthetic_labels(B, n_tasks, seed, device, loss="sigmoid_ce"):
     """sigmoid_ce: Bernoulli(0.1) labels as one-hot float targets [B, 2T], weights [B, 2T] = 1 (SURVEY.md 8d).
-    softmax_ce: uniform class labels as one-hot [B, T], per-sample weights [B] = 1."""
+    softmax_ce: uniform class labels as one-hot [B, T], per-sample weights [B] = 1.
+    weighted_l2: N(0, 1) targets [B, T], 0/1 weights [B, T] with about 10 % zeros (missing labels)."""
     rng = np.random.default_rng(seed)
+    if loss == "weighted_l2":
+        y = rng.standard_normal((B, n_tasks)).astype(np.float32)
+        w = (rng.random((B, n_tasks)) >= 0.1).astype(np.float32)
+        return torch.from_numpy(y).to(device), torch.from_numpy(w).to(device)
     if loss == "softmax_ce":
         y = rng.integers(0, n_tasks, B)
         onehot = np.zeros((B, n_tasks), np.float32)

@@ -254,13 +254,21 @@ int agcn_expand_labels(const uint8_t* y, const float* w, int32_t B, int32_t n_ta
  *   Needs Fm >= 32 and a multiple of 4 (the logits contraction runs on the tensor cores with the loss as its
  *   epilogue); the other contractions fall back to CUDA-core kernels when their shape is not TMA-compatible.
  *
- *   agcn_head_loss_grad_ex adds `loss_kind`: AGCN_LOSS_SIGMOID_CE (the multitask head above) or
+ *   agcn_head_loss_grad_ex adds `loss_kind`: AGCN_LOSS_SIGMOID_CE (the multitask head above),
  *   AGCN_LOSS_SOFTMAX_CE = the single-task multi-class head of SingletaskGraphClassifier
  *   (models/tf_modules/singletask_classifier.py:124-151, get_loss_fn('softmax_cross_entropy') of
  *   multitask_classifier.py:45-48): Nt = n_classes, d_targets [B,Nt] one-hot, d_weights [B] per-sample weights,
- *   loss = scale * sum_b w_b (logsumexp(x_b) - <y_b, x_b>). */
+ *   loss = scale * sum_b w_b (logsumexp(x_b) - <y_b, x_b>), or
+ *   AGCN_LOSS_WEIGHTED_L2 = the regression head of MultitaskGraphRegressor (models/tf_modules/multitask_regressor.py,
+ *   DeepChem 1.x, default final_loss='weighted_L2'; restated, parity unpinned): Nt = n_tasks, head_W [Fm,Nt] is one
+ *   [Fm,1] fully connected layer per task side by side, x[b,t] = (mol head_W + head_b)[b,t] with no activation,
+ *   d_targets / d_weights [B,Nt] float (no label expansion),
+ *   loss = scale * sum_b sum_t (w[b,t] (x[b,t] - y[b,t]))^2, d loss / d x = 2 w^2 (x - y) scale.  The weight enters
+ *   squared (tf.square(tf.mul(tf.sub(x, t), w))): with 0/1 weights masking missing labels that is w (x - y)^2.  The loss
+ *   and its gradient are the epilogue of the output GEMM, as for the sigmoid heads. */
 #define AGCN_LOSS_SIGMOID_CE 0
 #define AGCN_LOSS_SOFTMAX_CE 1
+#define AGCN_LOSS_WEIGHTED_L2 2
 int agcn_head_workspace_bytes(const agcn_plan* plan, int32_t Fh, int32_t Fm, int32_t Nt, size_t* bytes);
 int agcn_head_loss_grad(const agcn_plan* plan, const float* d_H, const float* d_dense_W, const float* d_dense_b,
                         const float* d_head_W, const float* d_head_b, const float* d_targets, const float* d_weights,
@@ -282,6 +290,8 @@ int agcn_head_loss_grad_ex(const agcn_plan* plan, const float* d_H, const float*
  *     MultitaskGraphClassifier.predict_proba (a softmax over every task's [B, 2] logits).  Nt must be even.  The
  *     probabilities are the epilogue of the logits GEMM: the logits never reach memory.
  *   AGCN_LOSS_SOFTMAX_CE: probs[b, :] = softmax over the Nt class logits.
+ *   AGCN_LOSS_WEIGHTED_L2: d_probs receives the regression values x [B, Nt = n_tasks] themselves (predict of
+ *     MultitaskGraphRegressor), written by the output GEMM's epilogue; there is no probability.
  *   d_probs [B,Nt] out.  d_targets / d_weights / d_loss are all NULL, or all set: then d_loss [1] also receives the
  *   weighted loss x scale, bit-identical to the loss agcn_head_loss_grad_ex writes for the same inputs.
  *   Same size rules as agcn_head_loss_grad_ex (Fm >= 32 and a multiple of 4). */
@@ -312,8 +322,9 @@ int agcn_stack_loss_grad(const agcn_stack* stack, const agcn_plan* plan, const f
                          const float* d_targets, const float* d_weights, float scale, const float* d_params,
                          float* d_grads, float* d_loss, void* d_work, size_t work_bytes, agcn_stack_notify_fn notify,
                          void* notify_user, void* stream);
-/* Forward-only counterpart of agcn_stack_loss_grad (predict_proba / evaluate of the reference's classifiers): the layers
- * run without AGCN_SAVE_FOR_BACKWARD, then agcn_head_predict.  d_probs [B,Nt] as agcn_head_predict; d_targets /
+/* Forward-only counterpart of agcn_stack_loss_grad (predict_proba / evaluate of the reference's classifiers, predict /
+ * evaluate of its regressor): the layers run without AGCN_SAVE_FOR_BACKWARD, then agcn_head_predict.  d_probs [B,Nt] as
+ * agcn_head_predict (the values x for AGCN_LOSS_WEIGHTED_L2); d_targets /
  * d_weights / d_loss all NULL or all set (then d_loss [1] is bit-identical to agcn_stack_loss_grad's loss for the same
  * batch, parameters and scale).  Nothing outside d_probs, d_loss and d_work is written; no allocation, no
  * synchronisation, no host callback (capturable).  The arena holds two [R, max Fo] activation buffers and ONE `saved`

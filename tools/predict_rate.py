@@ -1,6 +1,6 @@
 """Prediction rate of the SimpleAGCN stack against its training step, on bench.py's workloads.
 
-    python tools/predict_rate.py --out DIR [--configs C1,C2,C3] [--warmup 20] [--iters 100]
+    python tools/predict_rate.py --out DIR [--configs C1,C2,C3] [--warmup 20] [--iters 100] [--regression C1:1,C2:617]
 
 For every workload, with the batch resident in HBM (bench.py's inputs, one GPU):
   predict_eager     SimpleAGCNStep.predict_proba (one agcn_stack_predict call), eager launches
@@ -11,6 +11,10 @@ Each is the median over `iters` calls timed with CUDA events after `warmup` unti
 not timed) before every timed call, as bench.py does.  graphs/s = B / median.  The per-kernel table of one eager
 prediction comes from the library's own launch profiler (agcn_profile_enable / agcn_profile_read).  The card's name and
 power limit are read with a read-only nvidia-smi query in the same run.  Writes DIR/predict_rate.json and prints it.
+
+--regression KEY:T,... (opt-in) times the same four calls for the regression head (loss="weighted_l2", T outputs) on the
+inputs of workload KEY, with synthetic N(0, 1) targets and 0/1 weights; predict_* is SimpleAGCNStep.predict (the values).
+The results go to "regression" in the record, beside the classifiers of "configs".
 """
 import argparse
 import json
@@ -67,28 +71,40 @@ def captured(fn):
     return graph
 
 
-def run_config(key, warmup, iters, flush):
+def run_config(key, warmup, iters, flush, regression_tasks=None):
+    """regression_tasks = T: the weighted-L2 regressor with T outputs on workload `key`'s inputs instead of its
+    classifier."""
     import agcn_b200
     from agcn_b200 import _lib
-    from agcn_b200.simple_agcn import SimpleAGCNStep
+    from agcn_b200.simple_agcn import SimpleAGCNStep, synthetic_labels
     cfg = bench.WORKLOADS[key]
     dev = torch.device("cuda:0")
     X, L, n, tg, w = bench.make_inputs(cfg, 0)
     B = cfg["B"]
-    model = SimpleAGCNStep(cfg["F"], bench.FILTERS, bench.FINAL, cfg["n_tasks"], bench.K_ORDER, B, device=dev,
-                           loss=cfg["loss"])
+    loss, n_tasks = cfg["loss"], cfg["n_tasks"]
+    if regression_tasks is not None:
+        loss, n_tasks = "weighted_l2", regression_tasks
+    model = SimpleAGCNStep(cfg["F"], bench.FILTERS, bench.FINAL, n_tasks, bench.K_ORDER, B, device=dev, loss=loss)
     batch = agcn_b200.GraphBatch(n, cfg["Nmax"], device=dev)
     Xd, Ld = batch.pack_nodes(torch.from_numpy(X).to(dev)), batch.pack_lap(torch.from_numpy(L).to(dev))
-    tg_d, w_d = torch.from_numpy(tg).to(dev), torch.from_numpy(w).to(dev)
+    if regression_tasks is None:
+        tg_d, w_d = torch.from_numpy(tg).to(dev), torch.from_numpy(w).to(dev)
+    else:
+        tg_d, w_d = synthetic_labels(B, n_tasks, cfg["seed"], dev, loss)
 
     def predict():
-        model.predict_proba(Xd, Ld, batch)
+        if regression_tasks is None:
+            model.predict_proba(Xd, Ld, batch)
+        else:
+            model.predict(Xd, Ld, batch)
 
     def train():
         model.loss_and_grads(Xd, Ld, batch, tg_d, w_d)
         model.apply_adam()
 
     res = {"workload": cfg["name"], "B": B}
+    if regression_tasks is not None:
+        res.update(loss=loss, n_tasks=n_tasks)
     ms = {"predict_eager": median_ms(predict, warmup, iters, flush)}
     g = captured(predict)
     ms["predict_replay"] = median_ms(g.replay, warmup, iters, flush)
@@ -120,7 +136,13 @@ def main():
     ap.add_argument("--configs", default="C1,C2,C3")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--iters", type=int, default=100)
+    ap.add_argument("--regression", default="",
+                    help="opt-in: KEY:T,... times the weighted-L2 regressor with T outputs on workload KEY's inputs")
     args = ap.parse_args()
+    regression = [(k, int(t)) for k, t in (item.split(":") for item in args.regression.split(",") if item)]
+    for k, t in regression:
+        if k not in bench.WORKLOADS or t < 1:
+            raise SystemExit("--regression: KEY:T with KEY one of %s and T >= 1" % sorted(bench.WORKLOADS))
     if not torch.cuda.is_available():
         raise SystemExit("predict_rate.py measures on the GPU; no CUDA device found")
     flush = torch.empty(256 * 1024 * 1024 // 4, dtype=torch.float32, device="cuda:0")
@@ -131,6 +153,16 @@ def main():
         r = out["configs"][key]
         print("%s: predict %.0f graphs/s eager, %.0f replay; train step %.0f eager, %.0f replay; %d launches per predict"
               % (key, r["predict_eager"]["graphs_per_s"], r["predict_replay"]["graphs_per_s"],
+                 r["train_eager"]["graphs_per_s"], r["train_replay"]["graphs_per_s"], r["predict_launches"]),
+              flush=True)
+    if regression:
+        out["regression"] = {}
+    for key, t in regression:
+        name = "%s_T%d" % (key, t)
+        out["regression"][name] = r = run_config(key, args.warmup, args.iters, flush, regression_tasks=t)
+        print("%s weighted_l2: predict %.0f graphs/s eager, %.0f replay; train step %.0f eager, %.0f replay; "
+              "%d launches per predict"
+              % (name, r["predict_eager"]["graphs_per_s"], r["predict_replay"]["graphs_per_s"],
                  r["train_eager"]["graphs_per_s"], r["train_replay"]["graphs_per_s"], r["predict_launches"]),
               flush=True)
     os.makedirs(args.out, exist_ok=True)
