@@ -16,6 +16,7 @@ METRIC_GRAD = {"reference": 0, "full": 1}
 ACT = {"linear": 0, "relu": 1}
 LOSS = {"sigmoid_ce": 0, "softmax_ce": 1, "weighted_l2": 2}
 ADJ_RULE = {"mean_distance": 0, "cutoff": 1}
+NODE = {"sgcll": 0, "block_end": 1}
 NOTIFY_FN = ctypes.CFUNCTYPE(None, ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p)
 OUT_RES_L, OUT_RES_W, OUT_L_ALL, SAVE_FOR_BACKWARD = 1, 2, 4, 8
 
@@ -28,6 +29,11 @@ class Desc(ctypes.Structure):
     _fields_ = [("F", ctypes.c_int32), ("Fo", ctypes.c_int32), ("K", ctypes.c_int32), ("variant", ctypes.c_int32),
                 ("laplacian_mode", ctypes.c_int32), ("metric_grad", ctypes.c_int32), ("activation", ctypes.c_int32),
                 ("flags", ctypes.c_uint32)]
+
+
+class StackNode(ctypes.Structure):
+    """agcn_stack_node: one node of agcn_stack_create_nodes."""
+    _fields_ = [("kind", ctypes.c_int32), ("desc", Desc), ("src", ctypes.c_int32)]
 
 
 _P = ctypes.c_void_p
@@ -91,6 +97,8 @@ _SIGNATURES = {
                                                 ctypes.c_int32] + [_P] * 3 + [ctypes.c_size_t, _P]),
     "agcn_stack_create": (ctypes.c_int, [_P, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _P,
                                          ctypes.POINTER(_P)]),
+    "agcn_stack_create_nodes": (ctypes.c_int, [_P, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _P,
+                                               ctypes.POINTER(_P)]),
     "agcn_stack_destroy": (ctypes.c_int, [_P]),
     "agcn_stack_workspace_bytes": (ctypes.c_int, [_P, _P, ctypes.POINTER(ctypes.c_size_t)]),
     "agcn_stack_loss_grad": (ctypes.c_int, [_P] * 6 + [ctypes.c_float] + [_P] * 4 + [ctypes.c_size_t, _P, _P, _P]),

@@ -8,16 +8,28 @@
 // agcn_sgcll_forward / agcn_head_loss_grad_ex / agcn_sgcll_backward -- the very entry points the layer classes
 // use -- over one caller-provided arena, so a step costs one FFI crossing instead of ~10 autograd nodes with
 // their allocations.  Nothing new is computed here; the kernels are the ones of the per-layer entry points.
+//
+// A stack is a list of nodes (agcn_stack_create_nodes): SGC_LL layers, SGC_LL_Reslap layers whose L_prev is an earlier
+// Reslap layer's L_all (ResidualGraphMolResLap, tf_graphs.py:159-223), and BlockEnd nodes that close a residual block
+// (blockend.py:67-86, through agcn_node_gemm / agcn_gemm_tn as functional._NodeLinear calls them).
+// agcn_stack_create is the list of SGC_LL layers.
 #include <algorithm>
 #include <cmath>
+#include <string>
 #include <vector>
 
 #include "agcn_internal.cuh"
 
 struct agcn_stack {
-  std::vector<agcn_sgcll_desc> layers;
+  std::vector<agcn_stack_node> nodes;  // desc.flags as the layer classes set them
   int32_t Fm = 0, Nt = 0, loss_kind = 0;
-  std::vector<int64_t> off;  // 5 per layer {weight, bias, M_L, alpha, beta | -1}, then dense_W, dense_b, head_W, head_b
+  std::vector<int64_t> off;  // 5 per node {weight, bias, M_L, alpha, beta | -1}, then dense_W, dense_b, head_W, head_b
+  // topology, derived once by agcn_stack_create_nodes
+  std::vector<int32_t> lall_user;   // Reslap node i: the Reslap node whose L_prev is L_all[i], or -1
+  std::vector<int32_t> res_user;    // node i: the BlockEnd whose x_res is H[i], or -1
+  // agcn_stack_predict: slot of the activation buffer each node writes, slot of the L_all each Reslap node writes
+  std::vector<int32_t> pred_h, pred_l;
+  int32_t n_pred_h = 0, n_pred_l = 0;
 };
 
 namespace agcn {
@@ -48,22 +60,53 @@ __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, const 
 }
 __global__ void adam_advance_kernel(int32_t* step) { *step += 1; }
 
+// BlockEnd backward: dpre = dY * act'(Y), written as functional._NodeLinear writes it (dC * (C > 0) for relu, a copy of
+// dC for linear), so that the stack and the layer classes feed bit-identical operands to the products that follow.
+__global__ void __launch_bounds__(256) act_grad_kernel(const float* __restrict__ dY, const float* __restrict__ Y,
+                                                       float* __restrict__ dpre, long long n, int relu) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+    dpre[i] = relu ? dY[i] * (Y[i] > 0.f ? 1.f : 0.f) : dY[i];
+}
+
 namespace {
 
 inline size_t al256(size_t x) { return (x + 255) & ~(size_t)255; }
 
+bool is_reslap(const agcn_stack_node& n) {
+  return n.kind == AGCN_NODE_SGCLL && n.desc.variant == AGCN_VARIANT_SGC_LL_RESLAP;
+}
+
+// flags of a layer in agcn_stack_predict: no SAVE_FOR_BACKWARD (the `saved` area is forward scratch), the rest as in
+// training, so that every layer takes the same kernels in both calls
+agcn_sgcll_desc forward_only(const agcn_sgcll_desc& d) {
+  agcn_sgcll_desc f = d;
+  f.flags &= ~AGCN_SAVE_FOR_BACKWARD;
+  return f;
+}
+
+// scratch of a BlockEnd's products: agcn_node_gemm forward / dX (sized as functional._NodeLinear sizes it) and the TN dW
+size_t block_end_work(const agcn_sgcll_desc& d, const agcn_plan* plan) {
+  const int m = std::max(d.F, d.Fo);
+  return std::max(agcn_node_gemm_scratch_bytes(m, m), agcn_gemm_tn_scratch_bytes((int32_t)plan->R, d.F, d.Fo, 1));
+}
+
 struct StackWork {
-  std::vector<float*> H;      // activated output of layer l, [R, Fo_l]
-  std::vector<void*> saved;   // forward -> backward area of layer l
+  std::vector<float*> H;      // activated output of node i, [R, Fo_i]
+  std::vector<void*> saved;   // forward -> backward area of SGC-LL node i
   float* dA = nullptr;        // gradient ping-pong buffers [R, maxF]
   float* dB = nullptr;
   void* layer_work = nullptr;
   size_t layer_work_bytes = 0;
   void* head_work = nullptr;
   size_t head_work_bytes = 0;
+  std::vector<float*> Lall;   // Reslap node i: its L_all [sum n^2]
+  std::vector<float*> dLall;  // Reslap node i with a consumer: gradient into L_all[i] [sum n^2]
+  std::vector<float*> dpre;   // BlockEnd node i: dY * act'(Y) [R, Fo_i], alive until its dX product has run
   size_t bytes = 0;
 };
 
+// A plain SGC_LL stack (agcn_stack_create) carves exactly the areas it always had, in the same order; the Reslap and
+// BlockEnd areas come after them.
 int carve_stack(const agcn_stack* s, const agcn_plan* plan, void* base, StackWork* w) {
   char* b = reinterpret_cast<char*>(base);
   size_t off = 0;
@@ -72,15 +115,21 @@ int carve_stack(const agcn_stack* s, const agcn_plan* plan, void* base, StackWor
     off += al256(bytes);
     return r;
   };
-  const size_t R = (size_t)plan->R;
+  const size_t R = (size_t)plan->R, LL = (size_t)plan->LL;
+  const int n = (int)s->nodes.size();
   int maxF = 0;
   size_t work_max = 0;
-  for (const agcn_sgcll_desc& d : s->layers) {
+  for (const agcn_stack_node& nd : s->nodes) {
+    const agcn_sgcll_desc& d = nd.desc;
     size_t saved = 0, work = 0;
-    int rc = agcn_sgcll_workspace_bytes(&d, plan, &saved, &work);
-    if (rc) return rc;
+    if (nd.kind == AGCN_NODE_SGCLL) {
+      int rc = agcn_sgcll_workspace_bytes(&d, plan, &saved, &work);
+      if (rc) return rc;
+    } else {
+      work = block_end_work(d, plan);
+    }
     w->H.push_back(reinterpret_cast<float*>(take(R * d.Fo * sizeof(float))));
-    w->saved.push_back(take(saved));
+    w->saved.push_back(nd.kind == AGCN_NODE_SGCLL ? take(saved) : nullptr);
     work_max = std::max(work_max, work);
     maxF = std::max(maxF, std::max(d.F, d.Fo));
   }
@@ -89,19 +138,33 @@ int carve_stack(const agcn_stack* s, const agcn_plan* plan, void* base, StackWor
   w->layer_work_bytes = work_max;
   w->layer_work = take(work_max);
   size_t hb = 0;
-  int rc = agcn_head_workspace_bytes(plan, s->layers.back().Fo, s->Fm, s->Nt, &hb);
+  int rc = agcn_head_workspace_bytes(plan, s->nodes.back().desc.Fo, s->Fm, s->Nt, &hb);
   if (rc) return rc;
   w->head_work_bytes = hb;
   w->head_work = take(hb);
+  w->Lall.assign(n, nullptr);
+  w->dLall.assign(n, nullptr);
+  w->dpre.assign(n, nullptr);
+  for (int i = 0; i < n; ++i) {
+    const agcn_stack_node& nd = s->nodes[i];
+    if (is_reslap(nd)) {
+      w->Lall[i] = reinterpret_cast<float*>(take(LL * sizeof(float)));
+      if (s->lall_user[i] >= 0) w->dLall[i] = reinterpret_cast<float*>(take(LL * sizeof(float)));
+    } else if (nd.kind == AGCN_NODE_BLOCK_END) {
+      w->dpre[i] = reinterpret_cast<float*>(take(R * nd.desc.Fo * sizeof(float)));
+    }
+  }
   w->bytes = off;
   return AGCN_OK;
 }
 
-// Forward-only arena of agcn_stack_predict: nothing outlives a layer call, so two ping-pong activation buffers and one
-// `saved` area (the layers run without AGCN_SAVE_FOR_BACKWARD; it is their forward scratch) serve every layer.
+// Forward-only arena of agcn_stack_predict: one `saved` area serves every layer (the layers run without
+// AGCN_SAVE_FOR_BACKWARD; it is their forward scratch), and the activations and L_all matrices live in slots that are
+// reused as soon as their last reader has run (agcn_stack_create_nodes assigns them).  A plain SGC_LL stack gets two
+// activation slots, used alternately, and no L_all slot.
 struct PredictWork {
-  float* A = nullptr;  // activation ping-pong buffers [R, max Fo]
-  float* B = nullptr;
+  std::vector<float*> H;      // activation slots [R, max Fo]
+  std::vector<float*> L;      // L_all slots [sum n^2]
   void* saved = nullptr;
   void* layer_work = nullptr;
   size_t layer_work_bytes = 0;
@@ -109,12 +172,6 @@ struct PredictWork {
   size_t head_work_bytes = 0;
   size_t bytes = 0;
 };
-
-agcn_sgcll_desc forward_only(const agcn_sgcll_desc& d) {
-  agcn_sgcll_desc f = d;
-  f.flags = 0;
-  return f;
-}
 
 int carve_predict(const agcn_stack* s, const agcn_plan* plan, void* base, PredictWork* w) {
   char* b = reinterpret_cast<char*>(base);
@@ -127,27 +184,57 @@ int carve_predict(const agcn_stack* s, const agcn_plan* plan, void* base, Predic
   const size_t R = (size_t)plan->R;
   int maxFo = 0;
   size_t saved_max = 0, work_max = 0;
-  for (const agcn_sgcll_desc& d : s->layers) {
-    const agcn_sgcll_desc f = forward_only(d);
+  for (const agcn_stack_node& nd : s->nodes) {
     size_t saved = 0, work = 0;
-    int rc = agcn_sgcll_workspace_bytes(&f, plan, &saved, &work);
-    if (rc) return rc;
+    if (nd.kind == AGCN_NODE_SGCLL) {
+      const agcn_sgcll_desc f = forward_only(nd.desc);
+      int rc = agcn_sgcll_workspace_bytes(&f, plan, &saved, &work);
+      if (rc) return rc;
+    } else {
+      work = block_end_work(nd.desc, plan);
+    }
     saved_max = std::max(saved_max, saved);
     work_max = std::max(work_max, work);
-    maxFo = std::max(maxFo, d.Fo);
+    maxFo = std::max(maxFo, nd.desc.Fo);
   }
-  w->A = reinterpret_cast<float*>(take(R * maxFo * sizeof(float)));
-  w->B = reinterpret_cast<float*>(take(R * maxFo * sizeof(float)));
+  for (int k = 0; k < s->n_pred_h; ++k) w->H.push_back(reinterpret_cast<float*>(take(R * maxFo * sizeof(float))));
   w->saved = take(saved_max);
   w->layer_work_bytes = work_max;
   w->layer_work = take(work_max);
   size_t hb = 0;
-  int rc = agcn_head_predict_workspace_bytes(plan, s->layers.back().Fo, s->Fm, s->Nt, &hb);
+  int rc = agcn_head_predict_workspace_bytes(plan, s->nodes.back().desc.Fo, s->Fm, s->Nt, &hb);
   if (rc) return rc;
   w->head_work_bytes = hb;
   w->head_work = take(hb);
+  for (int k = 0; k < s->n_pred_l; ++k) w->L.push_back(reinterpret_cast<float*>(take((size_t)plan->LL * sizeof(float))));
   w->bytes = off;
   return AGCN_OK;
+}
+
+// Greedy slot assignment over the node order: value i is written by node i and read for the last time by node
+// last[i]; it takes the lowest slot whose value has had its last read before node i (a node's inputs stay untouched
+// while it writes its output).  want[i] = false: node i writes no value.
+int assign_slots(const std::vector<int32_t>& last, const std::vector<bool>& want, std::vector<int32_t>* slot) {
+  std::vector<int32_t> busy_until;   // per slot: last reader of the value it holds
+  slot->assign(last.size(), -1);
+  for (size_t i = 0; i < last.size(); ++i) {
+    if (!want[i]) continue;
+    int k = 0;
+    while (k < (int)busy_until.size() && busy_until[k] >= (int32_t)i) ++k;
+    if (k == (int)busy_until.size()) busy_until.push_back(0);
+    busy_until[k] = last[i];
+    (*slot)[i] = k;
+  }
+  return (int)busy_until.size();
+}
+
+// forward of BlockEnd node i (blockend.py:67-86) as functional._NodeLinear runs it: C = H[i-1], then
+// C += H[src] W with the activation in the product's epilogue
+int block_end_forward(const agcn_sgcll_desc& d, const agcn_plan* plan, const float* x, const float* x_res,
+                      const float* W, float* out, void* work, cudaStream_t st) {
+  const int32_t R = (int32_t)plan->R;
+  AGCN_CUDA(cudaMemcpyAsync(out, x, (size_t)R * d.Fo * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  return agcn_node_gemm(x_res, d.F, W, d.Fo, 0, out, d.Fo, R, d.Fo, d.F, nullptr, nullptr, 1, d.activation, work, st);
 }
 
 }  // namespace
@@ -157,25 +244,82 @@ using namespace agcn;
 
 extern "C" {
 
-int agcn_stack_create(const agcn_sgcll_desc* layer_descs, int32_t n_layers, int32_t Fm, int32_t Nt, int32_t loss_kind,
-                      const int64_t* param_offsets, agcn_stack** out) {
-  AGCN_REQUIRE(layer_descs && n_layers >= 1 && param_offsets && out, "stack_create: bad arguments");
+int agcn_stack_create_nodes(const agcn_stack_node* nodes, int32_t n_nodes, int32_t Fm, int32_t Nt, int32_t loss_kind,
+                            const int64_t* param_offsets, agcn_stack** out) {
+  AGCN_REQUIRE(nodes && n_nodes >= 1 && param_offsets && out, "stack_create: bad arguments");
+  *out = nullptr;
   AGCN_REQUIRE(Fm >= 1 && Nt >= 1, "stack_create: Fm and Nt must be positive");
   // the head calls take loss_kind as it is: agcn_stack_loss_grad / agcn_stack_predict need nothing per kind
   AGCN_REQUIRE(loss_kind == AGCN_LOSS_SIGMOID_CE || loss_kind == AGCN_LOSS_SOFTMAX_CE ||
                    loss_kind == AGCN_LOSS_WEIGHTED_L2,
                "stack_create: unknown loss_kind");
+  std::vector<int32_t> lall_user(n_nodes, -1), res_user(n_nodes, -1);
+  for (int i = 0; i < n_nodes; ++i) {
+    const agcn_stack_node& nd = nodes[i];
+    const agcn_sgcll_desc& d = nd.desc;
+    const std::string at = "stack_create_nodes: node " + std::to_string(i) + ": ";
+    AGCN_REQUIRE(nd.kind == AGCN_NODE_SGCLL || nd.kind == AGCN_NODE_BLOCK_END, at + "unknown kind");
+    if (nd.kind == AGCN_NODE_BLOCK_END) {
+      AGCN_REQUIRE(i > 0, at + "a BlockEnd cannot be the first node (it adds to the previous node's output)");
+      AGCN_REQUIRE(nd.src >= 0 && nd.src < i, at + "src must be an earlier node");
+      AGCN_REQUIRE(res_user[nd.src] < 0, at + "two BlockEnds name the same src");
+      AGCN_REQUIRE(d.F == nodes[nd.src].desc.Fo && d.Fo == nodes[i - 1].desc.Fo,
+                   at + "widths do not chain (F must be the width of H[src], Fo the width of H[i-1])");
+      res_user[nd.src] = i;
+      continue;
+    }
+    AGCN_REQUIRE(d.variant == AGCN_VARIANT_SGC_LL || d.variant == AGCN_VARIANT_SGC_LL_RESLAP, at + "unknown variant");
+    AGCN_REQUIRE(i == 0 || d.F == nodes[i - 1].desc.Fo, at + "widths do not chain (F must be the width of H[i-1])");
+    if (d.variant == AGCN_VARIANT_SGC_LL) {
+      AGCN_REQUIRE(nd.src == -1, at + "an SGC_LL layer takes no src (-1)");
+      continue;
+    }
+    AGCN_REQUIRE(param_offsets[5 * (size_t)i + 4] >= 0, at + "a Reslap layer needs a beta offset");
+    AGCN_REQUIRE(nd.src >= -1 && nd.src < i, at + "src must be an earlier node or -1");
+    if (nd.src >= 0) {
+      AGCN_REQUIRE(is_reslap(nodes[nd.src]), at + "a Reslap src must be a Reslap node (its L_all is this layer's L_prev)");
+      AGCN_REQUIRE(lall_user[nd.src] < 0, at + "two Reslap layers name the same src (the L_all chain is linear)");
+      lall_user[nd.src] = i;
+    }
+  }
+  agcn_stack* s = new agcn_stack();
+  s->nodes.assign(nodes, nodes + n_nodes);
+  for (agcn_stack_node& nd : s->nodes) {
+    // as functional._SGCLLFunction runs the layer classes
+    nd.desc.flags = AGCN_SAVE_FOR_BACKWARD | (is_reslap(nd) ? AGCN_OUT_L_ALL : 0u);
+    if (nd.kind == AGCN_NODE_SGCLL && !is_reslap(nd)) nd.src = -1;
+  }
+  s->Fm = Fm; s->Nt = Nt; s->loss_kind = loss_kind;
+  s->off.assign(param_offsets, param_offsets + 5 * (size_t)n_nodes + 4);
+  s->lall_user = lall_user;
+  s->res_user = res_user;
+  // prediction slots: H[i] is last read by node i+1 (the head for the last node) or by the BlockEnd it feeds x_res to;
+  // L_all[i] by the Reslap layer it is L_prev of
+  std::vector<int32_t> last_h(n_nodes), last_l(n_nodes);
+  std::vector<bool> all(n_nodes, true), reslap(n_nodes);
+  for (int i = 0; i < n_nodes; ++i) {
+    last_h[i] = std::max(i + 1, res_user[i]);
+    last_l[i] = std::max(i, lall_user[i]);
+    reslap[i] = is_reslap(s->nodes[i]);
+  }
+  s->n_pred_h = assign_slots(last_h, all, &s->pred_h);
+  s->n_pred_l = assign_slots(last_l, reslap, &s->pred_l);
+  *out = s;
+  return AGCN_OK;
+}
+
+int agcn_stack_create(const agcn_sgcll_desc* layer_descs, int32_t n_layers, int32_t Fm, int32_t Nt, int32_t loss_kind,
+                      const int64_t* param_offsets, agcn_stack** out) {
+  AGCN_REQUIRE(layer_descs && n_layers >= 1 && param_offsets && out, "stack_create: bad arguments");
+  std::vector<agcn_stack_node> nodes(n_layers);
   for (int l = 0; l < n_layers; ++l) {
     AGCN_REQUIRE(layer_descs[l].variant == AGCN_VARIANT_SGC_LL, "stack_create: SGC_LL layers only (basic_AGCN.py:35-47)");
     AGCN_REQUIRE(l == 0 || layer_descs[l].F == layer_descs[l - 1].Fo, "stack_create: layer widths do not chain");
+    nodes[l].kind = AGCN_NODE_SGCLL;
+    nodes[l].desc = layer_descs[l];
+    nodes[l].src = -1;
   }
-  agcn_stack* s = new agcn_stack();
-  s->layers.assign(layer_descs, layer_descs + n_layers);
-  for (agcn_sgcll_desc& d : s->layers) d.flags = AGCN_SAVE_FOR_BACKWARD;
-  s->Fm = Fm; s->Nt = Nt; s->loss_kind = loss_kind;
-  s->off.assign(param_offsets, param_offsets + 5 * (size_t)n_layers + 4);
-  *out = s;
-  return AGCN_OK;
+  return agcn_stack_create_nodes(nodes.data(), n_layers, Fm, Nt, loss_kind, param_offsets, out);
 }
 
 int agcn_stack_destroy(agcn_stack* s) {
@@ -205,40 +349,78 @@ int agcn_stack_loss_grad(const agcn_stack* s, const agcn_plan* plan, const float
     set_error("stack_loss_grad: workspace too small");
     return AGCN_ERR_WORKSPACE;
   }
-  const int nl = (int)s->layers.size();
+  cudaStream_t st = (cudaStream_t)stream;
+  const int nl = (int)s->nodes.size();
+  const int32_t R = (int32_t)plan->R;
   auto P = [&](int l, int k) { return s->off[5 * (size_t)l + k] >= 0 ? d_params + s->off[5 * (size_t)l + k] : nullptr; };
   auto G = [&](int l, int k) { return s->off[5 * (size_t)l + k] >= 0 ? d_grads + s->off[5 * (size_t)l + k] : nullptr; };
   const int64_t* ho = &s->off[5 * (size_t)nl];
-  // ---- forward (graphconv.py:85-125 per layer)
+  // ---- forward (graphconv.py:85-125 / graphconv_reslap.py:45-89 per layer, blockend.py:67-86 per BlockEnd)
   const float* x = d_X;
   for (int l = 0; l < nl; ++l) {
-    const agcn_sgcll_desc& d = s->layers[l];
-    rc = agcn_sgcll_forward(&d, plan, x, d_Lint, nullptr, P(l, 2), P(l, 0), P(l, 1), P(l, 3), nullptr, w.H[l], nullptr,
-                            nullptr, nullptr, w.saved[l], w.layer_work, w.layer_work_bytes, stream);
+    const agcn_stack_node& nd = s->nodes[l];
+    const agcn_sgcll_desc& d = nd.desc;
+    if (nd.kind == AGCN_NODE_BLOCK_END) {
+      rc = block_end_forward(d, plan, x, w.H[nd.src], P(l, 0), w.H[l], w.layer_work, st);
+    } else {
+      const float* Lprev = (is_reslap(nd) && nd.src >= 0) ? w.Lall[nd.src] : nullptr;
+      rc = agcn_sgcll_forward(&d, plan, x, d_Lint, Lprev, P(l, 2), P(l, 0), P(l, 1), P(l, 3), P(l, 4), w.H[l], nullptr,
+                              nullptr, w.Lall[l], w.saved[l], w.layer_work, w.layer_work_bytes, stream);
+    }
     if (rc) return rc;
     x = w.H[l];
   }
   // ---- DenseMol + GraphGatherMol + logits + loss, with every gradient of that part
-  const agcn_sgcll_desc& last = s->layers[nl - 1];
+  const agcn_sgcll_desc& last = s->nodes[nl - 1].desc;
   rc = agcn_head_loss_grad_ex(plan, w.H[nl - 1], d_params + ho[0], d_params + ho[1], d_params + ho[2], d_params + ho[3],
                               d_targets, d_weights, scale, s->loss_kind, last.Fo, s->Fm, s->Nt, d_loss, w.dA,
                               d_grads + ho[0], d_grads + ho[1], d_grads + ho[2], d_grads + ho[3], w.head_work,
                               w.head_work_bytes, stream);
   if (rc) return rc;
   if (notify) notify(notify_user, nl, stream);
-  // ---- backward, last layer first; the first layer's input has no gradient unless the metric is differentiable
+  // ---- backward, last node first; the first layer's input has no gradient unless the metric is differentiable.
+  // dH[i-1] is written by node i (an SGC-LL layer's dX, or a BlockEnd's dpre, which is the gradient of its residual
+  // add); a BlockEnd whose x_res is H[i-1] then adds dpre W^T to it, as autograd sums the two contributions.
   float* dcur = w.dA;
-  float* dnext = w.dB;
   for (int l = nl - 1; l >= 0; --l) {
-    const agcn_sgcll_desc& d = s->layers[l];
-    const bool full = d.laplacian_mode == AGCN_LAP_PAPER && d.metric_grad == AGCN_METRIC_GRAD_FULL;
-    float* dX = (l > 0 || full) ? dnext : nullptr;
-    rc = agcn_sgcll_backward(&d, plan, l == 0 ? d_X : w.H[l - 1], d_Lint, nullptr, P(l, 2), P(l, 0), P(l, 3), nullptr,
-                             w.H[l], dcur, nullptr, w.saved[l], dX, G(l, 2), G(l, 0), G(l, 1), G(l, 3), nullptr, nullptr,
-                             w.layer_work, w.layer_work_bytes, stream);
-    if (rc) return rc;
+    const agcn_stack_node& nd = s->nodes[l];
+    const agcn_sgcll_desc& d = nd.desc;
+    float* dnext = dcur == w.dA ? w.dB : w.dA;
+    float* dprev = nullptr;   // dH[l-1]
+    if (nd.kind == AGCN_NODE_BLOCK_END) {
+      const long long n = (long long)R * d.Fo;
+      act_grad_kernel<<<(unsigned)std::min<long long>((n + 255) / 256, 148 * 8), 256, 0, st>>>(
+          dcur, w.H[l], w.dpre[l], n, d.activation == AGCN_ACT_RELU);
+      AGCN_LAUNCH_CHECK();
+      // dW = H[src]^T dpre, on the kernel functional._NodeLinear picks for this shape
+      const int use_tc = (d.F <= 128 && d.F % 4 == 0 && d.Fo % 4 == 0 && R >= 32) ? 1 : 0;
+      rc = agcn_gemm_tn(w.H[nd.src], nullptr, w.dpre[l], G(l, 0), R, d.F, d.Fo, 1, w.layer_work, use_tc, stream);
+      if (rc) return rc;
+      dprev = w.dpre[l];
+      if (s->res_user[l - 1] >= 0) {   // more is added to dH[l-1]: keep dpre itself for this BlockEnd's dX product
+        AGCN_CUDA(cudaMemcpyAsync(dnext, dprev, (size_t)R * d.Fo * sizeof(float), cudaMemcpyDeviceToDevice, st));
+        dprev = dnext;
+      }
+    } else {
+      const bool full = d.laplacian_mode == AGCN_LAP_PAPER && d.metric_grad == AGCN_METRIC_GRAD_FULL;
+      const bool reslap = is_reslap(nd);
+      const float* Lprev = (reslap && nd.src >= 0) ? w.Lall[nd.src] : nullptr;
+      dprev = (l > 0 || full) ? dnext : nullptr;
+      rc = agcn_sgcll_backward(&d, plan, l == 0 ? d_X : w.H[l - 1], d_Lint, Lprev, P(l, 2), P(l, 0), P(l, 3), P(l, 4),
+                               w.H[l], dcur, reslap ? w.dLall[l] : nullptr, w.saved[l], dprev, G(l, 2), G(l, 0),
+                               G(l, 1), G(l, 3), G(l, 4), Lprev ? w.dLall[nd.src] : nullptr, w.layer_work,
+                               w.layer_work_bytes, stream);
+      if (rc) return rc;
+    }
     if (notify) notify(notify_user, l, stream);
-    std::swap(dcur, dnext);
+    if (l > 0 && s->res_user[l - 1] >= 0) {   // BlockEnd b's x_res is H[l-1]: dH[l-1] += dpre_b W_b^T
+      const int bn = s->res_user[l - 1];
+      const agcn_sgcll_desc& bd = s->nodes[bn].desc;
+      rc = agcn_node_gemm(w.dpre[bn], bd.Fo, P(bn, 0), bd.Fo, 1, dprev, bd.F, R, bd.F, bd.Fo, nullptr, nullptr, 1,
+                          AGCN_ACT_LINEAR, w.layer_work, stream);
+      if (rc) return rc;
+    }
+    dcur = dprev;
   }
   return AGCN_OK;
 }
@@ -265,21 +447,28 @@ int agcn_stack_predict(const agcn_stack* s, const agcn_plan* plan, const float* 
     set_error("stack_predict: workspace too small");
     return AGCN_ERR_WORKSPACE;
   }
-  const int nl = (int)s->layers.size();
+  const int nl = (int)s->nodes.size();
   auto P = [&](int l, int k) { return s->off[5 * (size_t)l + k] >= 0 ? d_params + s->off[5 * (size_t)l + k] : nullptr; };
   const int64_t* ho = &s->off[5 * (size_t)nl];
   const float* x = d_X;
-  float* out = w.A;
   for (int l = 0; l < nl; ++l) {
-    const agcn_sgcll_desc d = forward_only(s->layers[l]);
-    rc = agcn_sgcll_forward(&d, plan, x, d_Lint, nullptr, P(l, 2), P(l, 0), P(l, 1), P(l, 3), nullptr, out, nullptr,
-                            nullptr, nullptr, w.saved, w.layer_work, w.layer_work_bytes, stream);
+    const agcn_stack_node& nd = s->nodes[l];
+    const agcn_sgcll_desc d = forward_only(nd.desc);
+    float* out = w.H[s->pred_h[l]];
+    if (nd.kind == AGCN_NODE_BLOCK_END) {
+      rc = block_end_forward(d, plan, x, w.H[s->pred_h[nd.src]], P(l, 0), out, w.layer_work, (cudaStream_t)stream);
+    } else {
+      const bool reslap = is_reslap(nd);
+      const float* Lprev = (reslap && nd.src >= 0) ? w.L[s->pred_l[nd.src]] : nullptr;
+      rc = agcn_sgcll_forward(&d, plan, x, d_Lint, Lprev, P(l, 2), P(l, 0), P(l, 1), P(l, 3), P(l, 4), out, nullptr,
+                              nullptr, reslap ? w.L[s->pred_l[l]] : nullptr, w.saved, w.layer_work,
+                              w.layer_work_bytes, stream);
+    }
     if (rc) return rc;
     x = out;
-    out = out == w.A ? w.B : w.A;
   }
   return agcn_head_predict(plan, x, d_params + ho[0], d_params + ho[1], d_params + ho[2], d_params + ho[3], d_targets,
-                           d_weights, scale, s->loss_kind, s->layers.back().Fo, s->Fm, s->Nt, d_probs, d_loss,
+                           d_weights, scale, s->loss_kind, s->nodes.back().desc.Fo, s->Fm, s->Nt, d_probs, d_loss,
                            w.head_work, w.head_work_bytes, stream);
 }
 

@@ -55,9 +55,7 @@ class SimpleAGCNStep(object):
             raise ValueError("final_feature_n must be >= 32 and a multiple of 4 (agcn_head_loss_grad)")
         torch.manual_seed(seed)  # identical replicas on every rank
         _gc.DEFAULT_DEVICE[0] = str(self.device)
-        dims = [n_feat] + list(filters)
-        self.layers = [SGC_LL(dims[i + 1], dims[i], batch_size, K=K, activation='relu', laplacian=laplacian,
-                              metric_grad=metric_grad) for i in range(len(filters))]
+        self._build_layers(n_feat, filters, batch_size, K, laplacian, metric_grad)
         for l in self.layers:
             l.build()
         lim = float(np.sqrt(6.0 / (filters[-1] + final_feature_n)))
@@ -86,7 +84,7 @@ class SimpleAGCNStep(object):
             for name, v in l.vars.items():
                 per[name] = off
                 off += v.numel()
-            offs += [per["weight"], per["bias"], per["M_L"], per["alpha"], -1]
+            offs += [per.get(k, -1) for k in ("weight", "bias", "M_L", "alpha", "beta")]
             self._stage_slices.append((start, off))
         start = off
         for t in (self.dense_W, self.dense_b, self.head_W, self.head_b):
@@ -95,14 +93,7 @@ class SimpleAGCNStep(object):
         self._stage_slices.append((start, off))      # stage n_layers = dense + head
         assert off == self.flat_grad.numel()
         self._stack = ctypes.c_void_p()
-        descs = (_lib.Desc * len(self.layers))()
-        for i, l in enumerate(self.layers):
-            lap, mg = l._semantics()
-            descs[i] = _lib.Desc(l.n_atom_feature, l.nb_filter, l.K, _lib.VARIANT["SGC_LL"], _lib.LAPLACIAN[lap],
-                                 _lib.METRIC_GRAD[mg], _lib.ACT["relu"], _lib.SAVE_FOR_BACKWARD)
-        offs_c = (ctypes.c_int64 * len(offs))(*offs)
-        _lib.check(_lib.lib().agcn_stack_create(descs, len(self.layers), self.Fm, self.Nt, _lib.LOSS[loss], offs_c,
-                                                ctypes.byref(self._stack)))
+        self._create_stack((ctypes.c_int64 * len(offs))(*offs))
         self._arena = None
         self._pred_arena = None
         self._step_graph = ctypes.c_void_p()
@@ -117,6 +108,28 @@ class SimpleAGCNStep(object):
         self._loss = torch.zeros(1, device=self.device, dtype=torch.float32)
         self._pending = []
         self._notify = _lib.NOTIFY_FN(self._on_stage)     # keep the ctypes thunk alive
+
+    # ---- the body of the network (ResAGCNStep overrides these three) ---------------------------------------------
+    def _build_layers(self, n_feat, filters, batch_size, K, laplacian, metric_grad):
+        """self.layers, in the order of the flat buffers (basic_AGCN.py:35-45: SGC_LL layers with relu)."""
+        dims = [n_feat] + list(filters)
+        self.layers = [SGC_LL(dims[i + 1], dims[i], batch_size, K=K, activation='relu', laplacian=laplacian,
+                              metric_grad=metric_grad) for i in range(len(filters))]
+
+    def _create_stack(self, offs):
+        """self._stack from the layers and the flat-buffer offsets (5 per layer, then the 4 head tensors)."""
+        descs = (_lib.Desc * len(self.layers))()
+        for i, l in enumerate(self.layers):
+            descs[i] = _layer_desc(l)
+        _lib.check(_lib.lib().agcn_stack_create(descs, len(self.layers), self.Fm, self.Nt, _lib.LOSS[self.loss_kind],
+                                                offs, ctypes.byref(self._stack)))
+
+    def _body(self, x):
+        """The layer classes on the input dict of the drop-in path -> PackedNodes output of the last layer."""
+        for layer in self.layers:
+            out, _, _ = layer(x)
+            x = dict(x, node_features=out)
+        return out
 
     def __del__(self):
         try:
@@ -173,9 +186,7 @@ class SimpleAGCNStep(object):
         from .functional import head_loss
         x = {'node_features': PackedNodes(X, batch), 'original_laplacian': PackedLaplacians(Lint, batch),
              'data_slice': None, 'lap_slice': None, '_batch': batch}
-        for layer in self.layers:
-            out, _, _ = layer(x)
-            x = dict(x, node_features=out)
+        out = self._body(x)
         return head_loss(out.data, self.dense_W, self.dense_b, self.head_W, self.head_b, targets, weights, batch,
                          1.0 / self.global_batch, unit_grad=True, loss_kind=self.loss_kind)
 
@@ -222,9 +233,7 @@ class SimpleAGCNStep(object):
         x = {'node_features': PackedNodes(X, batch), 'original_laplacian': PackedLaplacians(Lint, batch),
              'data_slice': None, 'lap_slice': None, '_batch': batch}
         with torch.no_grad():
-            for layer in self.layers:
-                out, _, _ = layer(x)
-                x = dict(x, node_features=out)
+            out = self._body(x)
             return head_predict(out.data, self.dense_W, self.dense_b, self.head_W, self.head_b, batch, self.loss_kind,
                                 targets, weights, scale)
 
@@ -321,6 +330,13 @@ class SimpleAGCNStep(object):
                 # executable graph goes back to eager launches for good
                 self._graph_disabled = True
         return loss
+
+
+def _layer_desc(layer):
+    """agcn_sgcll_desc of an SGC_LL / SGC_LL_Reslap layer with a fused relu (the stack sets the flags)."""
+    lap, mg = layer._semantics()
+    return _lib.Desc(layer.n_atom_feature, layer.nb_filter, layer.K, _lib.VARIANT[layer.variant], _lib.LAPLACIAN[lap],
+                     _lib.METRIC_GRAD[mg], _lib.ACT["relu"], _lib.SAVE_FOR_BACKWARD)
 
 
 def expand_labels(y, w, targets, weights, stream=None):

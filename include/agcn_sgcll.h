@@ -334,6 +334,38 @@ int agcn_stack_predict(const agcn_stack* stack, const agcn_plan* plan, const flo
                        const float* d_targets, const float* d_weights, float scale, const float* d_params,
                        float* d_probs, float* d_loss, void* d_work, size_t work_bytes, void* stream);
 
+/* ---- residual networks in the same calls: a stack described as a list of nodes.  Node i takes H[i-1] as input (node 0
+ *      takes d_X); the last node's output feeds the head.  This is ResidualGraphMolResLap of the reference
+ *      (models/networks/tf_graphs.py:159-223): SGC_LL_Reslap layers whose L_prev is an earlier Reslap layer's L_all
+ *      (L_all = leaky_a(clip(leaky_a(clip(res_L)) + L_int + beta L_prev)), graphconv_reslap.py:91-230) and BlockEnd
+ *      nodes that close a residual block (blockend.py:67-86).
+ *   AGCN_NODE_SGCLL      an SGC_LL layer (desc.variant AGCN_VARIANT_SGC_LL, src -1) or an SGC_LL_Reslap layer
+ *                        (AGCN_VARIANT_SGC_LL_RESLAP; src = the earlier Reslap node whose L_all is its L_prev, or -1 for
+ *                        res_lap = []).  desc.flags is ignored: the stack sets what the layer classes set.
+ *   AGCN_NODE_BLOCK_END  H[i] = act(H[src] W + H[i-1]), act = desc.activation (relu or linear); desc.F = width of
+ *                        H[src], desc.Fo = width of H[i-1], the other desc fields 0.
+ *   param_offsets: 5 per node, then the 4 head tensors, as agcn_stack_create: SGC_LL {weight, bias, M_L, alpha, -1},
+ *      Reslap {weight, bias, M_L, alpha, beta}, BlockEnd {weight [F, Fo], -1, -1, -1, -1}.
+ *   Rejected (AGCN_ERR_INVALID, agcn_last_error names the node): an unknown kind or variant, a BlockEnd as node 0, a
+ *      src that is not an earlier node, a Reslap src that is not a Reslap node, two Reslap nodes or two BlockEnds
+ *      naming the same src, widths that do not chain, a Reslap node without a beta offset, an SGC_LL node with a src.
+ *   agcn_stack_workspace_bytes, agcn_stack_loss_grad, agcn_stack_predict(_workspace_bytes) and agcn_stack_destroy take
+ *   either kind of stack.  notify stages: n_nodes = head + dense, then node i's parameters, last node first.  The calls
+ *   chain agcn_sgcll_forward / agcn_sgcll_backward, agcn_node_gemm, agcn_gemm_tn and the head calls with the arguments
+ *   the layer classes pass them, so their results equal the layer classes' under torch.autograd bit for bit.  The
+ *   training arena keeps every node's output and `saved` area, one L_all per Reslap node and the gradients the
+ *   dependencies need; the prediction arena reuses activation and L_all slots once their last reader has run.
+ *   agcn_stack_create(descs, n, ...) is agcn_stack_create_nodes with every node an SGC_LL layer and src = -1. */
+#define AGCN_NODE_SGCLL 0
+#define AGCN_NODE_BLOCK_END 1
+typedef struct agcn_stack_node {
+  int32_t kind;           /* AGCN_NODE_*                                                                   */
+  agcn_sgcll_desc desc;   /* the layer (SGCLL) or {F, Fo, 0, 0, 0, 0, activation, 0} (BLOCK_END)          */
+  int32_t src;            /* Reslap: the L_prev producer or -1; BLOCK_END: the node whose output is x_res  */
+} agcn_stack_node;
+int agcn_stack_create_nodes(const agcn_stack_node* nodes, int32_t n_nodes, int32_t Fm, int32_t Nt, int32_t loss_kind,
+                            const int64_t* param_offsets, agcn_stack** out);
+
 /* tf.train.AdamOptimizer's update (multitask_classifier.py:233-237) over a flat parameter buffer:
  *   t = *d_step + 1;  lr_t = lr sqrt(1 - beta2^t) / (1 - beta1^t);  m = beta1 m + (1 - beta1) g;
  *   v = beta2 v + (1 - beta2) g^2;  p -= lr_t m / (sqrt(v) + eps);  *d_step = t.

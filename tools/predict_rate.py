@@ -15,6 +15,10 @@ power limit are read with a read-only nvidia-smi query in the same run.  Writes 
 --regression KEY:T,... (opt-in) times the same four calls for the regression head (loss="weighted_l2", T outputs) on the
 inputs of workload KEY, with synthetic N(0, 1) targets and 0/1 weights; predict_* is SimpleAGCNStep.predict (the values).
 The results go to "regression" in the record, beside the classifiers of "configs".
+
+--residual KEY,... (opt-in) times the same four calls for ResAGCNStep (agcn_b200.residual_agcn: the default residual
+body of SGC_LL_Reslap layers and BlockEnd blocks, then workload KEY's head) on workload KEY's inputs, and also counts the
+launches of one training step.  The results go to "residual" in the record.
 """
 import argparse
 import json
@@ -71,11 +75,12 @@ def captured(fn):
     return graph
 
 
-def run_config(key, warmup, iters, flush, regression_tasks=None):
+def run_config(key, warmup, iters, flush, regression_tasks=None, residual=False):
     """regression_tasks = T: the weighted-L2 regressor with T outputs on workload `key`'s inputs instead of its
-    classifier."""
+    classifier.  residual: ResAGCNStep's body instead of SimpleAGCN's."""
     import agcn_b200
     from agcn_b200 import _lib
+    from agcn_b200.residual_agcn import ResAGCNStep
     from agcn_b200.simple_agcn import SimpleAGCNStep, synthetic_labels
     cfg = bench.WORKLOADS[key]
     dev = torch.device("cuda:0")
@@ -84,7 +89,11 @@ def run_config(key, warmup, iters, flush, regression_tasks=None):
     loss, n_tasks = cfg["loss"], cfg["n_tasks"]
     if regression_tasks is not None:
         loss, n_tasks = "weighted_l2", regression_tasks
-    model = SimpleAGCNStep(cfg["F"], bench.FILTERS, bench.FINAL, n_tasks, bench.K_ORDER, B, device=dev, loss=loss)
+    if residual:
+        model = ResAGCNStep(cfg["F"], final_feature_n=bench.FINAL, n_tasks=n_tasks, K=bench.K_ORDER, batch_size=B,
+                            device=dev, loss=loss)
+    else:
+        model = SimpleAGCNStep(cfg["F"], bench.FILTERS, bench.FINAL, n_tasks, bench.K_ORDER, B, device=dev, loss=loss)
     batch = agcn_b200.GraphBatch(n, cfg["Nmax"], device=dev)
     Xd, Ld = batch.pack_nodes(torch.from_numpy(X).to(dev)), batch.pack_lap(torch.from_numpy(L).to(dev))
     if regression_tasks is None:
@@ -125,6 +134,12 @@ def run_config(key, warmup, iters, flush, regression_tasks=None):
     table = _lib.profile_read()
     _lib.profile_enable(False)
     res["predict_launches"] = c1 - c0
+    if residual:
+        res["layout"] = [type(l).__name__ for l in model.layers]
+        c0 = _lib.launch_count()
+        train()
+        res["train_launches"] = _lib.launch_count() - c0
+        torch.cuda.synchronize()
     res["predict_kernels_ms"] = {k: {"launches": v[0], "ms": v[1]} for k, v in sorted(table.items(),
                                                                                     key=lambda kv: -kv[1][1])}
     return res
@@ -138,11 +153,17 @@ def main():
     ap.add_argument("--iters", type=int, default=100)
     ap.add_argument("--regression", default="",
                     help="opt-in: KEY:T,... times the weighted-L2 regressor with T outputs on workload KEY's inputs")
+    ap.add_argument("--residual", default="",
+                    help="opt-in: KEY,... times ResAGCNStep (the residual body) on workload KEY's inputs")
     args = ap.parse_args()
     regression = [(k, int(t)) for k, t in (item.split(":") for item in args.regression.split(",") if item)]
     for k, t in regression:
         if k not in bench.WORKLOADS or t < 1:
             raise SystemExit("--regression: KEY:T with KEY one of %s and T >= 1" % sorted(bench.WORKLOADS))
+    residual = [k for k in args.residual.split(",") if k]
+    for k in residual:
+        if k not in bench.WORKLOADS:
+            raise SystemExit("--residual: KEY,... with KEY one of %s" % sorted(bench.WORKLOADS))
     if not torch.cuda.is_available():
         raise SystemExit("predict_rate.py measures on the GPU; no CUDA device found")
     flush = torch.empty(256 * 1024 * 1024 // 4, dtype=torch.float32, device="cuda:0")
@@ -165,6 +186,15 @@ def main():
               % (name, r["predict_eager"]["graphs_per_s"], r["predict_replay"]["graphs_per_s"],
                  r["train_eager"]["graphs_per_s"], r["train_replay"]["graphs_per_s"], r["predict_launches"]),
               flush=True)
+    if residual:
+        out["residual"] = {}
+    for key in residual:
+        out["residual"][key] = r = run_config(key, args.warmup, args.iters, flush, residual=True)
+        print("%s residual: predict %.0f graphs/s eager, %.0f replay; train step %.0f eager, %.0f replay; "
+              "%d launches per predict, %d per training step"
+              % (key, r["predict_eager"]["graphs_per_s"], r["predict_replay"]["graphs_per_s"],
+                 r["train_eager"]["graphs_per_s"], r["train_replay"]["graphs_per_s"], r["predict_launches"],
+                 r["train_launches"]), flush=True)
     os.makedirs(args.out, exist_ok=True)
     with open(os.path.join(args.out, "predict_rate.json"), "w") as f:
         json.dump(out, f, indent=1)
