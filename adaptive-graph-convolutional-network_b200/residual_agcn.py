@@ -25,6 +25,7 @@ import ctypes
 
 from . import _lib
 from .layers import BlockEnd, SGC_LL_Reslap
+from .layers.blockend import fused_activation
 from .simple_agcn import SimpleAGCNStep, _layer_desc
 
 
@@ -63,8 +64,12 @@ class ResAGCNStep(SimpleAGCNStep):
         arr = (_lib.StackNode * len(self.layers))()
         for i, (l, src) in enumerate(zip(self.layers, self.srcs)):
             if isinstance(l, BlockEnd):
+                act, host_act = fused_activation(l.activation)
+                if host_act is not None:
+                    raise ValueError("node %d: a BlockEnd in the stack must be relu or linear (its activation is "
+                                     "fused into the product)" % i)
                 arr[i] = _lib.StackNode(_lib.NODE["block_end"],
-                                        _lib.Desc(l.res_n_features, l.n_features, 0, 0, 0, 0, _lib.ACT["relu"], 0), src)
+                                        _lib.Desc(l.res_n_features, l.n_features, 0, 0, 0, 0, _lib.ACT[act], 0), src)
             else:
                 arr[i] = _lib.StackNode(_lib.NODE["sgcll"], _layer_desc(l), src)
         return arr
@@ -78,8 +83,10 @@ class ResAGCNStep(SimpleAGCNStep):
         for i, (layer, src) in enumerate(zip(self.layers, self.srcs)):
             if isinstance(layer, BlockEnd):
                 out = layer(dict(x, block_outputs=outs[src]))                    # blockend.py:46-65
-            else:
+            elif isinstance(layer, SGC_LL_Reslap):
                 out, _, _, lall[i] = layer(dict(x, res_lap=lall[src] if src >= 0 else []))
+            else:                                                                   # plain SGC_LL: no L_all
+                out, _, _ = layer(x)
             outs.append(out)
             x = dict(x, node_features=out)
         return out

@@ -1,6 +1,7 @@
 """The residual stack (agcn_stack_create_nodes, ResAGCNStep) without a GPU: the node constants of the C ABI and their
 binding, every rejection of agcn_stack_create_nodes with its message, the default layout accepted, ResAGCNStep's
-argument checks and flat-buffer offsets, and the residual oracle's BlockEnd gradient against its closed form."""
+argument checks and flat-buffer offsets, every topology of the device sweep accepted and laid out, and the residual
+oracle's BlockEnd gradient against its closed form."""
 import ctypes
 import os
 import re
@@ -9,6 +10,7 @@ import pytest
 import torch
 
 import residual_oracle as RES
+import residual_topologies as RT
 from oracle import sgcll_oracle as O
 
 AGCN_ERR_INVALID = -1
@@ -216,3 +218,51 @@ def test_oracle_block_end_gradient_matches_its_closed_form():
     assert float(W.grad.abs().max()) > 0
     # the second layer's beta weighs the first layer's L_all (its L_prev)
     assert p1["beta"].grad is not None and float(p1["beta"].grad.abs()) > 0
+
+
+@pytest.mark.parametrize("name", sorted(RT.TOPOLOGIES))
+def test_topology_sweep_is_accepted_and_laid_out(name):
+    """Every topology of tests/test_gpu_residual_topologies.py passes agcn_stack_create_nodes' checks, and the model
+    built on it hands the stack 5 offsets per node (beta only on Reslap nodes, -1 where a node has no such tensor)
+    plus the 4 head tensors, in the order of the flat buffers."""
+    from agcn_b200 import BlockEnd, SGC_LL_Reslap, _lib
+    spec = RT.widths(RT.TOPOLOGIES[name])
+    kind = {"R": 0, "S": 0, "BE": 1}
+    variant = {"R": _lib.VARIANT["SGC_LL_Reslap"], "S": _lib.VARIANT["SGC_LL"], "BE": 0}
+    assert _create([(kind[k], (F, Fo, 3 if k != "BE" else 0, variant[k], 0, 0, _lib.ACT[act], 0), src)
+                    for k, F, Fo, src, act in spec])[0] == 0
+
+    got = {}
+
+    def probe(model, offs):
+        got["offs"] = list(offs)
+
+    model = RT.topology_model(RT.TOPOLOGIES[name], batch_size=8, device="cpu", create_stack=probe)
+    assert model.srcs == [s[3] for s in spec]
+    nodes = model.nodes()
+    base = model.flat_params.flat.data_ptr()
+    for i, (l, (k, F, Fo, src, act)) in enumerate(zip(model.layers, spec)):
+        assert (nodes[i].kind, nodes[i].desc.F, nodes[i].desc.Fo, nodes[i].src) == (kind[k], F, Fo, src)
+        assert nodes[i].desc.activation == _lib.ACT[act]
+        assert isinstance(l, BlockEnd) == (k == "BE") and isinstance(l, SGC_LL_Reslap) == (k == "R")
+        want = [(l.vars[t].data_ptr() - base) // 4 if t in l.vars else -1
+                for t in ("weight", "bias", "M_L", "alpha", "beta")]
+        assert got["offs"][5 * i:5 * i + 5] == want
+        assert (want[4] >= 0) == (k == "R")
+        assert (want[1] >= 0) == (k != "BE")
+    n = len(spec)
+    assert len(got["offs"]) == 5 * n + 4
+    assert got["offs"][5 * n:] == [(getattr(model, t).data_ptr() - base) // 4
+                                   for t in ("dense_W", "dense_b", "head_W", "head_b")]
+    assert tuple(model.dense_W.shape) == (spec[-1][2], 256)
+
+
+def test_block_end_activation_reaches_the_stack():
+    """A BlockEnd node carries its layer's activation (a linear BlockEnd trains linear in the stack, as under autograd);
+    one the product cannot fuse is refused."""
+    from agcn_b200 import _lib
+    spec = [("R", 64, -1), ("R", 64, 0), ("BE", 0, "linear")]
+    model = RT.topology_model(spec, batch_size=8, device="cpu")
+    assert [model.nodes()[i].desc.activation for i in range(3)] == [_lib.ACT["relu"]] * 2 + [_lib.ACT["linear"]]
+    with pytest.raises(ValueError, match="node 2: a BlockEnd in the stack must be relu or linear"):
+        RT.topology_model([("R", 64, -1), ("R", 64, 0), ("BE", 0, "tanh")], batch_size=8, device="cpu")
