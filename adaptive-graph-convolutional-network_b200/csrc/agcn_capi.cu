@@ -9,8 +9,6 @@ using namespace agcn;
 
 namespace {
 
-inline size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
-
 // node-level GEMM: tensor cores when the operands are TMA-compatible, CUDA cores otherwise (F = 75)
 int node_gemm_tn(const GemmTNArgs& t, cudaStream_t st) {
   if (tc_gemm_tn_supported(t)) return tc_gemm_tn(t, st);
@@ -52,17 +50,6 @@ GemmArgs g_gemm_args(const agcn_sgcll_desc* d, int R, const float* dYp, const fl
   return g;
 }
 
-struct Carver {
-  char* base;
-  size_t off = 0;
-  explicit Carver(void* p) : base(reinterpret_cast<char*>(p)) {}
-  float* take(size_t floats) {
-    float* r = base ? reinterpret_cast<float*>(base + off) : nullptr;
-    off += align256(floats * sizeof(float));
-    return r;
-  }
-};
-
 struct Modes {
   bool shortcut, paper, reslap, full, need_dL;
 };
@@ -85,7 +72,7 @@ struct Saved {
 
 Saved carve_saved(const agcn_sgcll_desc* d, const agcn_plan* p, void* base) {
   const Modes m = modes_of(d);
-  Carver c(base);
+  Arena c(base);
   Saved s{};
   s.T = c.take((size_t)(d->K > 1 ? d->K - 1 : 0) * p->R * d->F);
   s.Lall = m.shortcut ? nullptr : c.take((size_t)p->LL);
@@ -95,7 +82,7 @@ Saved carve_saved(const agcn_sgcll_desc* d, const agcn_plan* p, void* base) {
   s.XW = m.full ? c.take((size_t)p->R * d->F) : nullptr;
   s.tcG = c.take(tc_gemm_scratch_floats(d->F, d->Fo, 1, d->K));  // hi / lo of W_k^T for the backward G GEMM
   s.ftG = c.take(fused_w_floats(d->F, d->Fo, d->K));             // the same operand in the fused backward's layout
-  s.bytes = c.off;
+  s.bytes = c.bytes;
   return s;
 }
 
@@ -116,7 +103,7 @@ struct Work {
 
 Work carve_work(const agcn_sgcll_desc* d, const agcn_plan* p, void* base) {
   const Modes m = modes_of(d);
-  Carver c(base);
+  Arena c(base);
   Work w{};
   w.XW = c.take((size_t)p->R * d->F);  // forward: X M_L (when the similarity is needed and not saved)
   w.dYp = c.take((size_t)p->R * d->Fo);
@@ -142,7 +129,7 @@ Work carve_work(const agcn_sgcll_desc* d, const agcn_plan* p, void* base) {
   w.tcM = c.take(tc_gemm_scratch_floats(d->F, d->F, 1, 1));
   w.big = c.take(big_work_floats(p, m.full));  // sweeps of the graphs with n > AGCN_SMALL_MAX
   w.ftY = c.take(fused_w_floats(d->Fo, d->F, d->K));  // pre-split W_k of the fused forward kernel
-  w.bytes = c.off;
+  w.bytes = c.bytes;
   return w;
 }
 
@@ -187,12 +174,12 @@ struct PadSaved {
   size_t bytes;
 };
 PadSaved carve_pad_saved(const agcn_sgcll_desc* d2, const agcn_plan* p, void* base) {
-  Carver c(base);
+  Arena c(base);
   PadSaved s{};
   s.Xp = c.take((size_t)p->R * d2->F);
   s.Wp = c.take((size_t)d2->F * d2->K * d2->Fo);
-  s.inner = base ? reinterpret_cast<char*>(base) + c.off : nullptr;
-  s.bytes = c.off + carve_saved(d2, p, nullptr).bytes + 256;
+  s.inner = c.area(carve_saved(d2, p, nullptr).bytes + 256);
+  s.bytes = c.bytes;
   return s;
 }
 struct PadWork {
@@ -201,15 +188,39 @@ struct PadWork {
   size_t inner_bytes, bytes;
 };
 PadWork carve_pad_work(const agcn_sgcll_desc* d2, const agcn_plan* p, void* base) {
-  Carver c(base);
+  Arena c(base);
   PadWork w{};
   w.dXp = c.take((size_t)p->R * d2->F);
   w.dWp = c.take((size_t)d2->F * d2->K * d2->Fo);
   w.dMp = c.take((size_t)d2->F * d2->F);
-  w.inner = base ? reinterpret_cast<char*>(base) + c.off : nullptr;
   w.inner_bytes = carve_work(d2, p, nullptr).bytes + 256;
-  w.bytes = c.off + w.inner_bytes;
+  w.inner = c.area(w.inner_bytes);
+  w.bytes = c.bytes;
   return w;
+}
+
+// agcn_sgcll_forward_host's scratch: the padded wire layouts of X, L and Y, their packed copies, the layer's areas
+struct HostScratch {
+  float *Xpad, *Lpad, *Ypad, *X, *L, *Y;
+  void *saved, *work;
+  size_t work_bytes, bytes;
+};
+HostScratch carve_host(const agcn_sgcll_desc* d, const agcn_plan* p, void* base) {
+  size_t saved = 0;
+  Arena c(base);
+  HostScratch h{};
+  agcn_sgcll_workspace_bytes(d, p, &saved, &h.work_bytes);
+  const size_t B = p->B, N = p->Nmax;
+  h.Xpad = c.take(B * N * d->F);
+  h.Lpad = c.take(B * N * N);
+  h.Ypad = c.take(B * N * d->Fo);
+  h.X = c.take((size_t)p->R * d->F);
+  h.L = c.take((size_t)p->LL);
+  h.Y = c.take((size_t)p->R * d->Fo);
+  h.saved = c.area(saved);
+  h.work = c.area(h.work_bytes);
+  h.bytes = c.bytes;
+  return h;
 }
 
 // dst[r, c] = c < Fs ? src[r, c] : 0   (rows x Fd)
@@ -656,15 +667,7 @@ int agcn_fused_debug_set(void* d_buf) {
 
 int agcn_sgcll_host_scratch_bytes(const agcn_sgcll_desc* desc, const agcn_plan* plan, size_t* bytes) {
   AGCN_REQUIRE(desc && plan && bytes, "null pointer");
-  size_t saved = 0, work = 0;
-  agcn_sgcll_workspace_bytes(desc, plan, &saved, &work);
-  const size_t B = plan->B, N = plan->Nmax;
-  size_t total = 0;
-  total += align256(B * N * desc->F * 4) + align256(B * N * N * 4) + align256(B * N * desc->Fo * 4);  // padded X, L, Y
-  total += align256((size_t)plan->R * desc->F * 4) + align256((size_t)plan->LL * 4) +
-           align256((size_t)plan->R * desc->Fo * 4);  // packed X, L, Y
-  total += align256(saved) + align256(work);
-  *bytes = total;
+  *bytes = carve_host(desc, plan, nullptr).bytes;
   return AGCN_OK;
 }
 
@@ -678,26 +681,13 @@ int agcn_sgcll_forward_host(const agcn_sgcll_desc* desc, const agcn_plan* plan, 
   AGCN_REQUIRE(desc->variant == AGCN_VARIANT_SGC_LL, "forward_host: SGC_LL only");
   AGCN_REQUIRE((desc->flags & (AGCN_OUT_RES_L | AGCN_OUT_RES_W | AGCN_OUT_L_ALL)) == 0,
                "forward_host: optional outputs are not supported");
-  size_t need = 0, saved = 0, work = 0;
-  agcn_sgcll_host_scratch_bytes(desc, plan, &need);
-  if (need > scratch_bytes) {
+  const HostScratch h = carve_host(desc, plan, d_scratch);
+  if (h.bytes > scratch_bytes) {
     set_error("forward_host: scratch too small");
     return AGCN_ERR_WORKSPACE;
   }
-  agcn_sgcll_workspace_bytes(desc, plan, &saved, &work);
   cudaStream_t st = (cudaStream_t)stream;
   const size_t B = plan->B, N = plan->Nmax;
-  char* base = reinterpret_cast<char*>(d_scratch);
-  size_t off = 0;
-  auto take = [&](size_t bytes) { char* r = base + off; off += align256(bytes); return r; };
-  float* dXpad = (float*)take(B * N * desc->F * 4);
-  float* dLpad = (float*)take(B * N * N * 4);
-  float* dYpad = (float*)take(B * N * desc->Fo * 4);
-  float* dX = (float*)take((size_t)plan->R * desc->F * 4);
-  float* dL = (float*)take((size_t)plan->LL * 4);
-  float* dY = (float*)take((size_t)plan->R * desc->Fo * 4);
-  void* dsaved = take(saved);
-  void* dwork = take(work);
   // Page-locked host arrays are mapped into the device's address space: the pack kernels then read them in place
   // and only the n_g real rows of every graph cross PCIe (the zero padding of the wire layout, 98 % of a
   // molecule batch, never moves).  Pageable arrays are staged through the copy engine.
@@ -714,20 +704,20 @@ int agcn_sgcll_forward_host(const agcn_sgcll_desc* desc, const agcn_plan* plan, 
   const float* xsrc = device_view(h_X_padded);
   const float* lsrc = device_view(h_L_padded);
   if (!xsrc) {
-    AGCN_CUDA(cudaMemcpyAsync(dXpad, h_X_padded, B * N * desc->F * 4, cudaMemcpyHostToDevice, st));
-    xsrc = dXpad;
+    AGCN_CUDA(cudaMemcpyAsync(h.Xpad, h_X_padded, B * N * desc->F * 4, cudaMemcpyHostToDevice, st));
+    xsrc = h.Xpad;
   }
   if (!lsrc) {
-    AGCN_CUDA(cudaMemcpyAsync(dLpad, h_L_padded, B * N * N * 4, cudaMemcpyHostToDevice, st));
-    lsrc = dLpad;
+    AGCN_CUDA(cudaMemcpyAsync(h.Lpad, h_L_padded, B * N * N * 4, cudaMemcpyHostToDevice, st));
+    lsrc = h.Lpad;
   }
-  if ((rc = agcn_pack_nodes(plan, xsrc, dX, desc->F, st))) return rc;
-  if ((rc = agcn_pack_lap(plan, lsrc, dL, st))) return rc;
-  if ((rc = agcn_sgcll_forward(desc, plan, dX, dL, nullptr, d_M_L, d_weight, d_bias, d_alpha, nullptr, dY, nullptr,
-                               nullptr, nullptr, dsaved, dwork, work, st)))
+  if ((rc = agcn_pack_nodes(plan, xsrc, h.X, desc->F, st))) return rc;
+  if ((rc = agcn_pack_lap(plan, lsrc, h.L, st))) return rc;
+  if ((rc = agcn_sgcll_forward(desc, plan, h.X, h.L, nullptr, d_M_L, d_weight, d_bias, d_alpha, nullptr, h.Y, nullptr,
+                               nullptr, nullptr, h.saved, h.work, h.work_bytes, st)))
     return rc;
-  if ((rc = agcn_unpack_nodes(plan, dY, dYpad, desc->Fo, st))) return rc;
-  AGCN_CUDA(cudaMemcpyAsync(h_Y_padded, dYpad, B * N * desc->Fo * 4, cudaMemcpyDeviceToHost, st));
+  if ((rc = agcn_unpack_nodes(plan, h.Y, h.Ypad, desc->Fo, st))) return rc;
+  AGCN_CUDA(cudaMemcpyAsync(h_Y_padded, h.Ypad, B * N * desc->Fo * 4, cudaMemcpyDeviceToHost, st));
   AGCN_CUDA(cudaStreamSynchronize(st));
   return AGCN_OK;
 }

@@ -585,40 +585,36 @@ __global__ void big_trans_fold_kernel(TransArgs p) {
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-size_t big_work_floats(const agcn_plan* plan, bool full) {
-  if (plan->large_count == 0) return 0;
-  const size_t ncb = (size_t)(plan->max_n + PT - 1) / PT;
-  size_t f = (size_t)plan->R * ncb + 64;            // rowpart
-  f += (size_t)plan->big_tiles * 8 + 64;            // tilepart
-  f += 2 * ((size_t)plan->B * 4 + 64);              // gstat, stats_tmp
-  f += (size_t)plan->R + 128 + (size_t)plan->B * 256;  // norms + per-graph mean rows (tensor-core pair kernel, F <= 256)
-  if (full) f += 2 * (size_t)plan->R + (size_t)plan->LL + 192;  // dd, rs, C
-  return f;
-}
-
 namespace {
 struct BigWork {
   float *rowpart, *tilepart, *gstat, *stats_tmp, *norms, *dd, *rs, *C;
   int ncb;
+  size_t bytes;
 };
 BigWork carve_big(const agcn_plan* plan, float* base, bool full) {
+  Arena c(base);
   BigWork w{};
   w.ncb = (plan->max_n + PT - 1) / PT;
-  auto r64 = [](size_t x) { return (x + 63) & ~(size_t)63; };
-  size_t off = 0;
-  w.rowpart = base + off; off += r64((size_t)plan->R * w.ncb);
-  w.tilepart = base + off; off += r64((size_t)plan->big_tiles * 8);
-  w.gstat = base + off; off += r64((size_t)plan->B * 4);
-  w.stats_tmp = base + off; off += r64((size_t)plan->B * 4);
-  w.norms = base + off; off += r64((size_t)plan->R) + r64((size_t)plan->B * 256);
+  w.rowpart = c.take((size_t)plan->R * w.ncb);
+  w.tilepart = c.take((size_t)plan->big_tiles * 8);
+  w.gstat = c.take((size_t)plan->B * 4);
+  w.stats_tmp = c.take((size_t)plan->B * 4);
+  w.norms = c.take((size_t)plan->R);
+  c.take((size_t)plan->B * 256);  // per-graph mean rows behind the norms (tensor-core pair kernel, F <= 256)
   if (full) {
-    w.dd = base + off; off += r64((size_t)plan->R);
-    w.rs = base + off; off += r64((size_t)plan->R);
-    w.C = base + off; off += r64((size_t)plan->LL);
+    w.dd = c.take((size_t)plan->R);
+    w.rs = c.take((size_t)plan->R);
+    w.C = c.take((size_t)plan->LL);
   }
+  w.bytes = c.bytes;
   return w;
 }
 }  // namespace
+
+size_t big_work_floats(const agcn_plan* plan, bool full) {
+  if (plan->large_count == 0) return 0;
+  return carve_big(plan, nullptr, full).bytes / sizeof(float);
+}
 
 int big_build_laplacian(const GraphArgs& a, bool need_W, float* big_work, cudaStream_t st) {
   const agcn_plan* plan = a.plan;

@@ -127,13 +127,17 @@ __global__ void copy_pitched_kernel(const float* __restrict__ src, int lds, floa
 // Single-task multi-class head (SingletaskGraphClassifier: models/tf_modules/singletask_classifier.py:124-151 with
 // get_loss_fn('softmax_cross_entropy'), multitask_classifier.py:45-48): one warp per sample,
 //   loss_b = w_b * sum_c y_c (logsumexp(x) - x_c),   d loss / d x_c = w_b (softmax_c * sum y - y_c) * scale
-// `logits` [B, ld] is overwritten by the gradient; part[b] receives loss_b * scale.
-__global__ void softmax_ce_kernel(float* __restrict__ logits, int ld, const float* __restrict__ y, const float* __restrict__ w,
-                                  int B, int C, float scale, float* __restrict__ part) {
+// GRAD (training): `logits` [B, ld] is overwritten by the gradient.  Otherwise (prediction) probs[b, :] = softmax(x_b)
+// = exp(x_b - logsumexp(x_b)), and y may be NULL.  With y, part[b] receives loss_b * scale: one expression for both
+// calls, so the evaluation loss is bit-identical to the training loss.
+template <bool GRAD>
+__global__ void softmax_ce_kernel(float* __restrict__ logits, int ld, const float* __restrict__ y,
+                                  const float* __restrict__ w, int B, int C, float scale, float* __restrict__ probs,
+                                  float* __restrict__ part) {
   const int b = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (b >= B) return;
   float* x = logits + (int64_t)b * ld;
-  const float* yb = y + (int64_t)b * C;
+  const float* yb = y ? y + (int64_t)b * C : nullptr;
   float mx = -INFINITY;
   for (int c = lane; c < C; c += 32) mx = fmaxf(mx, x[c]);
 #pragma unroll
@@ -141,38 +145,7 @@ __global__ void softmax_ce_kernel(float* __restrict__ logits, int ld, const floa
   float se = 0.f, sy = 0.f, sxy = 0.f;
   for (int c = lane; c < C; c += 32) {
     se += expf(x[c] - mx);
-    sy += yb[c];
-    sxy += yb[c] * x[c];
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    se += __shfl_xor_sync(0xffffffffu, se, o);
-    sy += __shfl_xor_sync(0xffffffffu, sy, o);
-    sxy += __shfl_xor_sync(0xffffffffu, sxy, o);
-  }
-  const float lse = mx + logf(se), wb = w[b];
-  for (int c = lane; c < C; c += 32) x[c] = wb * (expf(x[c] - lse) * sy - yb[c]) * scale;
-  if (lane == 0) part[b] = wb * (lse * sy - sxy) * scale;
-}
-
-// Prediction side of the same head (agcn_head_predict): probs[b, :] = softmax(x_b) = exp(x_b - logsumexp(x_b)), one warp
-// per sample.  With targets, part[b] receives the loss term of softmax_ce_kernel, evaluated by the same expressions in
-// the same order, so that the summed loss is bit-identical to the training step's.
-__global__ void softmax_predict_kernel(const float* __restrict__ logits, int ld, const float* __restrict__ y,
-                                       const float* __restrict__ w, int B, int C, float scale, float* __restrict__ probs,
-                                       float* __restrict__ part) {
-  const int b = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-  if (b >= B) return;
-  const float* x = logits + (int64_t)b * ld;
-  float mx = -INFINITY;
-  for (int c = lane; c < C; c += 32) mx = fmaxf(mx, x[c]);
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-  float se = 0.f, sy = 0.f, sxy = 0.f;
-  for (int c = lane; c < C; c += 32) se += expf(x[c] - mx);
-  if (y) {
-    const float* yb = y + (int64_t)b * C;
-    for (int c = lane; c < C; c += 32) {
+    if (GRAD || yb) {
       sy += yb[c];
       sxy += yb[c] * x[c];
     }
@@ -184,12 +157,14 @@ __global__ void softmax_predict_kernel(const float* __restrict__ logits, int ld,
     sxy += __shfl_xor_sync(0xffffffffu, sxy, o);
   }
   const float lse = mx + logf(se);
-  float* pb = probs + (int64_t)b * C;
-  for (int c = lane; c < C; c += 32) pb[c] = expf(x[c] - lse);
-  if (y && lane == 0) {
+  if (GRAD) {
     const float wb = w[b];
-    part[b] = wb * (lse * sy - sxy) * scale;
+    for (int c = lane; c < C; c += 32) x[c] = wb * (expf(x[c] - lse) * sy - yb[c]) * scale;
+  } else {
+    float* pb = probs + (int64_t)b * C;
+    for (int c = lane; c < C; c += 32) pb[c] = expf(x[c] - lse);
   }
+  if (yb && lane == 0) part[b] = w[b] * (lse * sy - sxy) * scale;
 }
 
 __global__ void sum_parts_kernel(const float* __restrict__ parts, int n, float* __restrict__ out) {
@@ -216,77 +191,204 @@ size_t tn_any_partial(const GemmTNArgs& t) {
   return std::max(tc_gemm_tn_partial_floats(t), gemm_tn_partial_floats(t.M, t.Kd, t.N, t.S));
 }
 
-inline size_t al256(size_t x) { return (x + 255) & ~(size_t)255; }
 inline int pad4(int x) { return (x + 3) & ~3; }
 
+// The forward areas come first: they are agcn_head_predict's whole work area, and training adds its backward areas
+// behind them.
 struct HeadWork {
-  float *hsum, *pre, *mol, *dlog, *dmol, *dhsum, *dWh_pad, *loss_part, *tcA, *tcB, *tcC, *tcD, *tn_part, *splitk;
+  float *hsum, *pre, *mol, *dlog, *loss_part, *tcB;
+  float *dmol, *dhsum, *dWh_pad, *tcC, *tcD, *tn_part, *splitk;
   size_t bytes;
 };
 
-HeadWork carve_head(const agcn_plan* plan, int Fh, int Fm, int Nt, void* base) {
-  char* b = reinterpret_cast<char*>(base);
-  size_t off = 0;
-  auto take = [&](size_t floats) {
-    float* r = b ? reinterpret_cast<float*>(b + off) : nullptr;
-    off += al256(floats * sizeof(float));
-    return r;
-  };
+HeadWork carve_head(const agcn_plan* plan, int Fh, int Fm, int Nt, bool train, void* base) {
+  Arena c(base);
   const size_t B = plan->B;
   const int Ntp = pad4(Nt);
   HeadWork w{};
-  w.hsum = take(B * Fh);
-  w.pre = take(B * Fm);
-  w.mol = take(B * Fm);
-  w.dlog = take(B * Ntp);        // d loss / d logits, row pitch Ntp (pad columns stay zero)
-  w.dmol = take(B * Fm);
-  w.dhsum = take(B * Fh);
-  w.dWh_pad = take((size_t)Fm * Ntp);
+  w.hsum = c.take(B * Fh);
+  w.pre = c.take(B * Fm);
+  w.mol = c.take(B * Fm);
+  w.dlog = c.take(B * Ntp);   // row pitch Ntp: d loss / d logits (pad columns stay zero), or the single-task logits
   GemmArgs g;
   g.M = (int)B; g.N = Nt; g.Z = 1; g.prob = 1;  // sized for the tiles of the fused-loss product
-  w.loss_part = take(std::max((size_t)tc_gemm_loss_parts(g), B) + 64);
-  w.tcA = take(tc_gemm_scratch_floats(Fm, Fh, 1, 1));   // dense_W            (pre   = hsum dense_W)
-  w.tcB = take(tc_gemm_scratch_floats(Nt, Fm, 1, 1));   // head_W             (logits = mol head_W)
-  w.tcC = take(tc_gemm_scratch_floats(Fm, Nt, 1, 1));   // head_W^T operand   (dmol  = dlog head_W^T)
-  w.tcD = take(tc_gemm_scratch_floats(Fh, Fm, 1, 1));   // dense_W^T operand  (dhsum = dpre dense_W^T)
-  GemmTNArgs t;
-  t.M = (int)B; t.Kd = std::min(Fm, 128); t.N = Ntp; t.S = 1;
-  size_t tn = tn_any_partial(t);
-  t.Kd = Fh; t.N = Fm;
-  tn = std::max(tn, tn_any_partial(t));
-  w.tn_part = take(tn);
-  w.splitk = take((size_t)8 * B * std::max(Fm, Fh));  // split-K partial sums of the two long contractions
-  w.bytes = off;
+  w.loss_part = c.take(std::max((size_t)tc_gemm_loss_parts(g), B) + 64);
+  w.tcB = c.take(tc_gemm_scratch_floats(Nt, Fm, 1, 1));   // head_W             (logits = mol head_W)
+  if (train) {
+    w.dmol = c.take(B * Fm);
+    w.dhsum = c.take(B * Fh);
+    w.dWh_pad = c.take((size_t)Fm * Ntp);
+    w.tcC = c.take(tc_gemm_scratch_floats(Fm, Nt, 1, 1));   // head_W^T operand   (dmol  = dlog head_W^T)
+    w.tcD = c.take(tc_gemm_scratch_floats(Fh, Fm, 1, 1));   // dense_W^T operand  (dhsum = dpre dense_W^T)
+    GemmTNArgs t;
+    t.M = (int)B; t.Kd = std::min(Fm, 128); t.N = Ntp; t.S = 1;
+    size_t tn = tn_any_partial(t);
+    t.Kd = Fh; t.N = Fm;
+    tn = std::max(tn, tn_any_partial(t));
+    w.tn_part = c.take(tn);
+    w.splitk = c.take((size_t)8 * B * std::max(Fm, Fh));  // split-K partial sums of the two long contractions
+  }
+  w.bytes = c.bytes;
   return w;
 }
 
-// agcn_head_predict's work area: the forward half of carve_head, plus the logits of the single-task head (the
-// multitask head's probabilities come straight out of the logits GEMM's epilogue)
-struct HeadPredictWork {
-  float *hsum, *pre, *mol, *logits, *loss_part, *tcB;
-  size_t bytes;
+// Parameter gradients of agcn_head_loss_grad_ex
+struct HeadGrads {
+  float *dH, *ddense_W, *ddense_b, *dhead_W, *dhead_b;
 };
 
-HeadPredictWork carve_head_predict(const agcn_plan* plan, int Fh, int Fm, int Nt, void* base) {
-  char* b = reinterpret_cast<char*>(base);
-  size_t off = 0;
-  auto take = [&](size_t floats) {
-    float* r = b ? reinterpret_cast<float*>(b + off) : nullptr;
-    off += al256(floats * sizeof(float));
-    return r;
-  };
-  const size_t B = plan->B;
-  HeadPredictWork w{};
-  w.hsum = take(B * Fh);
-  w.pre = take(B * Fm);
-  w.mol = take(B * Fm);
-  w.logits = take(B * pad4(Nt));
-  GemmArgs g;
-  g.M = (int)B; g.N = Nt; g.Z = 1; g.prob = 1;
-  w.loss_part = take(std::max((size_t)tc_gemm_loss_parts(g), B) + 64);
-  w.tcB = take(tc_gemm_scratch_floats(Nt, Fm, 1, 1));
-  w.bytes = off;
-  return w;
+// Both head calls.  The forward runs the same products with the same tile configurations for training (grads set) and
+// prediction (grads NULL): `pre` on the CUDA cores, the logits on the tensor cores with the loss (or the probabilities)
+// in their epilogue, the single-task softmax in softmax_ce_kernel.  The evaluation loss is therefore bit-identical to
+// the training loss.  Prediction writes the probabilities (weighted L2: the values) to d_probs and the loss to d_loss
+// when targets are given; training writes the loss and every gradient.
+int head_run(const char* who, const agcn_plan* plan, const float* d_H, const float* d_dense_W, const float* d_dense_b,
+             const float* d_head_W, const float* d_head_b, const float* d_targets, const float* d_weights, float scale,
+             int32_t loss_kind, int32_t Fh, int32_t Fm, int32_t Nt, float* d_probs, float* d_loss, const HeadGrads* gr,
+             void* d_work, size_t work_bytes, cudaStream_t st) {
+  const std::string at = std::string(who) + ": ";
+  AGCN_REQUIRE(loss_kind == AGCN_LOSS_SIGMOID_CE || loss_kind == AGCN_LOSS_SOFTMAX_CE ||
+                   loss_kind == AGCN_LOSS_WEIGHTED_L2,
+               at + "unknown loss_kind");
+  // the logits GEMM carries the loss epilogue on the tensor cores: its contraction (Fm) must reach one k-block with
+  // 16-byte operand pitches; every other contraction falls back to the CUDA-core kernels when its shape is not
+  // TMA-compatible (e.g. 12 tasks: Nt = 24)
+  AGCN_REQUIRE(Fh >= 1 && Fm >= 32 && Fm % 4 == 0 && Nt >= 1,
+               at + "unsupported sizes (need Fm >= 32 and a multiple of 4)");
+  const bool train = gr != nullptr, softmax = loss_kind == AGCN_LOSS_SOFTMAX_CE;
+  AGCN_REQUIRE(train || loss_kind != AGCN_LOSS_SIGMOID_CE || Nt % 2 == 0,
+               at + "the multitask head needs two logits per task (Nt even)");
+  int rc = plan_use(plan, st);
+  if (rc) return rc;
+  HeadWork w = carve_head(plan, Fh, Fm, Nt, train, d_work);
+  if (w.bytes > work_bytes) {
+    set_error(at + "workspace too small");
+    return AGCN_ERR_WORKSPACE;
+  }
+  const int B = plan->B, Ntp = pad4(Nt);
+  cudaStream_t side = plan->side;
+
+  GemmArgs g_pre, g_log;
+  g_pre.M = B; g_pre.N = Fm; g_pre.Kd = Fh;
+  g_pre.A0 = w.hsum; g_pre.lda0 = Fh;
+  g_pre.B = d_dense_W; g_pre.ldb = Fm;
+  g_pre.C = w.pre; g_pre.ldc = Fm;
+  g_log.M = B; g_log.N = Nt; g_log.Kd = Fm;
+  g_log.A0 = w.mol; g_log.lda0 = Fm;
+  g_log.B = d_head_W; g_log.ldb = Nt;
+  g_log.C = w.dlog; g_log.ldc = Ntp;
+  g_log.bias = d_head_b;
+  if (!softmax) {  // sigmoid cross-entropy or weighted L2: the loss is the GEMM's epilogue
+    g_log.l2 = loss_kind == AGCN_LOSS_WEIGHTED_L2;
+    if (d_targets) {
+      g_log.bce_y = d_targets; g_log.bce_w = d_weights; g_log.bce_ld = Nt; g_log.bce_scale = scale;
+      g_log.loss_part = w.loss_part;
+    }
+    if (!train) {  // C receives the pairwise softmax of the logits (weighted L2: the values x) instead of the gradient
+      g_log.C = d_probs; g_log.ldc = Nt;
+      g_log.prob = 1;
+    }
+  }
+  AGCN_REQUIRE(tc_gemm_supported(g_log), at + "operands are not TMA-compatible (alignment)");
+  GemmArgs g_dmol, g_dhs;
+  g_dmol.M = B; g_dmol.N = Fm; g_dmol.Kd = Nt;
+  g_dmol.A0 = w.dlog; g_dmol.lda0 = Ntp;
+  g_dmol.B = d_head_W; g_dmol.ldb = Nt; g_dmol.transB = 1;  // head_W is [Fm, Nt] = [N, Kd]
+  g_dmol.C = w.dmol; g_dmol.ldc = Fm; g_dmol.split_k_partial = w.splitk;
+  g_dhs.M = B; g_dhs.N = Fh; g_dhs.Kd = Fm;
+  g_dhs.A0 = w.dmol; g_dhs.lda0 = Fm;
+  g_dhs.B = d_dense_W; g_dhs.ldb = Fm; g_dhs.transB = 1;    // dense_W is [Fh, Fm] = [N, Kd]
+  g_dhs.C = w.dhsum; g_dhs.ldc = Fh; g_dhs.split_k_partial = w.splitk;
+  // dhsum = dpre dense_W^T is [B, Fm] x [Fm, Fh] with Fh = 64: eight 128-row tiles of eight k-blocks each -- a latency chain
+  // of 30 us on 8 SMs on the tensor-core kernel, 12 us spread over every SM on the CUDA cores (33 MFLOP)
+  const bool tc_dmol = train && tc_gemm_supported(g_dmol),
+             tc_dhs = train && tc_gemm_supported(g_dhs) && (int64_t)B * Fh * Fm > (1ll << 26);
+
+  // parameter operands (hi / lo split, K-major) on the side stream while the gather runs
+  AGCN_CUDA(cudaEventRecord(plan->ev_side_fork, st));
+  AGCN_CUDA(cudaStreamWaitEvent(side, plan->ev_side_fork, 0));
+  if ((rc = tc_gemm_split_b(g_log, w.tcB, side))) return rc;
+  if (tc_dmol && (rc = tc_gemm_split_b(g_dmol, w.tcC, side))) return rc;
+  if (tc_dhs && (rc = tc_gemm_split_b(g_dhs, w.tcD, side))) return rc;
+  if (train && (rc = zero_async(w.dlog, (size_t)B * Ntp, side))) return rc;  // pad columns of dlog
+  AGCN_CUDA(cudaEventRecord(plan->ev_side_join, side));
+
+  // GraphGatherMol + DenseMol (commuted) + tanh.  `pre` feeds a tanh that the sum over a molecule's atoms saturates:
+  // tanh'(a) = sech^2(a) has relative sensitivity 2 |da|, so the absolute error of this [B, Fh] x [Fh, Fm] product (a
+  // few MFLOP) decides the accuracy of every gradient behind it.  Plain fp32 FMAs (gemm_rows) keep it at fp32 rounding
+  // level; 3xTF32 is ~4x coarser.
+  segment_sum_kernel<<<(B + 7) / 8, 256, 0, st>>>(d_H, plan->d_node_off, B, Fh, w.hsum);
+  AGCN_LAUNCH_CHECK();
+  if ((rc = gemm_rows(g_pre, st))) return rc;
+  {
+    const int64_t total = (int64_t)B * Fm;
+    gather_tanh_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(w.pre, d_dense_b, plan->d_n, B, Fm, w.mol);
+    AGCN_LAUNCH_CHECK();
+  }
+  // logits + loss epilogue: C receives d loss / d logits (training), the probabilities (prediction) or, for the
+  // single-task head, the logits; the loss its per-warp partial sums
+  AGCN_CUDA(cudaStreamWaitEvent(st, plan->ev_side_join, 0));
+  if ((rc = tc_gemm(g_log, w.tcB, st))) return rc;
+  int n_parts = tc_gemm_loss_parts(g_log);
+  if (softmax) {  // softmax cross-entropy row by row
+    (train ? softmax_ce_kernel<true> : softmax_ce_kernel<false>)<<<(B + 7) / 8, 256, 0, st>>>(
+        w.dlog, Ntp, d_targets, d_weights, B, Nt, scale, d_probs, w.loss_part);
+    AGCN_LAUNCH_CHECK();
+    n_parts = B;
+  }
+  if (d_loss) {
+    sum_parts_kernel<<<1, 256, 0, st>>>(w.loss_part, n_parts, d_loss);
+    AGCN_LAUNCH_CHECK();
+  }
+  if (!train) return AGCN_OK;
+
+  // parameter gradients of the heads on the side stream, beside the chain back to dH
+  AGCN_CUDA(cudaEventRecord(plan->ev_side_fork, st));
+  AGCN_CUDA(cudaStreamWaitEvent(side, plan->ev_side_fork, 0));
+  weighted_colsum_kernel<<<(Nt + 31) / 32, 256, 0, side>>>(w.dlog, Ntp, B, Nt, nullptr, gr->dhead_b);
+  AGCN_LAUNCH_CHECK();
+  for (int f0 = 0; f0 < Fm; f0 += 128) {  // dhead_W = mol^T dlog, 128 rows of the result per contraction
+    GemmTNArgs t;
+    t.M = B; t.Kd = std::min(128, Fm - f0); t.N = Ntp; t.S = 1;
+    t.A0 = w.mol + f0; t.lda0 = Fm;
+    t.D = w.dlog; t.ldd = Ntp;
+    t.out = w.dWh_pad + (size_t)f0 * Ntp; t.partial = w.tn_part;
+    if ((rc = tn_any(t, side))) return rc;
+  }
+  {
+    const int64_t total = (int64_t)Fm * Nt;
+    copy_pitched_kernel<<<(unsigned)((total + 255) / 256), 256, 0, side>>>(w.dWh_pad, Ntp, gr->dhead_W, Nt, Fm, Nt);
+    AGCN_LAUNCH_CHECK();
+  }
+
+  // main stream: dmol = dlog head_W^T, through tanh, ddense_b, dhsum, dH
+  auto gemm_any = [&](const GemmArgs& g, const float* scratch, bool tc) { return tc ? tc_gemm(g, scratch, st) : gemm_rows(g, st); };
+  if ((rc = gemm_any(g_dmol, w.tcC, tc_dmol))) return rc;
+  {
+    const int64_t total = (int64_t)B * Fm;
+    tanh_bwd_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(w.pre, w.dmol, total);  // dmol := dpre
+    AGCN_LAUNCH_CHECK();
+  }
+  if ((rc = gemm_any(g_dhs, w.tcD, tc_dhs))) return rc;
+  segment_broadcast_kernel<<<(B + 7) / 8, 256, 0, st>>>(w.dhsum, plan->d_node_off, B, Fh, gr->dH);
+  AGCN_LAUNCH_CHECK();
+  // dense parameter gradients (need dpre; the dhead_W contraction on the side stream is done with tn_part by now
+  // only if we wait for it, so they follow it on the side stream)
+  AGCN_CUDA(cudaEventRecord(plan->ev_fork, st));
+  AGCN_CUDA(cudaStreamWaitEvent(side, plan->ev_fork, 0));
+  weighted_colsum_kernel<<<(Fm + 31) / 32, 256, 0, side>>>(w.dmol, Fm, B, Fm, plan->d_n, gr->ddense_b);
+  AGCN_LAUNCH_CHECK();
+  {
+    GemmTNArgs t;  // ddense_W = hsum^T dpre
+    t.M = B; t.Kd = Fh; t.N = Fm; t.S = 1;
+    t.A0 = w.hsum; t.lda0 = Fh;
+    t.D = w.dmol; t.ldd = Fm;
+    t.out = gr->ddense_W; t.partial = w.tn_part;
+    if ((rc = tn_any(t, side))) return rc;
+  }
+  AGCN_CUDA(cudaEventRecord(plan->ev_side_join, side));
+  AGCN_CUDA(cudaStreamWaitEvent(st, plan->ev_side_join, 0));
+  return AGCN_OK;
 }
 
 }  // namespace
@@ -311,7 +413,7 @@ int agcn_expand_labels(const uint8_t* y, const float* w, int32_t B, int32_t n_ta
 
 int agcn_head_workspace_bytes(const agcn_plan* plan, int32_t Fh, int32_t Fm, int32_t Nt, size_t* bytes) {
   AGCN_REQUIRE(plan && bytes && Fh >= 1 && Fm >= 1 && Nt >= 1, "head_workspace_bytes: bad arguments");
-  *bytes = carve_head(plan, Fh, Fm, Nt, nullptr).bytes + 256;
+  *bytes = carve_head(plan, Fh, Fm, Nt, true, nullptr).bytes + 256;
   return AGCN_OK;
 }
 
@@ -333,141 +435,14 @@ int agcn_head_loss_grad_ex(const agcn_plan* plan, const float* d_H, const float*
   AGCN_REQUIRE(plan && d_H && d_dense_W && d_dense_b && d_head_W && d_head_b && d_targets && d_weights && d_loss &&
                    d_dH && d_ddense_W && d_ddense_b && d_dhead_W && d_dhead_b && d_work,
                "head_loss_grad: null pointer");
-  AGCN_REQUIRE(loss_kind == AGCN_LOSS_SIGMOID_CE || loss_kind == AGCN_LOSS_SOFTMAX_CE ||
-                   loss_kind == AGCN_LOSS_WEIGHTED_L2,
-               "head_loss_grad: unknown loss_kind");
-  // the logits GEMM carries the cross-entropy epilogue on the tensor cores: its contraction (Fm) must reach one
-  // k-block with 16-byte operand pitches; every other contraction falls back to the CUDA-core kernels when its
-  // shape is not TMA-compatible (e.g. 12 tasks: Nt = 24)
-  AGCN_REQUIRE(Fh >= 1 && Fm >= 32 && Fm % 4 == 0 && Nt >= 1,
-               "head_loss_grad: unsupported sizes (need Fm >= 32 and a multiple of 4)");
-  cudaStream_t st = (cudaStream_t)stream;
-  int rc = plan_use(plan, st);
-  if (rc) return rc;
-  HeadWork w = carve_head(plan, Fh, Fm, Nt, d_work);
-  if (w.bytes > work_bytes) {
-    set_error("head_loss_grad: workspace too small");
-    return AGCN_ERR_WORKSPACE;
-  }
-  const int B = plan->B, Ntp = pad4(Nt);
-  const int R = (int)plan->R;
-  (void)R;
-  cudaStream_t side = plan->side;
-
-  // parameter operands (hi / lo split, K-major) on the side stream while the gather runs
-  GemmArgs g_pre, g_log, g_dmol, g_dhs;
-  g_pre.M = B; g_pre.N = Fm; g_pre.Kd = Fh;
-  g_pre.A0 = w.hsum; g_pre.lda0 = Fh;
-  g_pre.B = d_dense_W; g_pre.ldb = Fm;
-  g_pre.C = w.pre; g_pre.ldc = Fm;
-  g_log.M = B; g_log.N = Nt; g_log.Kd = Fm;
-  g_log.A0 = w.mol; g_log.lda0 = Fm;
-  g_log.B = d_head_W; g_log.ldb = Nt;
-  g_log.C = w.dlog; g_log.ldc = Ntp;
-  g_log.bias = d_head_b;
-  const bool softmax = loss_kind == AGCN_LOSS_SOFTMAX_CE;
-  if (!softmax) {  // sigmoid cross-entropy or weighted L2: the loss is the GEMM's epilogue
-    g_log.bce_y = d_targets; g_log.bce_w = d_weights; g_log.bce_ld = Nt; g_log.bce_scale = scale;
-    g_log.loss_part = w.loss_part;
-    g_log.l2 = loss_kind == AGCN_LOSS_WEIGHTED_L2;
-  }
-  g_dmol.M = B; g_dmol.N = Fm; g_dmol.Kd = Nt;
-  g_dmol.A0 = w.dlog; g_dmol.lda0 = Ntp;
-  g_dmol.B = d_head_W; g_dmol.ldb = Nt; g_dmol.transB = 1;  // head_W is [Fm, Nt] = [N, Kd]
-  g_dmol.C = w.dmol; g_dmol.ldc = Fm; g_dmol.split_k_partial = w.splitk;
-  g_dhs.M = B; g_dhs.N = Fh; g_dhs.Kd = Fm;
-  g_dhs.A0 = w.dmol; g_dhs.lda0 = Fm;
-  g_dhs.B = d_dense_W; g_dhs.ldb = Fm; g_dhs.transB = 1;    // dense_W is [Fh, Fm] = [N, Kd]
-  g_dhs.C = w.dhsum; g_dhs.ldc = Fh; g_dhs.split_k_partial = w.splitk;
-  AGCN_REQUIRE(tc_gemm_supported(g_log), "head_loss_grad: operands are not TMA-compatible (alignment)");
-  // `pre` feeds a tanh that the sum over a molecule's atoms saturates: tanh'(a) = sech^2(a) has relative sensitivity
-  // 2 |da|, so the absolute error of this [B, Fh] x [Fh, Fm] product (a few MFLOP) decides the accuracy of every
-  // gradient behind it.  Plain fp32 FMAs (gemm_rows) keep it at fp32 rounding level; 3xTF32 is ~4x coarser.
-  // dhsum = dpre dense_W^T is [B, Fm] x [Fm, Fh] with Fh = 64: eight 128-row tiles of eight k-blocks each -- a latency chain
-  // of 30 us on 8 SMs on the tensor-core kernel, 12 us spread over every SM on the CUDA cores (33 MFLOP)
-  const bool tc_pre = false, tc_dmol = tc_gemm_supported(g_dmol), tc_dhs = tc_gemm_supported(g_dhs) && (int64_t)B * Fh * Fm > (1ll << 26);
-  auto gemm_any = [&](const GemmArgs& g, const float* scratch, bool tc) { return tc ? tc_gemm(g, scratch, st) : gemm_rows(g, st); };
-  AGCN_CUDA(cudaEventRecord(plan->ev_side_fork, st));
-  AGCN_CUDA(cudaStreamWaitEvent(side, plan->ev_side_fork, 0));
-  if (tc_pre && (rc = tc_gemm_split_b(g_pre, w.tcA, side))) return rc;
-  if ((rc = tc_gemm_split_b(g_log, w.tcB, side))) return rc;
-  if (tc_dmol && (rc = tc_gemm_split_b(g_dmol, w.tcC, side))) return rc;
-  if (tc_dhs && (rc = tc_gemm_split_b(g_dhs, w.tcD, side))) return rc;
-  if ((rc = zero_async(w.dlog, (size_t)B * Ntp, side))) return rc;  // pad columns of dlog
-  AGCN_CUDA(cudaEventRecord(plan->ev_side_join, side));
-
-  // GraphGatherMol + DenseMol (commuted) + tanh
-  segment_sum_kernel<<<(B + 7) / 8, 256, 0, st>>>(d_H, plan->d_node_off, B, Fh, w.hsum);
-  AGCN_LAUNCH_CHECK();
-  AGCN_CUDA(cudaStreamWaitEvent(st, plan->ev_side_join, 0));
-  if ((rc = gemm_any(g_pre, w.tcA, tc_pre))) return rc;
-  {
-    const int64_t total = (int64_t)B * Fm;
-    gather_tanh_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(w.pre, d_dense_b, plan->d_n, B, Fm, w.mol);
-    AGCN_LAUNCH_CHECK();
-  }
-  // logits + weighted sigmoid cross-entropy (weighted L2): C receives d loss / d logits, the loss its per-warp partial sums
-  if ((rc = tc_gemm(g_log, w.tcB, st))) return rc;
-  int n_parts = tc_gemm_loss_parts(g_log);
-  if (softmax) {  // the GEMM wrote the logits; softmax cross-entropy and its gradient row by row
-    softmax_ce_kernel<<<(B + 7) / 8, 256, 0, st>>>(w.dlog, Ntp, d_targets, d_weights, B, Nt, scale, w.loss_part);
-    AGCN_LAUNCH_CHECK();
-    n_parts = B;
-  }
-  sum_parts_kernel<<<1, 256, 0, st>>>(w.loss_part, n_parts, d_loss);
-  AGCN_LAUNCH_CHECK();
-
-  // parameter gradients of the heads on the side stream, beside the chain back to dH
-  AGCN_CUDA(cudaEventRecord(plan->ev_side_fork, st));
-  AGCN_CUDA(cudaStreamWaitEvent(side, plan->ev_side_fork, 0));
-  weighted_colsum_kernel<<<(Nt + 31) / 32, 256, 0, side>>>(w.dlog, Ntp, B, Nt, nullptr, d_dhead_b);
-  AGCN_LAUNCH_CHECK();
-  for (int f0 = 0; f0 < Fm; f0 += 128) {  // dhead_W = mol^T dlog, 128 rows of the result per contraction
-    GemmTNArgs t;
-    t.M = B; t.Kd = std::min(128, Fm - f0); t.N = Ntp; t.S = 1;
-    t.A0 = w.mol + f0; t.lda0 = Fm;
-    t.D = w.dlog; t.ldd = Ntp;
-    t.out = w.dWh_pad + (size_t)f0 * Ntp; t.partial = w.tn_part;
-    if ((rc = tn_any(t, side))) return rc;
-  }
-  {
-    const int64_t total = (int64_t)Fm * Nt;
-    copy_pitched_kernel<<<(unsigned)((total + 255) / 256), 256, 0, side>>>(w.dWh_pad, Ntp, d_dhead_W, Nt, Fm, Nt);
-    AGCN_LAUNCH_CHECK();
-  }
-
-  // main stream: dmol = dlog head_W^T, through tanh, ddense_b, dhsum, dH
-  if ((rc = gemm_any(g_dmol, w.tcC, tc_dmol))) return rc;
-  {
-    const int64_t total = (int64_t)B * Fm;
-    tanh_bwd_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(w.pre, w.dmol, total);  // dmol := dpre
-    AGCN_LAUNCH_CHECK();
-  }
-  if ((rc = gemm_any(g_dhs, w.tcD, tc_dhs))) return rc;
-  segment_broadcast_kernel<<<(B + 7) / 8, 256, 0, st>>>(w.dhsum, plan->d_node_off, B, Fh, d_dH);
-  AGCN_LAUNCH_CHECK();
-  // dense parameter gradients (need dpre; the dhead_W contraction on the side stream is done with tn_part by now
-  // only if we wait for it, so they follow it on the side stream)
-  AGCN_CUDA(cudaEventRecord(plan->ev_fork, st));
-  AGCN_CUDA(cudaStreamWaitEvent(side, plan->ev_fork, 0));
-  weighted_colsum_kernel<<<(Fm + 31) / 32, 256, 0, side>>>(w.dmol, Fm, B, Fm, plan->d_n, d_ddense_b);
-  AGCN_LAUNCH_CHECK();
-  {
-    GemmTNArgs t;  // ddense_W = hsum^T dpre
-    t.M = B; t.Kd = Fh; t.N = Fm; t.S = 1;
-    t.A0 = w.hsum; t.lda0 = Fh;
-    t.D = w.dmol; t.ldd = Fm;
-    t.out = d_ddense_W; t.partial = w.tn_part;
-    if ((rc = tn_any(t, side))) return rc;
-  }
-  AGCN_CUDA(cudaEventRecord(plan->ev_side_join, side));
-  AGCN_CUDA(cudaStreamWaitEvent(st, plan->ev_side_join, 0));
-  return AGCN_OK;
+  const HeadGrads gr{d_dH, d_ddense_W, d_ddense_b, d_dhead_W, d_dhead_b};
+  return head_run("head_loss_grad", plan, d_H, d_dense_W, d_dense_b, d_head_W, d_head_b, d_targets, d_weights, scale,
+                  loss_kind, Fh, Fm, Nt, nullptr, d_loss, &gr, d_work, work_bytes, (cudaStream_t)stream);
 }
 
 int agcn_head_predict_workspace_bytes(const agcn_plan* plan, int32_t Fh, int32_t Fm, int32_t Nt, size_t* bytes) {
   AGCN_REQUIRE(plan && bytes && Fh >= 1 && Fm >= 1 && Nt >= 1, "head_predict_workspace_bytes: bad arguments");
-  *bytes = carve_head_predict(plan, Fh, Fm, Nt, nullptr).bytes + 256;
+  *bytes = carve_head(plan, Fh, Fm, Nt, false, nullptr).bytes + 256;
   return AGCN_OK;
 }
 
@@ -479,75 +454,8 @@ int agcn_head_predict(const agcn_plan* plan, const float* d_H, const float* d_de
                "head_predict: d_targets, d_weights and d_loss must be all NULL or all set");
   AGCN_REQUIRE(plan && d_H && d_dense_W && d_dense_b && d_head_W && d_head_b && d_probs && d_work,
                "head_predict: null pointer");
-  AGCN_REQUIRE(loss_kind == AGCN_LOSS_SIGMOID_CE || loss_kind == AGCN_LOSS_SOFTMAX_CE ||
-                   loss_kind == AGCN_LOSS_WEIGHTED_L2,
-               "head_predict: unknown loss_kind");
-  AGCN_REQUIRE(Fh >= 1 && Fm >= 32 && Fm % 4 == 0 && Nt >= 1,
-               "head_predict: unsupported sizes (need Fm >= 32 and a multiple of 4)");
-  const bool sigmoid = loss_kind == AGCN_LOSS_SIGMOID_CE, softmax = loss_kind == AGCN_LOSS_SOFTMAX_CE;
-  AGCN_REQUIRE(!sigmoid || Nt % 2 == 0, "head_predict: the multitask head needs two logits per task (Nt even)");
-  cudaStream_t st = (cudaStream_t)stream;
-  int rc = plan_use(plan, st);
-  if (rc) return rc;
-  HeadPredictWork w = carve_head_predict(plan, Fh, Fm, Nt, d_work);
-  if (w.bytes > work_bytes) {
-    set_error("head_predict: workspace too small");
-    return AGCN_ERR_WORKSPACE;
-  }
-  const int B = plan->B, Ntp = pad4(Nt);
-  cudaStream_t side = plan->side;
-
-  // The products of agcn_head_loss_grad_ex with the same operands and the same tile configuration (the loss, when
-  // asked for, must be bit-identical to the training step's): `pre` on the CUDA cores, the logits on the tensor cores.
-  GemmArgs g_pre, g_log;
-  g_pre.M = B; g_pre.N = Fm; g_pre.Kd = Fh;
-  g_pre.A0 = w.hsum; g_pre.lda0 = Fh;
-  g_pre.B = d_dense_W; g_pre.ldb = Fm;
-  g_pre.C = w.pre; g_pre.ldc = Fm;
-  g_log.M = B; g_log.N = Nt; g_log.Kd = Fm;
-  g_log.A0 = w.mol; g_log.lda0 = Fm;
-  g_log.B = d_head_W; g_log.ldb = Nt;
-  g_log.bias = d_head_b;
-  if (!softmax) {  // pairwise softmax epilogue: probabilities straight to d_probs (weighted L2: the values x)
-    g_log.C = d_probs; g_log.ldc = Nt;
-    g_log.prob = 1;
-    g_log.l2 = loss_kind == AGCN_LOSS_WEIGHTED_L2;
-    if (d_targets) {
-      g_log.bce_y = d_targets; g_log.bce_w = d_weights; g_log.bce_ld = Nt; g_log.bce_scale = scale;
-      g_log.loss_part = w.loss_part;
-    }
-  } else {
-    g_log.C = w.logits; g_log.ldc = Ntp;
-  }
-  AGCN_REQUIRE(tc_gemm_supported(g_log), "head_predict: operands are not TMA-compatible (alignment)");
-  AGCN_CUDA(cudaEventRecord(plan->ev_side_fork, st));
-  AGCN_CUDA(cudaStreamWaitEvent(side, plan->ev_side_fork, 0));
-  if ((rc = tc_gemm_split_b(g_log, w.tcB, side))) return rc;
-  AGCN_CUDA(cudaEventRecord(plan->ev_side_join, side));
-
-  // GraphGatherMol + DenseMol (commuted) + tanh
-  segment_sum_kernel<<<(B + 7) / 8, 256, 0, st>>>(d_H, plan->d_node_off, B, Fh, w.hsum);
-  AGCN_LAUNCH_CHECK();
-  if ((rc = gemm_rows(g_pre, st))) return rc;
-  {
-    const int64_t total = (int64_t)B * Fm;
-    gather_tanh_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(w.pre, d_dense_b, plan->d_n, B, Fm, w.mol);
-    AGCN_LAUNCH_CHECK();
-  }
-  AGCN_CUDA(cudaStreamWaitEvent(st, plan->ev_side_join, 0));
-  if ((rc = tc_gemm(g_log, w.tcB, st))) return rc;
-  int n_parts = tc_gemm_loss_parts(g_log);
-  if (softmax) {
-    softmax_predict_kernel<<<(B + 7) / 8, 256, 0, st>>>(w.logits, Ntp, d_targets, d_weights, B, Nt, scale, d_probs,
-                                                         w.loss_part);
-    AGCN_LAUNCH_CHECK();
-    n_parts = B;
-  }
-  if (d_loss) {
-    sum_parts_kernel<<<1, 256, 0, st>>>(w.loss_part, n_parts, d_loss);
-    AGCN_LAUNCH_CHECK();
-  }
-  return AGCN_OK;
+  return head_run("head_predict", plan, d_H, d_dense_W, d_dense_b, d_head_W, d_head_b, d_targets, d_weights, scale,
+                  loss_kind, Fh, Fm, Nt, d_probs, d_loss, nullptr, d_work, work_bytes, (cudaStream_t)stream);
 }
 
 }  // extern "C"

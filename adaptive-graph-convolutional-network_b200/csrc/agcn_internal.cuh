@@ -382,6 +382,22 @@ class ProfScope {
 };
 
 // ---------------------------------------------------------------- helpers
+// Bump allocator of every workspace layout: each area starts at a multiple of 256 bytes from the base.  With a null
+// base every area is nullptr and `bytes` ends as what the same sequence of areas needs, so a *_workspace_bytes function
+// runs the carve of its call.
+struct Arena {
+  char* base;
+  size_t bytes = 0;
+  explicit Arena(void* p) : base(static_cast<char*>(p)) {}
+  void* area(size_t n) {
+    void* r = base ? base + bytes : nullptr;
+    bytes += (n + 255) & ~(size_t)255;
+    return r;
+  }
+  template <typename T = float>
+  T* take(size_t count) { return static_cast<T*>(area(count * sizeof(T))); }
+};
+
 int zero_async(float* dst, size_t floats, cudaStream_t st);  // zero fill by a kernel (never the copy engine)
 int plan_use(const agcn_plan* plan, cudaStream_t st);  // call first in every entry point that enqueues work
 int fork_streams(const agcn_plan* plan, cudaStream_t main, int n_aux);

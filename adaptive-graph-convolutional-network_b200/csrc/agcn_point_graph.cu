@@ -197,21 +197,15 @@ struct Work {
 };
 
 static Work carve(const agcn_plan* plan, void* base) {
-  char* b = reinterpret_cast<char*>(base);
-  size_t off = 0;
-  auto take = [&](size_t bytes) {
-    char* r = b ? b + off : nullptr;
-    off += (bytes + 255) & ~(size_t)255;
-    return r;
-  };
+  Arena c(base);
   Work w{};
-  w.rowpart = reinterpret_cast<double*>(take((size_t)plan->R * 8));
-  w.dinv = reinterpret_cast<double*>(take((size_t)plan->R * 8));
-  w.q = reinterpret_cast<double*>(take((size_t)plan->R * 8));
-  w.dlim = reinterpret_cast<float*>(take((size_t)plan->B * 4));
-  w.hist = reinterpret_cast<uint32_t*>(take((size_t)plan->B * 256 * 4));
-  w.sel = reinterpret_cast<uint32_t*>(take((size_t)plan->B * 8));
-  w.bytes = off;
+  w.rowpart = c.take<double>(plan->R);
+  w.dinv = c.take<double>(plan->R);
+  w.q = c.take<double>(plan->R);
+  w.dlim = c.take((size_t)plan->B);
+  w.hist = c.take<uint32_t>((size_t)plan->B * 256);
+  w.sel = c.take<uint32_t>((size_t)plan->B * 2);
+  w.bytes = c.bytes;
   return w;
 }
 

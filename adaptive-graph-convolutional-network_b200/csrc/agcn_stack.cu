@@ -70,8 +70,6 @@ __global__ void __launch_bounds__(256) act_grad_kernel(const float* __restrict__
 
 namespace {
 
-inline size_t al256(size_t x) { return (x + 255) & ~(size_t)255; }
-
 bool is_reslap(const agcn_stack_node& n) {
   return n.kind == AGCN_NODE_SGCLL && n.desc.variant == AGCN_VARIANT_SGC_LL_RESLAP;
 }
@@ -84,22 +82,33 @@ agcn_sgcll_desc forward_only(const agcn_sgcll_desc& d) {
   return f;
 }
 
-// scratch of a BlockEnd's products: agcn_node_gemm forward / dX (sized as functional._NodeLinear sizes it) and the TN dW
-size_t block_end_work(const agcn_sgcll_desc& d, const agcn_plan* plan) {
+// `saved` and scratch bytes of node i's forward (train) or forward-only call; a BlockEnd saves nothing, its scratch
+// serves agcn_node_gemm forward / dX (sized as functional._NodeLinear sizes it) and the TN dW
+int node_bytes(const agcn_stack_node& nd, const agcn_plan* plan, bool train, size_t* saved, size_t* work) {
+  const agcn_sgcll_desc& d = nd.desc;
+  *saved = 0;
+  if (nd.kind == AGCN_NODE_SGCLL) {
+    const agcn_sgcll_desc f = train ? d : forward_only(d);
+    return agcn_sgcll_workspace_bytes(&f, plan, saved, work);
+  }
   const int m = std::max(d.F, d.Fo);
-  return std::max(agcn_node_gemm_scratch_bytes(m, m), agcn_gemm_tn_scratch_bytes((int32_t)plan->R, d.F, d.Fo, 1));
+  *work = std::max(agcn_node_gemm_scratch_bytes(m, m), agcn_gemm_tn_scratch_bytes((int32_t)plan->R, d.F, d.Fo, 1));
+  return AGCN_OK;
 }
 
+// Where the forward walk finds node i's output, L_all and `saved` area, and the scratch of the layer and head calls.
+// Training gives every node areas of its own; prediction points the nodes at reused slots and one shared `saved` area.
 struct StackWork {
   std::vector<float*> H;      // activated output of node i, [R, Fo_i]
-  std::vector<void*> saved;   // forward -> backward area of SGC-LL node i
-  float* dA = nullptr;        // gradient ping-pong buffers [R, maxF]
-  float* dB = nullptr;
+  std::vector<float*> Lall;   // Reslap node i: its L_all [sum n^2]
+  std::vector<void*> saved;   // SGC-LL node i: its forward -> backward area (prediction: forward scratch)
   void* layer_work = nullptr;
   size_t layer_work_bytes = 0;
   void* head_work = nullptr;
   size_t head_work_bytes = 0;
-  std::vector<float*> Lall;   // Reslap node i: its L_all [sum n^2]
+  // training only
+  float* dA = nullptr;        // gradient ping-pong buffers [R, maxF]
+  float* dB = nullptr;
   std::vector<float*> dLall;  // Reslap node i with a consumer: gradient into L_all[i] [sum n^2]
   std::vector<float*> dpre;   // BlockEnd node i: dY * act'(Y) [R, Fo_i], alive until its dX product has run
   size_t bytes = 0;
@@ -108,53 +117,40 @@ struct StackWork {
 // A plain SGC_LL stack (agcn_stack_create) carves exactly the areas it always had, in the same order; the Reslap and
 // BlockEnd areas come after them.
 int carve_stack(const agcn_stack* s, const agcn_plan* plan, void* base, StackWork* w) {
-  char* b = reinterpret_cast<char*>(base);
-  size_t off = 0;
-  auto take = [&](size_t bytes) {
-    void* r = b ? b + off : nullptr;
-    off += al256(bytes);
-    return r;
-  };
+  Arena c(base);
   const size_t R = (size_t)plan->R, LL = (size_t)plan->LL;
   const int n = (int)s->nodes.size();
   int maxF = 0;
   size_t work_max = 0;
   for (const agcn_stack_node& nd : s->nodes) {
-    const agcn_sgcll_desc& d = nd.desc;
     size_t saved = 0, work = 0;
-    if (nd.kind == AGCN_NODE_SGCLL) {
-      int rc = agcn_sgcll_workspace_bytes(&d, plan, &saved, &work);
-      if (rc) return rc;
-    } else {
-      work = block_end_work(d, plan);
-    }
-    w->H.push_back(reinterpret_cast<float*>(take(R * d.Fo * sizeof(float))));
-    w->saved.push_back(nd.kind == AGCN_NODE_SGCLL ? take(saved) : nullptr);
+    int rc = node_bytes(nd, plan, true, &saved, &work);
+    if (rc) return rc;
+    w->H.push_back(c.take(R * nd.desc.Fo));
+    w->saved.push_back(nd.kind == AGCN_NODE_SGCLL ? c.area(saved) : nullptr);
     work_max = std::max(work_max, work);
-    maxF = std::max(maxF, std::max(d.F, d.Fo));
+    maxF = std::max(maxF, std::max(nd.desc.F, nd.desc.Fo));
   }
-  w->dA = reinterpret_cast<float*>(take(R * maxF * sizeof(float)));
-  w->dB = reinterpret_cast<float*>(take(R * maxF * sizeof(float)));
+  w->dA = c.take(R * maxF);
+  w->dB = c.take(R * maxF);
   w->layer_work_bytes = work_max;
-  w->layer_work = take(work_max);
-  size_t hb = 0;
-  int rc = agcn_head_workspace_bytes(plan, s->nodes.back().desc.Fo, s->Fm, s->Nt, &hb);
+  w->layer_work = c.area(work_max);
+  int rc = agcn_head_workspace_bytes(plan, s->nodes.back().desc.Fo, s->Fm, s->Nt, &w->head_work_bytes);
   if (rc) return rc;
-  w->head_work_bytes = hb;
-  w->head_work = take(hb);
+  w->head_work = c.area(w->head_work_bytes);
   w->Lall.assign(n, nullptr);
   w->dLall.assign(n, nullptr);
   w->dpre.assign(n, nullptr);
   for (int i = 0; i < n; ++i) {
     const agcn_stack_node& nd = s->nodes[i];
     if (is_reslap(nd)) {
-      w->Lall[i] = reinterpret_cast<float*>(take(LL * sizeof(float)));
-      if (s->lall_user[i] >= 0) w->dLall[i] = reinterpret_cast<float*>(take(LL * sizeof(float)));
+      w->Lall[i] = c.take(LL);
+      if (s->lall_user[i] >= 0) w->dLall[i] = c.take(LL);
     } else if (nd.kind == AGCN_NODE_BLOCK_END) {
-      w->dpre[i] = reinterpret_cast<float*>(take(R * nd.desc.Fo * sizeof(float)));
+      w->dpre[i] = c.take(R * nd.desc.Fo);
     }
   }
-  w->bytes = off;
+  w->bytes = c.bytes;
   return AGCN_OK;
 }
 
@@ -162,52 +158,36 @@ int carve_stack(const agcn_stack* s, const agcn_plan* plan, void* base, StackWor
 // AGCN_SAVE_FOR_BACKWARD; it is their forward scratch), and the activations and L_all matrices live in slots that are
 // reused as soon as their last reader has run (agcn_stack_create_nodes assigns them).  A plain SGC_LL stack gets two
 // activation slots, used alternately, and no L_all slot.
-struct PredictWork {
-  std::vector<float*> H;      // activation slots [R, max Fo]
-  std::vector<float*> L;      // L_all slots [sum n^2]
-  void* saved = nullptr;
-  void* layer_work = nullptr;
-  size_t layer_work_bytes = 0;
-  void* head_work = nullptr;
-  size_t head_work_bytes = 0;
-  size_t bytes = 0;
-};
-
-int carve_predict(const agcn_stack* s, const agcn_plan* plan, void* base, PredictWork* w) {
-  char* b = reinterpret_cast<char*>(base);
-  size_t off = 0;
-  auto take = [&](size_t bytes) {
-    void* r = b ? b + off : nullptr;
-    off += al256(bytes);
-    return r;
-  };
+int carve_predict(const agcn_stack* s, const agcn_plan* plan, void* base, StackWork* w) {
+  Arena c(base);
   const size_t R = (size_t)plan->R;
+  const int n = (int)s->nodes.size();
   int maxFo = 0;
   size_t saved_max = 0, work_max = 0;
   for (const agcn_stack_node& nd : s->nodes) {
     size_t saved = 0, work = 0;
-    if (nd.kind == AGCN_NODE_SGCLL) {
-      const agcn_sgcll_desc f = forward_only(nd.desc);
-      int rc = agcn_sgcll_workspace_bytes(&f, plan, &saved, &work);
-      if (rc) return rc;
-    } else {
-      work = block_end_work(nd.desc, plan);
-    }
+    int rc = node_bytes(nd, plan, false, &saved, &work);
+    if (rc) return rc;
     saved_max = std::max(saved_max, saved);
     work_max = std::max(work_max, work);
     maxFo = std::max(maxFo, nd.desc.Fo);
   }
-  for (int k = 0; k < s->n_pred_h; ++k) w->H.push_back(reinterpret_cast<float*>(take(R * maxFo * sizeof(float))));
-  w->saved = take(saved_max);
+  std::vector<float*> h_slot, l_slot;
+  for (int k = 0; k < s->n_pred_h; ++k) h_slot.push_back(c.take(R * maxFo));
+  void* saved = c.area(saved_max);
   w->layer_work_bytes = work_max;
-  w->layer_work = take(work_max);
-  size_t hb = 0;
-  int rc = agcn_head_predict_workspace_bytes(plan, s->nodes.back().desc.Fo, s->Fm, s->Nt, &hb);
+  w->layer_work = c.area(work_max);
+  int rc = agcn_head_predict_workspace_bytes(plan, s->nodes.back().desc.Fo, s->Fm, s->Nt, &w->head_work_bytes);
   if (rc) return rc;
-  w->head_work_bytes = hb;
-  w->head_work = take(hb);
-  for (int k = 0; k < s->n_pred_l; ++k) w->L.push_back(reinterpret_cast<float*>(take((size_t)plan->LL * sizeof(float))));
-  w->bytes = off;
+  w->head_work = c.area(w->head_work_bytes);
+  for (int k = 0; k < s->n_pred_l; ++k) l_slot.push_back(c.take((size_t)plan->LL));
+  for (int i = 0; i < n; ++i) {
+    const bool sgcll = s->nodes[i].kind == AGCN_NODE_SGCLL;
+    w->H.push_back(h_slot[s->pred_h[i]]);
+    w->Lall.push_back(s->pred_l[i] >= 0 ? l_slot[s->pred_l[i]] : nullptr);
+    w->saved.push_back(sgcll ? saved : nullptr);
+  }
+  w->bytes = c.bytes;
   return AGCN_OK;
 }
 
@@ -235,6 +215,36 @@ int block_end_forward(const agcn_sgcll_desc& d, const agcn_plan* plan, const flo
   const int32_t R = (int32_t)plan->R;
   AGCN_CUDA(cudaMemcpyAsync(out, x, (size_t)R * d.Fo * sizeof(float), cudaMemcpyDeviceToDevice, st));
   return agcn_node_gemm(x_res, d.F, W, d.Fo, 0, out, d.Fo, R, d.Fo, d.F, nullptr, nullptr, 1, d.activation, work, st);
+}
+
+// tensor k of node l's parameters (k: weight, bias, M_L, alpha, beta) in a flat buffer, NULL when the node has none
+template <typename T>
+T* node_param(const agcn_stack* s, T* flat, int l, int k) {
+  const int64_t o = s->off[5 * (size_t)l + k];
+  return o >= 0 ? flat + o : nullptr;
+}
+
+// The forward of every node (graphconv.py:85-125 / graphconv_reslap.py:45-89 per layer, blockend.py:67-86 per
+// BlockEnd) into the areas `w` names for it; train: the layers save what their backward needs.
+int forward_nodes(const agcn_stack* s, const agcn_plan* plan, const StackWork& w, const float* d_X, const float* d_Lint,
+                  const float* d_params, bool train, void* stream) {
+  const float* x = d_X;
+  for (int l = 0; l < (int)s->nodes.size(); ++l) {
+    const agcn_stack_node& nd = s->nodes[l];
+    const agcn_sgcll_desc d = train ? nd.desc : forward_only(nd.desc);
+    auto P = [&](int k) { return node_param(s, d_params, l, k); };
+    int rc;
+    if (nd.kind == AGCN_NODE_BLOCK_END) {
+      rc = block_end_forward(d, plan, x, w.H[nd.src], P(0), w.H[l], w.layer_work, (cudaStream_t)stream);
+    } else {
+      const float* Lprev = (is_reslap(nd) && nd.src >= 0) ? w.Lall[nd.src] : nullptr;
+      rc = agcn_sgcll_forward(&d, plan, x, d_Lint, Lprev, P(2), P(0), P(1), P(3), P(4), w.H[l], nullptr, nullptr,
+                              w.Lall[l], w.saved[l], w.layer_work, w.layer_work_bytes, stream);
+    }
+    if (rc) return rc;
+    x = w.H[l];
+  }
+  return AGCN_OK;
 }
 
 }  // namespace
@@ -352,24 +362,10 @@ int agcn_stack_loss_grad(const agcn_stack* s, const agcn_plan* plan, const float
   cudaStream_t st = (cudaStream_t)stream;
   const int nl = (int)s->nodes.size();
   const int32_t R = (int32_t)plan->R;
-  auto P = [&](int l, int k) { return s->off[5 * (size_t)l + k] >= 0 ? d_params + s->off[5 * (size_t)l + k] : nullptr; };
-  auto G = [&](int l, int k) { return s->off[5 * (size_t)l + k] >= 0 ? d_grads + s->off[5 * (size_t)l + k] : nullptr; };
+  auto P = [&](int l, int k) { return node_param(s, d_params, l, k); };
+  auto G = [&](int l, int k) { return node_param(s, d_grads, l, k); };
   const int64_t* ho = &s->off[5 * (size_t)nl];
-  // ---- forward (graphconv.py:85-125 / graphconv_reslap.py:45-89 per layer, blockend.py:67-86 per BlockEnd)
-  const float* x = d_X;
-  for (int l = 0; l < nl; ++l) {
-    const agcn_stack_node& nd = s->nodes[l];
-    const agcn_sgcll_desc& d = nd.desc;
-    if (nd.kind == AGCN_NODE_BLOCK_END) {
-      rc = block_end_forward(d, plan, x, w.H[nd.src], P(l, 0), w.H[l], w.layer_work, st);
-    } else {
-      const float* Lprev = (is_reslap(nd) && nd.src >= 0) ? w.Lall[nd.src] : nullptr;
-      rc = agcn_sgcll_forward(&d, plan, x, d_Lint, Lprev, P(l, 2), P(l, 0), P(l, 1), P(l, 3), P(l, 4), w.H[l], nullptr,
-                              nullptr, w.Lall[l], w.saved[l], w.layer_work, w.layer_work_bytes, stream);
-    }
-    if (rc) return rc;
-    x = w.H[l];
-  }
+  if ((rc = forward_nodes(s, plan, w, d_X, d_Lint, d_params, true, stream))) return rc;
   // ---- DenseMol + GraphGatherMol + logits + loss, with every gradient of that part
   const agcn_sgcll_desc& last = s->nodes[nl - 1].desc;
   rc = agcn_head_loss_grad_ex(plan, w.H[nl - 1], d_params + ho[0], d_params + ho[1], d_params + ho[2], d_params + ho[3],
@@ -427,7 +423,7 @@ int agcn_stack_loss_grad(const agcn_stack* s, const agcn_plan* plan, const float
 
 int agcn_stack_predict_workspace_bytes(const agcn_stack* s, const agcn_plan* plan, size_t* bytes) {
   AGCN_REQUIRE(s && plan && bytes, "stack_predict_workspace_bytes: null pointer");
-  PredictWork w;
+  StackWork w;
   int rc = carve_predict(s, plan, nullptr, &w);
   if (rc) return rc;
   *bytes = w.bytes + 256;
@@ -440,36 +436,19 @@ int agcn_stack_predict(const agcn_stack* s, const agcn_plan* plan, const float* 
   AGCN_REQUIRE(!d_targets == !d_weights && !d_targets == !d_loss,
                "stack_predict: d_targets, d_weights and d_loss must be all NULL or all set");
   AGCN_REQUIRE(s && plan && d_X && d_Lint && d_params && d_probs && d_work, "stack_predict: null pointer");
-  PredictWork w;
+  StackWork w;
   int rc = carve_predict(s, plan, d_work, &w);
   if (rc) return rc;
   if (w.bytes > work_bytes) {
     set_error("stack_predict: workspace too small");
     return AGCN_ERR_WORKSPACE;
   }
+  if ((rc = forward_nodes(s, plan, w, d_X, d_Lint, d_params, false, stream))) return rc;
   const int nl = (int)s->nodes.size();
-  auto P = [&](int l, int k) { return s->off[5 * (size_t)l + k] >= 0 ? d_params + s->off[5 * (size_t)l + k] : nullptr; };
   const int64_t* ho = &s->off[5 * (size_t)nl];
-  const float* x = d_X;
-  for (int l = 0; l < nl; ++l) {
-    const agcn_stack_node& nd = s->nodes[l];
-    const agcn_sgcll_desc d = forward_only(nd.desc);
-    float* out = w.H[s->pred_h[l]];
-    if (nd.kind == AGCN_NODE_BLOCK_END) {
-      rc = block_end_forward(d, plan, x, w.H[s->pred_h[nd.src]], P(l, 0), out, w.layer_work, (cudaStream_t)stream);
-    } else {
-      const bool reslap = is_reslap(nd);
-      const float* Lprev = (reslap && nd.src >= 0) ? w.L[s->pred_l[nd.src]] : nullptr;
-      rc = agcn_sgcll_forward(&d, plan, x, d_Lint, Lprev, P(l, 2), P(l, 0), P(l, 1), P(l, 3), P(l, 4), out, nullptr,
-                              nullptr, reslap ? w.L[s->pred_l[l]] : nullptr, w.saved, w.layer_work,
-                              w.layer_work_bytes, stream);
-    }
-    if (rc) return rc;
-    x = out;
-  }
-  return agcn_head_predict(plan, x, d_params + ho[0], d_params + ho[1], d_params + ho[2], d_params + ho[3], d_targets,
-                           d_weights, scale, s->loss_kind, s->nodes.back().desc.Fo, s->Fm, s->Nt, d_probs, d_loss,
-                           w.head_work, w.head_work_bytes, stream);
+  return agcn_head_predict(plan, w.H[nl - 1], d_params + ho[0], d_params + ho[1], d_params + ho[2], d_params + ho[3],
+                           d_targets, d_weights, scale, s->loss_kind, s->nodes.back().desc.Fo, s->Fm, s->Nt, d_probs,
+                           d_loss, w.head_work, w.head_work_bytes, stream);
 }
 
 int agcn_adam_step(float* d_params, const float* d_grads, float* d_m, float* d_v, int32_t* d_step, int64_t n, float lr,

@@ -163,21 +163,29 @@ class SimpleAGCNStep(object):
             self.grads.all_reduce()
 
     # ---- engines --------------------------------------------------------------------------------------------
-    def _ensure_arena(self, batch):
+    def _ensure_arena(self, batch, predict=False):
+        """The device arena of agcn_stack_loss_grad (self._arena) or, predict=True, of agcn_stack_predict
+        (self._pred_arena) for this batch: grown with 25 % headroom when it is too small, reused otherwise."""
+        lib = _lib.lib()
+        size_fn, attr = ((lib.agcn_stack_predict_workspace_bytes, "_pred_arena") if predict else
+                         (lib.agcn_stack_workspace_bytes, "_arena"))
         nbytes = ctypes.c_size_t()
-        _lib.check(_lib.lib().agcn_stack_workspace_bytes(self._stack, batch.handle, ctypes.byref(nbytes)))
-        if self._arena is None or self._arena.numel() < nbytes.value:
-            self._arena = torch.empty(int(nbytes.value * 1.25) + 4096, dtype=torch.uint8, device=self.device)
+        _lib.check(size_fn(self._stack, batch.handle, ctypes.byref(nbytes)))
+        arena = getattr(self, attr)
+        if arena is None or arena.numel() < nbytes.value:
+            arena = torch.empty(int(nbytes.value * 1.25) + 4096, dtype=torch.uint8, device=self.device)
+            setattr(self, attr, arena)
+        return arena
 
     def _loss_grad_stack(self, X, Lint, batch, targets, weights):
         lib = _lib.lib()
-        self._ensure_arena(batch)
+        arena = self._ensure_arena(batch)
         notify = ctypes.cast(self._notify, ctypes.c_void_p) if self.overlap_allreduce else None
         with torch.cuda.device(self.device):
             _lib.check(lib.agcn_stack_loss_grad(
                 self._stack, batch.handle, _ptr(X), _ptr(Lint), _ptr(targets), _ptr(weights),
                 1.0 / self.global_batch, _ptr(self.flat_params.flat), _ptr(self.flat_grad), _ptr(self._loss),
-                _ptr(self._arena), self._arena.numel(), notify, None, _stream_ptr(self.device)))
+                _ptr(arena), arena.numel(), notify, None, _stream_ptr(self.device)))
         return self._loss
 
     def forward_loss(self, X, Lint, batch, targets, weights):
@@ -205,17 +213,14 @@ class SimpleAGCNStep(object):
     # ---- prediction (predict_proba / predict / evaluate of the reference's classifiers and regressor) ------------
     def _predict_stack(self, X, Lint, batch, targets, weights, scale):
         lib = _lib.lib()
-        nbytes = ctypes.c_size_t()
-        _lib.check(lib.agcn_stack_predict_workspace_bytes(self._stack, batch.handle, ctypes.byref(nbytes)))
-        if self._pred_arena is None or self._pred_arena.numel() < nbytes.value:
-            self._pred_arena = torch.empty(int(nbytes.value * 1.25) + 4096, dtype=torch.uint8, device=self.device)
+        arena = self._ensure_arena(batch, predict=True)
         probs = torch.empty(batch.batch_size, self.Nt, device=self.device, dtype=torch.float32)
         loss = torch.empty(1, device=self.device, dtype=torch.float32) if targets is not None else None
         with torch.cuda.device(self.device):
             _lib.check(lib.agcn_stack_predict(
                 self._stack, batch.handle, _ptr(X), _ptr(Lint), _ptr(targets), _ptr(weights),
                 float(scale if scale is not None else 0.0), _ptr(self.flat_params.flat), _ptr(probs), _ptr(loss),
-                _ptr(self._pred_arena), self._pred_arena.numel(), _stream_ptr(self.device)))
+                _ptr(arena), arena.numel(), _stream_ptr(self.device)))
         return probs, (loss.reshape(()) if loss is not None else None)
 
     def _predict(self, X, Lint, batch, targets=None, weights=None, scale=None):
