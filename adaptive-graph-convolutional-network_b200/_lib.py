@@ -14,7 +14,8 @@ VARIANT = {"SGC_LL": 0, "SGC_LL_Reslap": 1}
 LAPLACIAN = {"reference_literal": 0, "paper": 1}
 METRIC_GRAD = {"reference": 0, "full": 1}
 ACT = {"linear": 0, "relu": 1}
-LOSS = {"sigmoid_ce": 0, "softmax_ce": 1, "weighted_l2": 2}
+LOSS = {"sigmoid_ce": 0, "softmax_ce": 1, "weighted_l2": 2}      # the graph heads (AGCN_LOSS_*)
+NODE_LOSS = {"node_softmax_ce": 4}                                 # the per-node head (AGCN_PER_NODE_*)
 ADJ_RULE = {"mean_distance": 0, "cutoff": 1}
 NODE = {"sgcll": 0, "block_end": 1}
 NOTIFY_FN = ctypes.CFUNCTYPE(None, ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p)
@@ -23,6 +24,15 @@ OUT_RES_L, OUT_RES_W, OUT_L_ALL, SAVE_FOR_BACKWARD = 1, 2, 4, 8
 
 class AgcnError(RuntimeError):
     pass
+
+
+def loss_code(name):
+    """The loss_kind value of agcn_stack_create(_nodes) for a loss name of LOSS or NODE_LOSS."""
+    if name in LOSS:
+        return LOSS[name]
+    if name in NODE_LOSS:
+        return NODE_LOSS[name]
+    raise ValueError("loss must be one of %s" % sorted(list(LOSS) + list(NODE_LOSS)))
 
 
 class Desc(ctypes.Structure):
@@ -95,6 +105,14 @@ _SIGNATURES = {
                                                           ctypes.POINTER(ctypes.c_size_t)]),
     "agcn_head_predict": (ctypes.c_int, [_P] * 8 + [ctypes.c_float, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
                                                 ctypes.c_int32] + [_P] * 3 + [ctypes.c_size_t, _P]),
+    "agcn_node_head_workspace_bytes": (ctypes.c_int, [_P, ctypes.c_int32, ctypes.c_int32,
+                                                       ctypes.POINTER(ctypes.c_size_t)]),
+    "agcn_node_head_loss_grad": (ctypes.c_int, [_P] * 6 + [ctypes.c_float, ctypes.c_int32, ctypes.c_int32] + [_P] * 5 +
+                                 [ctypes.c_size_t, _P]),
+    "agcn_node_head_predict_workspace_bytes": (ctypes.c_int, [_P, ctypes.c_int32, ctypes.c_int32,
+                                                               ctypes.POINTER(ctypes.c_size_t)]),
+    "agcn_node_head_predict": (ctypes.c_int, [_P] * 6 + [ctypes.c_float, ctypes.c_int32, ctypes.c_int32] + [_P] * 3 +
+                               [ctypes.c_size_t, _P]),
     "agcn_stack_create": (ctypes.c_int, [_P, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _P,
                                          ctypes.POINTER(_P)]),
     "agcn_stack_create_nodes": (ctypes.c_int, [_P, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _P,

@@ -12,6 +12,10 @@
 // then has B rows instead of R = sum n_g.  The n_tasks heads are one [n_feature, 2 n_tasks] matrix.  Every
 // contraction runs on the tcgen05 3xTF32 GEMMs of agcn_tc_gemm.cu; the cross-entropy (or the weighted L2) and its
 // gradient are the epilogue of the logits GEMM, so the [B, 2 n_tasks] logits never reach HBM as logits.
+//
+// The per-node head (agcn_node_head_*, the part labels of the reference's segmentation network; restated, parity
+// unpinned) has no DenseMol, gather or tanh: logits H head_W + head_b for every packed row, then the single-task head's
+// row softmax over R rows instead of B.
 #include <algorithm>
 
 #include "agcn_internal.cuh"
@@ -247,6 +251,8 @@ int head_run(const char* who, const agcn_plan* plan, const float* d_H, const flo
              int32_t loss_kind, int32_t Fh, int32_t Fm, int32_t Nt, float* d_probs, float* d_loss, const HeadGrads* gr,
              void* d_work, size_t work_bytes, cudaStream_t st) {
   const std::string at = std::string(who) + ": ";
+  AGCN_REQUIRE(loss_kind != AGCN_PER_NODE_SOFTMAX_CE,
+               at + "AGCN_PER_NODE_SOFTMAX_CE is the per-node head: call agcn_node_head_loss_grad / agcn_node_head_predict");
   AGCN_REQUIRE(loss_kind == AGCN_LOSS_SIGMOID_CE || loss_kind == AGCN_LOSS_SOFTMAX_CE ||
                    loss_kind == AGCN_LOSS_WEIGHTED_L2,
                at + "unknown loss_kind");
@@ -391,6 +397,144 @@ int head_run(const char* who, const agcn_plan* plan, const float* d_H, const flo
   return AGCN_OK;
 }
 
+// ---- per-node head (agcn_node_head_*): the logits of every packed row, softmax cross-entropy per row
+
+constexpr int COLSUM_ROWS = 64;  // rows per CTA of colsum_part_kernel
+
+// First stage of dhead_b = colsum(dlog) over the R rows: part[k, c] = sum of M[r, c] over the rows [64 k, 64 k + 64).
+// weighted_colsum_kernel would walk all R rows in each of its (C + 31) / 32 CTAs, a serial chain at R = 32 k; here every
+// CTA sums 64 rows, threads laid out [row lane][column] as act_bwd_colsum_kernel (coalesced, fixed order), and
+// colsum_reduce adds the ceil(R / 64) parts.  Deterministic: no atomics.
+__global__ void __launch_bounds__(256) colsum_part_kernel(const float* __restrict__ M, int ld, int64_t R, int C,
+                                                          float* __restrict__ part) {
+  __shared__ float red[256];
+  const int64_t r0 = (int64_t)blockIdx.x * COLSUM_ROWS, r1 = min(R, r0 + COLSUM_ROWS);
+  const int cols = min(C, 256), lanes = 256 / cols;
+  for (int cbase = 0; cbase < C; cbase += cols) {
+    const int c = cbase + (int)(threadIdx.x % cols), rl = threadIdx.x / cols;
+    float s = 0.f;
+    if (c < C && rl < lanes)
+      for (int64_t r = r0 + rl; r < r1; r += lanes) s += M[r * ld + c];
+    red[threadIdx.x] = s;
+    __syncthreads();
+    if (rl == 0 && c < C) {
+      for (int l = 1; l < lanes; ++l) s += red[l * cols + (threadIdx.x % cols)];
+      part[(int64_t)blockIdx.x * C + c] = s;
+    }
+    __syncthreads();
+  }
+}
+
+int colsum_parts(const agcn_plan* plan) { return (int)((plan->R + COLSUM_ROWS - 1) / COLSUM_ROWS); }
+
+// As carve_head: the forward areas are agcn_node_head_predict's whole work area, training adds its areas behind them.
+struct NodeHeadWork {
+  float *dlog, *loss_part, *tcB;
+  float *tcC, *dWh_pad, *tn_part, *colsum_part;
+  size_t bytes;
+};
+
+NodeHeadWork carve_node_head(const agcn_plan* plan, int Fh, int C, bool train, void* base) {
+  Arena c(base);
+  const size_t R = (size_t)plan->R;
+  const int Cp = pad4(C);
+  NodeHeadWork w{};
+  w.dlog = c.take(R * Cp);   // row pitch Cp: the logits, overwritten by d loss / d logits in training
+  w.loss_part = c.take(R);
+  w.tcB = c.take(tc_gemm_scratch_floats(C, Fh, 1, 1));   // head_W      (logits = H head_W)
+  if (train) {
+    w.tcC = c.take(tc_gemm_scratch_floats(Fh, C, 1, 1));  // head_W^T    (dH = dlog head_W^T)
+    w.dWh_pad = c.take((size_t)Fh * Cp);
+    GemmTNArgs t;
+    t.M = (int)R; t.Kd = std::min(Fh, 128); t.N = Cp; t.S = 1;
+    w.tn_part = c.take(tn_any_partial(t));
+    w.colsum_part = c.take((size_t)colsum_parts(plan) * C);
+  }
+  w.bytes = c.bytes;
+  return w;
+}
+
+// Both node-head calls: one forward for training (dH set) and prediction, so the evaluation loss is bit-identical to
+// the training loss.  Forward: logits GEMM (bias in its epilogue), softmax_ce_kernel over the R rows, loss partials
+// summed in fixed order.  Backward: dH = dlog head_W^T on `st`, dhead_W = H^T dlog and dhead_b = colsum(dlog) beside it
+// on the side stream.
+int node_head_run(const char* who, const agcn_plan* plan, const float* d_H, const float* d_head_W,
+                  const float* d_head_b, const float* d_targets, const float* d_weights, float scale, int32_t Fh,
+                  int32_t C, float* d_probs, float* d_loss, float* d_dH, float* d_dhead_W, float* d_dhead_b,
+                  void* d_work, size_t work_bytes, cudaStream_t st) {
+  const std::string at = std::string(who) + ": ";
+  AGCN_REQUIRE(Fh >= 1 && C >= 1, at + "unsupported sizes (need Fh >= 1 and C >= 1)");
+  const bool train = d_dH != nullptr;
+  int rc = plan_use(plan, st);
+  if (rc) return rc;
+  NodeHeadWork w = carve_node_head(plan, Fh, C, train, d_work);
+  if (w.bytes > work_bytes) {
+    set_error(at + "workspace too small");
+    return AGCN_ERR_WORKSPACE;
+  }
+  const int R = (int)plan->R, Cp = pad4(C);
+  cudaStream_t side = plan->side;
+
+  GemmArgs g_log, g_dH;
+  g_log.M = R; g_log.N = C; g_log.Kd = Fh;
+  g_log.A0 = d_H; g_log.lda0 = Fh;
+  g_log.B = d_head_W; g_log.ldb = C;
+  g_log.C = w.dlog; g_log.ldc = Cp;
+  g_log.bias = d_head_b;
+  // dH: contraction over the C classes, R / 128 row tiles -- enough tiles without split-K
+  g_dH.M = R; g_dH.N = Fh; g_dH.Kd = C;
+  g_dH.A0 = w.dlog; g_dH.lda0 = Cp;
+  g_dH.B = d_head_W; g_dH.ldb = C; g_dH.transB = 1;   // head_W is [Fh, C] = [N, Kd]
+  g_dH.C = d_dH; g_dH.ldc = Fh;
+  const bool tc_log = tc_gemm_supported(g_log), tc_dH = train && tc_gemm_supported(g_dH);
+
+  // parameter operands (hi / lo split, K-major) on the side stream
+  AGCN_CUDA(cudaEventRecord(plan->ev_side_fork, st));
+  AGCN_CUDA(cudaStreamWaitEvent(side, plan->ev_side_fork, 0));
+  if (tc_log && (rc = tc_gemm_split_b(g_log, w.tcB, side))) return rc;
+  if (tc_dH && (rc = tc_gemm_split_b(g_dH, w.tcC, side))) return rc;
+  AGCN_CUDA(cudaEventRecord(plan->ev_side_join, side));
+  AGCN_CUDA(cudaStreamWaitEvent(st, plan->ev_side_join, 0));
+
+  // logits (only the C real columns of dlog are written and read back: the pad columns feed nothing but the pad
+  // columns of dWh_pad, which are not copied out), then the row softmax: d loss / d logits in place (training) or the
+  // probabilities, and the per-row loss terms
+  if ((rc = tc_log ? tc_gemm(g_log, w.tcB, st) : gemm_rows(g_log, st))) return rc;
+  (train ? softmax_ce_kernel<true> : softmax_ce_kernel<false>)<<<(R + 7) / 8, 256, 0, st>>>(
+      w.dlog, Cp, d_targets, d_weights, R, C, scale, d_probs, w.loss_part);
+  AGCN_LAUNCH_CHECK();
+  if (d_loss) {
+    sum_parts_kernel<<<1, 256, 0, st>>>(w.loss_part, R, d_loss);
+    AGCN_LAUNCH_CHECK();
+  }
+  if (!train) return AGCN_OK;
+
+  // parameter gradients on the side stream, beside dH on the main stream
+  AGCN_CUDA(cudaEventRecord(plan->ev_side_fork, st));
+  AGCN_CUDA(cudaStreamWaitEvent(side, plan->ev_side_fork, 0));
+  colsum_part_kernel<<<colsum_parts(plan), 256, 0, side>>>(w.dlog, Cp, R, C, w.colsum_part);
+  AGCN_LAUNCH_CHECK();
+  if ((rc = colsum_reduce(w.colsum_part, colsum_parts(plan), C, d_dhead_b, side))) return rc;
+  for (int f0 = 0; f0 < Fh; f0 += 128) {  // dhead_W = H^T dlog, 128 rows of the result per contraction
+    GemmTNArgs t;
+    t.M = R; t.Kd = std::min(128, Fh - f0); t.N = Cp; t.S = 1;
+    t.A0 = d_H + f0; t.lda0 = Fh;
+    t.D = w.dlog; t.ldd = Cp;
+    t.out = w.dWh_pad + (size_t)f0 * Cp; t.partial = w.tn_part;
+    if ((rc = tn_any(t, side))) return rc;
+  }
+  {
+    const int64_t total = (int64_t)Fh * C;
+    copy_pitched_kernel<<<(unsigned)((total + 255) / 256), 256, 0, side>>>(w.dWh_pad, Cp, d_dhead_W, C, Fh, C);
+    AGCN_LAUNCH_CHECK();
+  }
+  AGCN_CUDA(cudaEventRecord(plan->ev_side_join, side));
+
+  if ((rc = tc_dH ? tc_gemm(g_dH, w.tcC, st) : gemm_rows(g_dH, st))) return rc;
+  AGCN_CUDA(cudaStreamWaitEvent(st, plan->ev_side_join, 0));
+  return AGCN_OK;
+}
+
 }  // namespace
 }  // namespace agcn
 
@@ -456,6 +600,39 @@ int agcn_head_predict(const agcn_plan* plan, const float* d_H, const float* d_de
                "head_predict: null pointer");
   return head_run("head_predict", plan, d_H, d_dense_W, d_dense_b, d_head_W, d_head_b, d_targets, d_weights, scale,
                   loss_kind, Fh, Fm, Nt, d_probs, d_loss, nullptr, d_work, work_bytes, (cudaStream_t)stream);
+}
+
+int agcn_node_head_workspace_bytes(const agcn_plan* plan, int32_t Fh, int32_t C, size_t* bytes) {
+  AGCN_REQUIRE(plan && bytes && Fh >= 1 && C >= 1, "node_head_workspace_bytes: bad arguments");
+  *bytes = carve_node_head(plan, Fh, C, true, nullptr).bytes + 256;
+  return AGCN_OK;
+}
+
+int agcn_node_head_loss_grad(const agcn_plan* plan, const float* d_H, const float* d_head_W, const float* d_head_b,
+                             const float* d_targets, const float* d_weights, float scale, int32_t Fh, int32_t C,
+                             float* d_loss, float* d_dH, float* d_dhead_W, float* d_dhead_b, void* d_work,
+                             size_t work_bytes, void* stream) {
+  AGCN_REQUIRE(plan && d_H && d_head_W && d_head_b && d_targets && d_weights && d_loss && d_dH && d_dhead_W &&
+                   d_dhead_b && d_work,
+               "node_head_loss_grad: null pointer");
+  return node_head_run("node_head_loss_grad", plan, d_H, d_head_W, d_head_b, d_targets, d_weights, scale, Fh, C,
+                       nullptr, d_loss, d_dH, d_dhead_W, d_dhead_b, d_work, work_bytes, (cudaStream_t)stream);
+}
+
+int agcn_node_head_predict_workspace_bytes(const agcn_plan* plan, int32_t Fh, int32_t C, size_t* bytes) {
+  AGCN_REQUIRE(plan && bytes && Fh >= 1 && C >= 1, "node_head_predict_workspace_bytes: bad arguments");
+  *bytes = carve_node_head(plan, Fh, C, false, nullptr).bytes + 256;
+  return AGCN_OK;
+}
+
+int agcn_node_head_predict(const agcn_plan* plan, const float* d_H, const float* d_head_W, const float* d_head_b,
+                           const float* d_targets, const float* d_weights, float scale, int32_t Fh, int32_t C,
+                           float* d_probs, float* d_loss, void* d_work, size_t work_bytes, void* stream) {
+  AGCN_REQUIRE(!d_targets == !d_weights && !d_targets == !d_loss,
+               "node_head_predict: d_targets, d_weights and d_loss must be all NULL or all set");
+  AGCN_REQUIRE(plan && d_H && d_head_W && d_head_b && d_probs && d_work, "node_head_predict: null pointer");
+  return node_head_run("node_head_predict", plan, d_H, d_head_W, d_head_b, d_targets, d_weights, scale, Fh, C, d_probs,
+                       d_loss, nullptr, nullptr, nullptr, d_work, work_bytes, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -247,6 +247,8 @@ size_t act_bwd_partial_floats(int64_t R, int Fo);
 int act_bwd_partials(const float* dY, const float* Y, float* dYp, float* partial, int64_t R, int Fo, int act,
                      cudaStream_t st);
 int act_bwd_reduce(const float* partial, float* dbias, int64_t R, int Fo, cudaStream_t st);
+// out[c] = sum_k partial[k * cols + c] over the n_part rows of per-CTA column sums, fixed order (act_bwd_reduce's stage)
+int colsum_reduce(const float* partial, int n_part, int cols, float* out, cudaStream_t st);
 
 // ---------------------------------------------------------------- per-graph kernels (agcn_graph_small.cu)
 struct GraphArgs {

@@ -326,8 +326,11 @@ int act_bwd_reduce(const float* partial, float* dbias, int64_t R, int Fo, cudaSt
     AGCN_CUDA(cudaMemsetAsync(dbias, 0, Fo * sizeof(float), st));
     return AGCN_OK;
   }
-  const int blocks = (int)((R + ACT_ROWS - 1) / ACT_ROWS);
-  colsum_reduce_kernel<<<(Fo + 31) / 32, 256, 0, st>>>(partial, dbias, blocks, Fo);
+  return colsum_reduce(partial, (int)((R + ACT_ROWS - 1) / ACT_ROWS), Fo, dbias, st);
+}
+
+int colsum_reduce(const float* partial, int n_part, int cols, float* out, cudaStream_t st) {
+  colsum_reduce_kernel<<<(cols + 31) / 32, 256, 0, st>>>(partial, out, n_part, cols);
   AGCN_LAUNCH_CHECK();
   return AGCN_OK;
 }

@@ -23,7 +23,8 @@
 struct agcn_stack {
   std::vector<agcn_stack_node> nodes;  // desc.flags as the layer classes set them
   int32_t Fm = 0, Nt = 0, loss_kind = 0;
-  std::vector<int64_t> off;  // 5 per node {weight, bias, M_L, alpha, beta | -1}, then dense_W, dense_b, head_W, head_b
+  std::vector<int64_t> off;  // 5 per node {weight, bias, M_L, alpha, beta | -1}, then dense_W, dense_b (-1, -1 for the
+                             // per-node head), head_W, head_b
   // topology, derived once by agcn_stack_create_nodes
   std::vector<int32_t> lall_user;   // Reslap node i: the Reslap node whose L_prev is L_all[i], or -1
   std::vector<int32_t> res_user;    // node i: the BlockEnd whose x_res is H[i], or -1
@@ -96,6 +97,18 @@ int node_bytes(const agcn_stack_node& nd, const agcn_plan* plan, bool train, siz
   return AGCN_OK;
 }
 
+bool node_head(const agcn_stack* s) { return s->loss_kind == AGCN_PER_NODE_SOFTMAX_CE; }
+
+// work area of the head call of agcn_stack_loss_grad (train) or agcn_stack_predict
+int head_bytes(const agcn_stack* s, const agcn_plan* plan, bool train, size_t* bytes) {
+  const int32_t Fh = s->nodes.back().desc.Fo;
+  if (node_head(s))
+    return train ? agcn_node_head_workspace_bytes(plan, Fh, s->Nt, bytes)
+                 : agcn_node_head_predict_workspace_bytes(plan, Fh, s->Nt, bytes);
+  return train ? agcn_head_workspace_bytes(plan, Fh, s->Fm, s->Nt, bytes)
+               : agcn_head_predict_workspace_bytes(plan, Fh, s->Fm, s->Nt, bytes);
+}
+
 // Where the forward walk finds node i's output, L_all and `saved` area, and the scratch of the layer and head calls.
 // Training gives every node areas of its own; prediction points the nodes at reused slots and one shared `saved` area.
 struct StackWork {
@@ -135,7 +148,7 @@ int carve_stack(const agcn_stack* s, const agcn_plan* plan, void* base, StackWor
   w->dB = c.take(R * maxF);
   w->layer_work_bytes = work_max;
   w->layer_work = c.area(work_max);
-  int rc = agcn_head_workspace_bytes(plan, s->nodes.back().desc.Fo, s->Fm, s->Nt, &w->head_work_bytes);
+  int rc = head_bytes(s, plan, true, &w->head_work_bytes);
   if (rc) return rc;
   w->head_work = c.area(w->head_work_bytes);
   w->Lall.assign(n, nullptr);
@@ -177,7 +190,7 @@ int carve_predict(const agcn_stack* s, const agcn_plan* plan, void* base, StackW
   void* saved = c.area(saved_max);
   w->layer_work_bytes = work_max;
   w->layer_work = c.area(work_max);
-  int rc = agcn_head_predict_workspace_bytes(plan, s->nodes.back().desc.Fo, s->Fm, s->Nt, &w->head_work_bytes);
+  int rc = head_bytes(s, plan, false, &w->head_work_bytes);
   if (rc) return rc;
   w->head_work = c.area(w->head_work_bytes);
   for (int k = 0; k < s->n_pred_l; ++k) l_slot.push_back(c.take((size_t)plan->LL));
@@ -258,11 +271,18 @@ int agcn_stack_create_nodes(const agcn_stack_node* nodes, int32_t n_nodes, int32
                             const int64_t* param_offsets, agcn_stack** out) {
   AGCN_REQUIRE(nodes && n_nodes >= 1 && param_offsets && out, "stack_create: bad arguments");
   *out = nullptr;
-  AGCN_REQUIRE(Fm >= 1 && Nt >= 1, "stack_create: Fm and Nt must be positive");
-  // the head calls take loss_kind as it is: agcn_stack_loss_grad / agcn_stack_predict need nothing per kind
+  const bool per_node = loss_kind == AGCN_PER_NODE_SOFTMAX_CE;
+  AGCN_REQUIRE(per_node || (Fm >= 1 && Nt >= 1), "stack_create: Fm and Nt must be positive");
+  // the graph-head calls take loss_kind as it is: agcn_stack_loss_grad / agcn_stack_predict need nothing per kind
+  // beyond choosing between them and the per-node head
   AGCN_REQUIRE(loss_kind == AGCN_LOSS_SIGMOID_CE || loss_kind == AGCN_LOSS_SOFTMAX_CE ||
-                   loss_kind == AGCN_LOSS_WEIGHTED_L2,
+                   loss_kind == AGCN_LOSS_WEIGHTED_L2 || per_node,
                "stack_create: unknown loss_kind");
+  if (per_node) {
+    AGCN_REQUIRE(Fm == 0 && Nt >= 1, "stack_create: the per-node head has no DenseMol (Fm must be 0) and Nt >= 1 classes");
+    AGCN_REQUIRE(param_offsets[5 * (size_t)n_nodes] == -1 && param_offsets[5 * (size_t)n_nodes + 1] == -1,
+                 "stack_create: the per-node head has no dense_W / dense_b (their offsets must be -1)");
+  }
   std::vector<int32_t> lall_user(n_nodes, -1), res_user(n_nodes, -1);
   for (int i = 0; i < n_nodes; ++i) {
     const agcn_stack_node& nd = nodes[i];
@@ -367,11 +387,17 @@ int agcn_stack_loss_grad(const agcn_stack* s, const agcn_plan* plan, const float
   const int64_t* ho = &s->off[5 * (size_t)nl];
   if ((rc = forward_nodes(s, plan, w, d_X, d_Lint, d_params, true, stream))) return rc;
   // ---- DenseMol + GraphGatherMol + logits + loss, with every gradient of that part
+  // (or the per-node head: logits + loss of every node)
   const agcn_sgcll_desc& last = s->nodes[nl - 1].desc;
-  rc = agcn_head_loss_grad_ex(plan, w.H[nl - 1], d_params + ho[0], d_params + ho[1], d_params + ho[2], d_params + ho[3],
-                              d_targets, d_weights, scale, s->loss_kind, last.Fo, s->Fm, s->Nt, d_loss, w.dA,
-                              d_grads + ho[0], d_grads + ho[1], d_grads + ho[2], d_grads + ho[3], w.head_work,
-                              w.head_work_bytes, stream);
+  if (node_head(s))
+    rc = agcn_node_head_loss_grad(plan, w.H[nl - 1], d_params + ho[2], d_params + ho[3], d_targets, d_weights, scale,
+                                  last.Fo, s->Nt, d_loss, w.dA, d_grads + ho[2], d_grads + ho[3], w.head_work,
+                                  w.head_work_bytes, stream);
+  else
+    rc = agcn_head_loss_grad_ex(plan, w.H[nl - 1], d_params + ho[0], d_params + ho[1], d_params + ho[2],
+                                d_params + ho[3], d_targets, d_weights, scale, s->loss_kind, last.Fo, s->Fm, s->Nt,
+                                d_loss, w.dA, d_grads + ho[0], d_grads + ho[1], d_grads + ho[2], d_grads + ho[3],
+                                w.head_work, w.head_work_bytes, stream);
   if (rc) return rc;
   if (notify) notify(notify_user, nl, stream);
   // ---- backward, last node first; the first layer's input has no gradient unless the metric is differentiable.
@@ -446,9 +472,13 @@ int agcn_stack_predict(const agcn_stack* s, const agcn_plan* plan, const float* 
   if ((rc = forward_nodes(s, plan, w, d_X, d_Lint, d_params, false, stream))) return rc;
   const int nl = (int)s->nodes.size();
   const int64_t* ho = &s->off[5 * (size_t)nl];
+  const int32_t Fh = s->nodes.back().desc.Fo;
+  if (node_head(s))
+    return agcn_node_head_predict(plan, w.H[nl - 1], d_params + ho[2], d_params + ho[3], d_targets, d_weights, scale, Fh,
+                                  s->Nt, d_probs, d_loss, w.head_work, w.head_work_bytes, stream);
   return agcn_head_predict(plan, w.H[nl - 1], d_params + ho[0], d_params + ho[1], d_params + ho[2], d_params + ho[3],
-                           d_targets, d_weights, scale, s->loss_kind, s->nodes.back().desc.Fo, s->Fm, s->Nt, d_probs,
-                           d_loss, w.head_work, w.head_work_bytes, stream);
+                           d_targets, d_weights, scale, s->loss_kind, Fh, s->Fm, s->Nt, d_probs, d_loss, w.head_work,
+                           w.head_work_bytes, stream);
 }
 
 int agcn_adam_step(float* d_params, const float* d_grads, float* d_m, float* d_v, int32_t* d_step, int64_t n, float lr,

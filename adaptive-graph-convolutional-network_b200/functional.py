@@ -210,6 +210,81 @@ def head_predict(H, dense_W, dense_b, head_W, head_b, batch, loss_kind, targets=
     return probs, (loss.reshape(()) if loss is not None else None)
 
 
+class _NodeHeadLossFunction(torch.autograd.Function):
+    """Per-node classification head (agcn_node_head_loss_grad): x = H head_W + head_b for every packed row, softmax
+    cross-entropy weighted per node * scale -> scalar loss.  The C call computes the loss AND every gradient; backward
+    hands them out as _HeadLossFunction does."""
+
+    @staticmethod
+    def forward(ctx, H, head_W, head_b, targets, weights, batch, scale, unit_grad):
+        H = H.contiguous()
+        R, Fh = H.shape
+        C = head_W.shape[1]
+        dev = H.device
+        assert head_W.shape == (Fh, C) and R == batch.total_nodes
+        assert targets.shape == (R, C) and weights.numel() == R
+        nbytes = ctypes.c_size_t()
+        _lib.check(_lib.lib().agcn_node_head_workspace_bytes(batch.handle, Fh, C, ctypes.byref(nbytes)))
+        work = _Workspace.get(dev, nbytes.value)
+        outs = [getattr(t, "_agcn_grad_out", None) for t in (head_W, head_b)]
+        grads = [o if o is not None else torch.empty_like(t) for o, t in zip(outs, (head_W, head_b))]
+        loss = torch.empty(1, device=dev, dtype=torch.float32)
+        dH = torch.empty_like(H)
+        with torch.cuda.device(dev):
+            _lib.check(_lib.lib().agcn_node_head_loss_grad(
+                batch.handle, _ptr(H), _ptr(head_W), _ptr(head_b), _ptr(targets.contiguous()),
+                _ptr(weights.contiguous()), float(scale), Fh, C, _ptr(loss), _ptr(dH), _ptr(grads[0]), _ptr(grads[1]),
+                _ptr(work), work.numel(), _stream_ptr(dev)))
+        ctx.unit_grad = unit_grad
+        ctx.in_place = [o is not None for o in outs]
+        ctx.save_for_backward(dH, *grads)
+        return loss.reshape(())
+
+    @staticmethod
+    def backward(ctx, g):
+        dH, *grads = ctx.saved_tensors
+        if not ctx.unit_grad:
+            dH = dH * g
+            grads = [t if ip else t * g for t, ip in zip(grads, ctx.in_place)]
+        out = [None if ip else t for t, ip in zip(grads, ctx.in_place)]
+        return (dH, out[0], out[1], None, None, None, None, None)
+
+
+def node_head_loss(H, head_W, head_b, targets, weights, batch, scale, unit_grad=False):
+    """Scalar loss of the per-node head on the packed output of the last node: H [R, Fh], head_W [Fh, C], head_b [C],
+    targets [R, C] one-hot float, weights [R] (0 masks a node); loss = scale * sum_r w_r (logsumexp(x_r) - <y_r, x_r>).
+    unit_grad as for head_loss."""
+    return _NodeHeadLossFunction.apply(H, head_W, head_b, targets, weights, batch, scale, unit_grad)
+
+
+def node_head_predict(H, head_W, head_b, batch, targets=None, weights=None, scale=None):
+    """Per-node class probabilities (agcn_node_head_predict), no autograd node: (probs [R, C], loss or None).  With
+    targets [R, C] and weights [R] the loss is also computed, bit for bit the loss of node_head_loss; scale defaults to
+    1 / batch size."""
+    if (targets is None) != (weights is None):
+        raise ValueError("node_head_predict: pass both targets and weights, or neither")
+    H = H.detach().contiguous()
+    R, Fh = H.shape
+    C = head_W.shape[1]
+    dev = H.device
+    assert head_W.shape == (Fh, C) and R == batch.total_nodes
+    loss = None
+    if targets is not None:
+        targets, weights = targets.detach().contiguous(), weights.detach().contiguous()
+        assert targets.shape == (R, C) and weights.numel() == R
+        scale = 1.0 / batch.batch_size if scale is None else scale
+        loss = torch.empty(1, device=dev, dtype=torch.float32)
+    nbytes = ctypes.c_size_t()
+    _lib.check(_lib.lib().agcn_node_head_predict_workspace_bytes(batch.handle, Fh, C, ctypes.byref(nbytes)))
+    work = _Workspace.get(dev, nbytes.value)
+    probs = torch.empty(R, C, device=dev, dtype=torch.float32)
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib().agcn_node_head_predict(
+            batch.handle, _ptr(H), _ptr(head_W.detach()), _ptr(head_b.detach()), _ptr(targets), _ptr(weights),
+            float(scale or 0.0), Fh, C, _ptr(probs), _ptr(loss), _ptr(work), work.numel(), _stream_ptr(dev)))
+    return probs, (loss.reshape(()) if loss is not None else None)
+
+
 class _UnpackNodes(torch.autograd.Function):
     @staticmethod
     def forward(ctx, packed, batch):

@@ -76,7 +76,7 @@ class ResAGCNStep(SimpleAGCNStep):
 
     def _create_stack(self, offs):
         _lib.check(_lib.lib().agcn_stack_create_nodes(self.nodes(), len(self.layers), self.Fm, self.Nt,
-                                                      _lib.LOSS[self.loss_kind], offs, ctypes.byref(self._stack)))
+                                                      _lib.loss_code(self.loss_kind), offs, ctypes.byref(self._stack)))
 
     def _body(self, x):
         outs, lall = [], {}

@@ -36,11 +36,12 @@ class SimpleAGCNStep(object):
                  beta1=0.9, beta2=0.999, epsilon=1e-8):
         """loss="sigmoid_ce": n_tasks two-class heads (Nt = 2 n_tasks logits);  loss="softmax_ce": one head with
         n_tasks classes (Nt = n_tasks logits);  loss="weighted_l2": n_tasks regression outputs (Nt = n_tasks),
-        loss = sum (w (x - y))^2 / global batch."""
+        loss = sum (w (x - y))^2 / global batch;  loss="node_softmax_ce": one label per NODE out of n_tasks classes
+        (part segmentation): no DenseMol / gather, head_W [filters[-1], n_tasks] on every node, softmax cross-entropy
+        weighted per node / global batch (final_feature_n is ignored)."""
         if engine not in ("stack", "autograd"):
             raise ValueError("engine must be 'stack' or 'autograd'")
-        if loss not in _lib.LOSS:
-            raise ValueError("loss must be one of %s" % sorted(_lib.LOSS))
+        _lib.loss_code(loss)
         self.device = torch.device(device)
         self.world_size = world_size
         self.global_batch = batch_size * world_size
@@ -50,23 +51,30 @@ class SimpleAGCNStep(object):
         self.overlap_allreduce = overlap_allreduce and world_size > 1
         self.lr, self.beta1, self.beta2, self.epsilon = learning_rate, beta1, beta2, epsilon
         self.Nt = 2 * n_tasks if loss == "sigmoid_ce" else n_tasks
-        self.Fm = final_feature_n
-        if final_feature_n < 32 or final_feature_n % 4:
+        self.node_head = loss in _lib.NODE_LOSS
+        self.Fm = 0 if self.node_head else final_feature_n
+        if not self.node_head and (final_feature_n < 32 or final_feature_n % 4):
             raise ValueError("final_feature_n must be >= 32 and a multiple of 4 (agcn_head_loss_grad)")
         torch.manual_seed(seed)  # identical replicas on every rank
         _gc.DEFAULT_DEVICE[0] = str(self.device)
         self._build_layers(n_feat, filters, batch_size, K, laplacian, metric_grad)
         for l in self.layers:
             l.build()
-        lim = float(np.sqrt(6.0 / (filters[-1] + final_feature_n)))
-        self.dense_W = ((torch.rand(filters[-1], final_feature_n) * 2 - 1) * lim).to(self.device).requires_grad_(True)
-        self.dense_b = torch.zeros(final_feature_n, device=self.device, requires_grad=True)
+        if self.node_head:          # the head reads the last node's output directly
+            self.dense_W = self.dense_b = None
+            head_in = filters[-1]
+        else:
+            lim = float(np.sqrt(6.0 / (filters[-1] + final_feature_n)))
+            self.dense_W = ((torch.rand(filters[-1], final_feature_n) * 2 - 1) * lim).to(
+                self.device).requires_grad_(True)
+            self.dense_b = torch.zeros(final_feature_n, device=self.device, requires_grad=True)
+            head_in = final_feature_n
         # n_tasks independent [n_feature, 2] logits heads == one [n_feature, 2 * n_tasks] matrix
-        self.head_W = torch.nn.init.trunc_normal_(torch.empty(final_feature_n, self.Nt), std=0.01, a=-0.02,
+        self.head_W = torch.nn.init.trunc_normal_(torch.empty(head_in, self.Nt), std=0.01, a=-0.02,
                                                   b=0.02).to(self.device).requires_grad_(True)
         self.head_b = torch.zeros(self.Nt, device=self.device, requires_grad=True)
-        self.params = [v for l in self.layers for v in l.vars.values()] + [self.dense_W, self.dense_b, self.head_W,
-                                                                           self.head_b]
+        self.params = [v for l in self.layers for v in l.vars.values()] + [t for t in (
+            self.dense_W, self.dense_b, self.head_W, self.head_b) if t is not None]
         # one flat gradient buffer and one flat parameter buffer; every parameter / .grad is a view into them, and every
         # producer (SGC-LL backward, head) OVERWRITES its gradients in place: nothing to zero, nothing to accumulate
         self.grads = FlatGradBuffer(self.params, direct=self.params)
@@ -88,6 +96,9 @@ class SimpleAGCNStep(object):
             self._stage_slices.append((start, off))
         start = off
         for t in (self.dense_W, self.dense_b, self.head_W, self.head_b):
+            if t is None:                             # the per-node head: no dense pair
+                offs.append(-1)
+                continue
             offs.append(off)
             off += t.numel()
         self._stage_slices.append((start, off))      # stage n_layers = dense + head
@@ -121,8 +132,8 @@ class SimpleAGCNStep(object):
         descs = (_lib.Desc * len(self.layers))()
         for i, l in enumerate(self.layers):
             descs[i] = _layer_desc(l)
-        _lib.check(_lib.lib().agcn_stack_create(descs, len(self.layers), self.Fm, self.Nt, _lib.LOSS[self.loss_kind],
-                                                offs, ctypes.byref(self._stack)))
+        _lib.check(_lib.lib().agcn_stack_create(descs, len(self.layers), self.Fm, self.Nt,
+                                                _lib.loss_code(self.loss_kind), offs, ctypes.byref(self._stack)))
 
     def _body(self, x):
         """The layer classes on the input dict of the drop-in path -> PackedNodes output of the last layer."""
@@ -190,11 +201,15 @@ class SimpleAGCNStep(object):
 
     def forward_loss(self, X, Lint, batch, targets, weights):
         """The drop-in path: layer classes + torch.autograd.  X [R, F] packed, Lint packed, targets [B, Nt] float,
-        weights [B, Nt] (sigmoid_ce, weighted_l2) or [B] (softmax_ce) -> scalar loss."""
-        from .functional import head_loss
+        weights [B, Nt] (sigmoid_ce, weighted_l2) or [B] (softmax_ce); node_softmax_ce: targets [R, Nt], weights [R]
+        -> scalar loss."""
+        from .functional import head_loss, node_head_loss
         x = {'node_features': PackedNodes(X, batch), 'original_laplacian': PackedLaplacians(Lint, batch),
              'data_slice': None, 'lap_slice': None, '_batch': batch}
         out = self._body(x)
+        if self.node_head:
+            return node_head_loss(out.data, self.head_W, self.head_b, targets, weights, batch, 1.0 / self.global_batch,
+                                  unit_grad=True)
         return head_loss(out.data, self.dense_W, self.dense_b, self.head_W, self.head_b, targets, weights, batch,
                          1.0 / self.global_batch, unit_grad=True, loss_kind=self.loss_kind)
 
@@ -203,7 +218,7 @@ class SimpleAGCNStep(object):
         X, Lint = X.contiguous(), Lint.contiguous()
         targets, weights = targets.contiguous(), weights.contiguous()
         assert X.shape[0] == batch.total_nodes and Lint.numel() == batch.total_lap
-        assert targets.shape == (batch.batch_size, self.Nt)
+        assert targets.shape == (self._label_rows(batch), self.Nt)
         if self.engine == "stack":
             return self._loss_grad_stack(X, Lint, batch, targets, weights)
         loss = self.forward_loss(X, Lint, batch, targets, weights)
@@ -211,10 +226,14 @@ class SimpleAGCNStep(object):
         return loss.detach().reshape(1)
 
     # ---- prediction (predict_proba / predict / evaluate of the reference's classifiers and regressor) ------------
+    def _label_rows(self, batch):
+        """Rows of the targets, probabilities and predictions: one per graph, or one per node for the per-node head."""
+        return batch.total_nodes if self.node_head else batch.batch_size
+
     def _predict_stack(self, X, Lint, batch, targets, weights, scale):
         lib = _lib.lib()
         arena = self._ensure_arena(batch, predict=True)
-        probs = torch.empty(batch.batch_size, self.Nt, device=self.device, dtype=torch.float32)
+        probs = torch.empty(self._label_rows(batch), self.Nt, device=self.device, dtype=torch.float32)
         loss = torch.empty(1, device=self.device, dtype=torch.float32) if targets is not None else None
         with torch.cuda.device(self.device):
             _lib.check(lib.agcn_stack_predict(
@@ -224,21 +243,23 @@ class SimpleAGCNStep(object):
         return probs, (loss.reshape(()) if loss is not None else None)
 
     def _predict(self, X, Lint, batch, targets=None, weights=None, scale=None):
-        """(probs [B, Nt] -- the values for weighted_l2 --, loss or None) of the current parameters; no gradient, no
-        parameter or optimizer state touched."""
+        """(probs [B, Nt] -- the values for weighted_l2, [R, Nt] for node_softmax_ce --, loss or None) of the current
+        parameters; no gradient, no parameter or optimizer state touched."""
         X, Lint = X.contiguous(), Lint.contiguous()
         assert X.shape[0] == batch.total_nodes and Lint.numel() == batch.total_lap
         if targets is not None:
             targets, weights = targets.contiguous(), weights.contiguous()
-            assert targets.shape == (batch.batch_size, self.Nt)
+            assert targets.shape == (self._label_rows(batch), self.Nt)
             scale = 1.0 / batch.batch_size if scale is None else scale
         if self.engine == "stack":
             return self._predict_stack(X, Lint, batch, targets, weights, scale)
-        from .functional import head_predict
+        from .functional import head_predict, node_head_predict
         x = {'node_features': PackedNodes(X, batch), 'original_laplacian': PackedLaplacians(Lint, batch),
              'data_slice': None, 'lap_slice': None, '_batch': batch}
         with torch.no_grad():
             out = self._body(x)
+            if self.node_head:
+                return node_head_predict(out.data, self.head_W, self.head_b, batch, targets, weights, scale)
             return head_predict(out.data, self.dense_W, self.dense_b, self.head_W, self.head_b, batch, self.loss_kind,
                                 targets, weights, scale)
 
@@ -247,14 +268,15 @@ class SimpleAGCNStep(object):
 
     def predict_proba(self, X, Lint, batch):
         """Class probabilities: [B, n_tasks, 2] for sigmoid_ce (softmax over each task's two logits), [B, n_classes]
-        for softmax_ce.  X [R, F] packed, Lint packed.  A weighted_l2 regressor has none: ValueError (use predict)."""
+        for softmax_ce, [R, n_classes] per packed node for node_softmax_ce (batch.unpack_nodes gives [B, Nmax,
+        n_classes]).  X [R, F] packed, Lint packed.  A weighted_l2 regressor has none: ValueError (use predict)."""
         if self.loss_kind == "weighted_l2":
             raise ValueError("predict_proba: a regressor (loss='weighted_l2') has no class probabilities; use predict")
         return self._shape_probs(self._predict(X, Lint, batch)[0])
 
     def predict(self, X, Lint, batch):
-        """Class labels (int64): [B, n_tasks] for sigmoid_ce, [B] for softmax_ce.  weighted_l2: the regression values
-        (float32) [B, n_tasks]."""
+        """Class labels (int64): [B, n_tasks] for sigmoid_ce, [B] for softmax_ce, [R] for node_softmax_ce.  weighted_l2:
+        the regression values (float32) [B, n_tasks]."""
         if self.loss_kind == "weighted_l2":
             return self._predict(X, Lint, batch)[0]
         return self.predict_proba(X, Lint, batch).argmax(-1)

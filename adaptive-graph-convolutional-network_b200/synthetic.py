@@ -177,3 +177,37 @@ def knn_like_batch(B, N, F, seed=1238, deg=16):
         np.fill_diagonal(A, False)
         L[g] = laplacian_from_dense_adjacency(A).astype(np.float32)
     return X, L, np.full(B, N, np.int32)
+
+
+# ---- per-node labels (the part labels of a segmentation batch) -------------------------------------------------------
+def synthetic_node_labels(batch, X, C, seed):
+    """One class out of C per node, learnable from the node's own features, in the packed row order.
+
+    batch: a GraphBatch, or its n_nodes array; X: the padded features [B, Nmax, F] of the batch (wire layout).
+      point clouds (F <= 8, xyz in the first three columns): the angular sector of (x, z) around the up axis y times
+      the height band of y within the cloud, S sectors x H bands with H = ceil(sqrt(C)), S = ceil(C / H), label
+      (sector * H + band) mod C;
+      molecules (75-d atom features): the index of the atom-type one-hot block (the first 44 columns) mod C.
+    Returns (targets [R, C] one-hot float32, weights [R] float32 of 0 / 1 with about 10 % zeros: unlabelled nodes)."""
+    n_nodes = np.asarray(getattr(batch, "n_nodes", batch), np.int64)
+    X = np.asarray(X)
+    rows = np.concatenate([X[g, :n] for g, n in enumerate(n_nodes)]).astype(np.float32)
+    if X.shape[-1] == 75:
+        label = rows[:, :44].argmax(1) % C
+    else:
+        H = int(np.ceil(np.sqrt(C)))
+        S = int(np.ceil(C / H))
+        ang = np.arctan2(rows[:, 2], rows[:, 0]) + np.pi                       # [0, 2 pi]
+        sector = np.minimum((ang * (S / (2 * np.pi))).astype(np.int64), S - 1)
+        band = np.empty(len(rows), np.int64)
+        off = 0
+        for n in n_nodes:
+            y = rows[off:off + n, 1]
+            lo, span = y.min(), max(float(y.max() - y.min()), 1e-12)
+            band[off:off + n] = np.minimum(((y - lo) * (H / span)).astype(np.int64), H - 1)
+            off += n
+        label = (sector * H + band) % C
+    targets = np.zeros((len(rows), C), np.float32)
+    targets[np.arange(len(rows)), label] = 1.0
+    weights = (np.random.default_rng(seed).random(len(rows)) >= 0.1).astype(np.float32)
+    return targets, weights

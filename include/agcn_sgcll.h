@@ -301,6 +301,32 @@ int agcn_head_predict(const agcn_plan* plan, const float* d_H, const float* d_de
                       float scale, int32_t loss_kind, int32_t Fh, int32_t Fm, int32_t Nt, float* d_probs, float* d_loss,
                       void* d_work, size_t work_bytes, void* stream);
 
+/* ---- per-node classification head: one label per node (the part segmentation of the reference's Seg_AGCN.py /
+ *      segmentation_module.py; restated, that code is not available here: parity unpinned).  No DenseMol, no gather,
+ *      no tanh: the logits of every packed row are
+ *        x[r, :] = H[r, :] head_W + head_b                      (no activation)
+ *      d_H [R,Fh] packed output of the last stack node; d_head_W [Fh,C], d_head_b [C]; d_targets [R,C] one-hot float
+ *      (as AGCN_LOSS_SOFTMAX_CE), d_weights [R] per node (0 masks an unlabelled node);
+ *        loss = scale * sum_r w_r sum_c y_rc (logsumexp(x_r) - x_rc),   d loss / d x_rc = w_r (softmax_c(x_r) sum y_r - y_rc) scale
+ *      (the stack passes scale = 1 / global batch in graphs; w_r = 1 / n_g gives a per-graph mean over nodes).
+ *   agcn_node_head_loss_grad: d_loss [1], d_dH [R,Fh], d_dhead_W [Fh,C], d_dhead_b [C] (overwritten).
+ *   agcn_node_head_predict: d_probs [R,C] = softmax(x_r) per row (agcn_unpack_nodes gives the padded [B,Nmax,C] layout);
+ *      d_targets / d_weights / d_loss all NULL or all set, then d_loss [1] is bit-identical to the training loss.
+ *   The row softmax is the single-task head's kernel; the products run on tcgen05 3xTF32 when the operands are
+ *   TMA-compatible (contraction >= 32, 16-byte pitches), on the CUDA cores otherwise.  Nothing is allocated; capturable.
+ *   AGCN_PER_NODE_SOFTMAX_CE is the loss_kind of a stack with this head (agcn_stack_create(_nodes) with Fm = 0 and the
+ *   dense_W / dense_b offsets -1; Nt = C).  The agcn_head_* calls reject it. */
+#define AGCN_PER_NODE_SOFTMAX_CE 4
+int agcn_node_head_workspace_bytes(const agcn_plan* plan, int32_t Fh, int32_t C, size_t* bytes);
+int agcn_node_head_loss_grad(const agcn_plan* plan, const float* d_H, const float* d_head_W, const float* d_head_b,
+                             const float* d_targets, const float* d_weights, float scale, int32_t Fh, int32_t C,
+                             float* d_loss, float* d_dH, float* d_dhead_W, float* d_dhead_b, void* d_work,
+                             size_t work_bytes, void* stream);
+int agcn_node_head_predict_workspace_bytes(const agcn_plan* plan, int32_t Fh, int32_t C, size_t* bytes);
+int agcn_node_head_predict(const agcn_plan* plan, const float* d_H, const float* d_head_W, const float* d_head_b,
+                           const float* d_targets, const float* d_weights, float scale, int32_t Fh, int32_t C,
+                           float* d_probs, float* d_loss, void* d_work, size_t work_bytes, void* stream);
+
 /* ---- one training step's loss and gradients as ONE call: the counterpart of `sess.run([train_op, loss, ...])`
  *      (models/tf_modules/multitask_classifier.py:255-264), which executes the whole graph of
  *      models/networks/basic_AGCN.py:35-47 inside the TensorFlow runtime.  A stack = n_layers SGC_LL layers (relu or
@@ -311,7 +337,10 @@ int agcn_head_predict(const agcn_plan* plan, const float* d_H, const float* d_de
  *      head_W [Fm,Nt], head_b [Nt].
  *   notify (optional): called on the host right after the gradients of a stage have been ENQUEUED on `stream`
  *      (stage n_layers = head + dense, then n_layers-1 .. 0 = that SGC_LL layer), so a data-parallel caller can start
- *      the all-reduce of a gradient bucket while the earlier layers are still running backward. */
+ *      the all-reduce of a gradient bucket while the earlier layers are still running backward.
+ *   loss_kind AGCN_PER_NODE_SOFTMAX_CE: the per-node head instead (agcn_node_head_loss_grad / _predict): Fm = 0, the
+ *      dense_W / dense_b offsets are -1, Nt = C classes, d_targets [R,C], d_weights [R], d_probs [R,C]; stage
+ *      n_layers covers head_W and head_b. */
 typedef struct agcn_stack agcn_stack;
 typedef void (*agcn_stack_notify_fn)(void* user, int32_t stage, void* stream);
 int agcn_stack_create(const agcn_sgcll_desc* layer_descs, int32_t n_layers, int32_t Fm, int32_t Nt, int32_t loss_kind,
