@@ -58,9 +58,6 @@ _SIGNATURES = {
     "agcn_plan_node_off_host": (_P, [_P]),
     "agcn_plan_lap_off_host": (_P, [_P]),
     "agcn_fused_tiles_host": (ctypes.c_int, [_P, ctypes.c_int32, _P, ctypes.c_int32, _P, ctypes.c_int32, _P, _P]),
-    "agcn_fused_debug_set": (ctypes.c_int, [_P]),
-    "agcn_fused_profile": (ctypes.c_int, [ctypes.c_int]),
-    "agcn_fused_profile_read": (ctypes.c_int, [ctypes.POINTER(ctypes.c_float), ctypes.POINTER(ctypes.c_int)]),
     "agcn_profile_enable": (ctypes.c_int, [ctypes.c_int]),
     "agcn_profile_read": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_size_t, ctypes.POINTER(ctypes.c_size_t)]),
     "agcn_profile_timeline": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_size_t, ctypes.POINTER(ctypes.c_size_t)]),
@@ -75,7 +72,6 @@ _SIGNATURES = {
     "agcn_unpack_lap": (ctypes.c_int, [_P, _P, _P, _P]),
     "agcn_debug_grouped_product": (ctypes.c_int, [_P, _P, _P, _P, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
                                                   ctypes.c_float, ctypes.c_int32, _P]),
-    "agcn_debug_grouped_timeline": (ctypes.c_int, [_P]),
     "agcn_pack_lap_csr": (ctypes.c_int, [_P, _P, _P, _P, _P, _P]),
     "agcn_point_laplacian_workspace_bytes": (ctypes.c_int, [_P, ctypes.POINTER(ctypes.c_size_t)]),
     "agcn_point_laplacian": (ctypes.c_int, [_P, _P, ctypes.c_int32, ctypes.c_int32, ctypes.c_float, _P, _P,

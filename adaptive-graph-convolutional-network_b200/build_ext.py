@@ -17,8 +17,7 @@ HDR = sorted(glob.glob(os.path.join(HERE, "csrc", "*.cuh"))) + [os.path.join(ROO
 OUT = os.path.join(HERE, "libagcn_sm100.so")
 
 NVCC_FLAGS = [
-    "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", *(["-DAGCN_TN_DEBUG"] if os.environ.get("AGCN_TN_DEBUG") else []),
-    *(["-DAGCN_AB_SWITCHES"] if os.environ.get("AGCN_AB_SWITCHES") else []), "-O3", "-std=c++17",
+    "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-shared", "-I", os.path.join(ROOT, "include"),
 ]
 

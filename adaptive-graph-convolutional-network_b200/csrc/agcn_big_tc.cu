@@ -23,7 +23,6 @@
 #include <cuda.h>
 
 #include <algorithm>
-#include <cstdlib>
 #include <mutex>
 
 #include "agcn_internal.cuh"
@@ -126,17 +125,6 @@ __device__ __forceinline__ float4 lds128(uint32_t a) {
 __device__ __forceinline__ float tf32_hi(float x) { return tf32_rn(x); }
 __device__ __forceinline__ float tf32_lo(float x, float hi) { return tf32_rn(x - hi); }
 
-__device__ __forceinline__ unsigned long long gtime() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;\n" : "=l"(t));
-  return t;
-}
-// timeline of CTA (0, 0): 8 slots per k-block (first 64) + 3 at 520.. (tools/tc_timeline.py)
-#define BT_STAMP(slot)                                     \
-  do {                                                     \
-    if (dbg_on) p.dbg[(slot)] = gtime();                   \
-  } while (0)
-
 __global__ void __launch_bounds__(THREADS, 1)
 grouped_tc_kernel(const __grid_constant__ CUtensorMap tmIn, GroupedArgs p) {
   const int g = p.tile_graph[blockIdx.x], m0 = p.tile_row[blockIdx.x];
@@ -152,8 +140,6 @@ grouped_tc_kernel(const __grid_constant__ CUtensorMap tmIn, GroupedArgs p) {
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 3 * STAGES + 1);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const bool dbg_on = p.dbg != nullptr && blockIdx.x == 0 && blockIdx.y == 0;
-  if (threadIdx.x == 0) BT_STAMP(520);
   const int n = p.n_nodes[g];
   const long long row0 = p.node_off[g];
   const float* __restrict__ Lg = p.L + p.lap_off[g];
@@ -186,7 +172,6 @@ grouped_tc_kernel(const __grid_constant__ CUtensorMap tmIn, GroupedArgs p) {
       for (int kb = 0; kb < num_kb; ++kb) {
         const int stage = kb % STAGES, phase = (kb / STAGES) & 1;
         mbar_wait(&empty_bar[stage], phase ^ 1);
-        if (kb < 64) BT_STAMP(8 * kb + 6);
         const uint32_t sb = sbase + stage * STAGE_BYTES + 2 * A_BYTES;
         mbar_expect_tx(&full_bar[stage], b_boxes * 4096);
         for (int b = 0; b < b_boxes; ++b)
@@ -201,7 +186,6 @@ grouped_tc_kernel(const __grid_constant__ CUtensorMap tmIn, GroupedArgs p) {
       for (int kb = 0; kb < num_kb; ++kb) {
         const int stage = kb % STAGES, phase = (kb / STAGES) & 1;
         mbar_wait(&split_bar[stage], phase);
-        if (kb < 64) BT_STAMP(8 * kb + 4);
         tc_fence_after();
         const uint32_t sa = sbase + stage * STAGE_BYTES, sa_lo = sa + A_BYTES;
         const uint32_t sb = sa + 2 * A_BYTES, sb_lo = sb + B_BYTES;
@@ -214,7 +198,6 @@ grouped_tc_kernel(const __grid_constant__ CUtensorMap tmIn, GroupedArgs p) {
           umma_tf32(tmem_base, a_hi, b_hi, idesc, 1);
         }
         umma_commit(&empty_bar[stage]);
-        if (kb < 64) BT_STAMP(8 * kb + 5);
       }
       umma_commit(tmem_full_bar);
     }
@@ -313,13 +296,10 @@ grouped_tc_kernel(const __grid_constant__ CUtensorMap tmIn, GroupedArgs p) {
       const uint32_t st = sbase + stage * STAGE_BYTES;
       if (lane == 0) mbar_wait(&empty_bar[stage], phase ^ 1);
       __syncwarp();
-      if (wt == 0 && kb < 64) BT_STAMP(8 * kb);
 #pragma unroll
       for (int t = 0; t < CPT; ++t) split_store(st + aoff[t], st + A_BYTES + aoff[t], v[t]);
       load_a(kb + AHEAD, v);             // AHEAD k-blocks ahead of their use
-      if (wt == 0 && kb < 64) BT_STAMP(8 * kb + 1);
       mbar_wait(&full_bar[stage], phase);  // every lane: the TMA bytes are read right below
-      if (wt == 0 && kb < 64) BT_STAMP(8 * kb + 2);
       const int valid = n - kb * BK;     // contraction rows of this k-block that belong to the graph
       const uint32_t sb = st + 2 * A_BYTES + 16 * wt;
       float4 x[CPT];
@@ -334,8 +314,6 @@ grouped_tc_kernel(const __grid_constant__ CUtensorMap tmIn, GroupedArgs p) {
       asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");  // generic-proxy writes -> tensor-core reads
       __syncwarp();
       if (lane == 0) mbar_arrive(&split_bar[stage]);
-      if (wt == 0 && kb < 64) BT_STAMP(8 * kb + 3);
-      if (wt == WORKERS - 32 && kb < 64) BT_STAMP(8 * kb + 7);
     };
     float4 va[CPT], vb[CPT], vc[CPT], vd[CPT];   // AHEAD register buffers, one per k-block in flight
     load_a(0, va);
@@ -352,7 +330,6 @@ grouped_tc_kernel(const __grid_constant__ CUtensorMap tmIn, GroupedArgs p) {
     if (lane == 0) mbar_wait(tmem_full_bar, 0);
     __syncwarp();
     tc_fence_after();
-    if (wt == 0) BT_STAMP(521);
     const int q = warp & 3;      // TMEM lane quarter of this warp
     const int h = ww >> 2;       // 32-column group of this warp (NW / 4 groups)
     // The operand stages are free now: the accumulator barrier fires after the last MMA, which waited for every warp's
@@ -402,7 +379,6 @@ grouped_tc_kernel(const __grid_constant__ CUtensorMap tmIn, GroupedArgs p) {
   }
   tc_fence_before();
   __syncthreads();
-  if (threadIdx.x == 0) BT_STAMP(522);
   if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 128;\n" ::"r"(tmem_base) : "memory");
 }
 
@@ -692,7 +668,6 @@ struct PairTcArgs {
   float* resW;                   //      optional
   float* rowpart;                //      optional [R][ncb] row sums of W per 64-column block
   int ncb;
-  int nofix;                     //      A/B builds only: skip the direct-difference fix-up (timing experiment)
 };
 
 template <bool DL>
@@ -931,7 +906,6 @@ pair_tcu_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
           }
           v[u] = d2;
         }
-        if (p.nofix) flagged = 0u;
 #pragma unroll
         for (int u = 0; u < 8; ++u)
           sts128(stg + 4 * (lane * 36 + 4 * u), make_float4(v[4 * u], v[4 * u + 1], v[4 * u + 2], v[4 * u + 3]));
@@ -1161,19 +1135,7 @@ static EncodeTiledFn encode_fn() {
 
 }  // namespace bt
 
-// AGCN_BIG_TC=0 sends every row-tiled product back to the SIMT kernel (A/B runs: tools/gpu_check.sh)
-#define AGCN_BIG_TC_DEFAULT 1
-static bool big_paths_on() {
-  static const bool on = [] {
-    const char* e = ab_env("AGCN_BIG_TC");
-    return e ? atoi(e) != 0 : AGCN_BIG_TC_DEFAULT != 0;
-  }();
-  return on;
-}
-
 bool grouped_tc_supported(const GroupedArgs& g) {
-  static const bool off = ab_env("AGCN_DISABLE_TCGEN05") != nullptr;
-  if (off || !big_paths_on()) return false;
   auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
   if (g.F < 16 || (g.F & 3)) return false;
   return al16(g.In) && al16(g.Out) && al16(g.Out2) && al16(g.Add) && al16(g.Sub) && al16(g.ScaleIn);
@@ -1245,9 +1207,8 @@ int grouped_tc(const agcn_plan* plan, int tiles, const GroupedArgs& g, cudaStrea
 
 // ---- pair matrices of big equal-size graphs on the tensor cores (see pair_tcu_kernel)
 bool pair_tc_supported(const agcn_plan* plan, int F) {
-  static const bool off = ab_env("AGCN_DISABLE_TCGEN05") != nullptr;
   const int un = plan->uniform_n;
-  return !off && big_paths_on() && un > 0 && un % bt::TM == 0 && F % bt::BK == 0 && F >= bt::BK && F <= 256 && plan->big_tiles == plan->large_tiles &&
+  return un > 0 && un % bt::TM == 0 && F % bt::BK == 0 && F >= bt::BK && F <= 256 && plan->big_tiles == plan->large_tiles &&
          plan->big_tiles > 0 && (long long)plan->B * un * 8 < (1ll << 31);
 }
 
@@ -1309,7 +1270,6 @@ int pair_tc_similarity(const agcn_plan* plan, const float* XW, int F, float* nor
   if ((rc = pair_map(&m, XW, (uint64_t)plan->R, F))) return rc;
   PairTcArgs k{};
   k.F = F; k.S = 1; k.mode = 0;
-  k.nofix = ab_env("AGCN_PAIR_NOFIX") != nullptr;
   k.XW = XW; k.mu = mu; k.norms = norms; k.dist = dist; k.resW = resW; k.rowpart = rowpart; k.ncb = ncb;
   return pair_launch(plan, m, m, m, k, "bt::pair_tcu_kernel<SIM>", st);
 }
@@ -1330,7 +1290,7 @@ int pair_tc_dL(const agcn_plan* plan, const float* U, const float* X, const floa
 }
 
 bool grouped_thin_supported(const GroupedArgs& g) {
-  return big_paths_on() && g.F >= 1 && g.F <= 8;
+  return g.F >= 1 && g.F <= 8;
 }
 
 int grouped_thin(int tiles, const GroupedArgs& g, cudaStream_t st) {

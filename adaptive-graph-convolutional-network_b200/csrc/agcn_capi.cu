@@ -652,19 +652,6 @@ int agcn_node_gemm(const float* d_A, int32_t lda, const float* d_B, int32_t ldb,
   return node_gemm(g, reinterpret_cast<float*>(d_scratch), (cudaStream_t)stream);
 }
 
-/* bench.py's roofline: CUDA-event timing of the fused forward kernel on its launching stream */
-int agcn_fused_profile(int enable) {
-  fused_profile_enable(enable);
-  return AGCN_OK;
-}
-int agcn_fused_profile_read(float* ms_sum, int* launches) { return fused_profile_read(ms_sum, launches); }
-
-/* tuning aid: per-tile timeline (nanosecond stamps) of the fused forward kernel; NULL switches it off */
-int agcn_fused_debug_set(void* d_buf) {
-  fused_debug_set(d_buf);
-  return AGCN_OK;
-}
-
 int agcn_sgcll_host_scratch_bytes(const agcn_sgcll_desc* desc, const agcn_plan* plan, size_t* bytes) {
   AGCN_REQUIRE(desc && plan && bytes, "null pointer");
   *bytes = carve_host(desc, plan, nullptr).bytes;

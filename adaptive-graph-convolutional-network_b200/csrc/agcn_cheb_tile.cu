@@ -80,17 +80,7 @@ struct CtArgs {
   const float* G;              // backward [K][R][F]  G_z = dYpre W_z^T
   long long gslice;
   float* dX;                   //          [R, F]
-  unsigned long long* dbg;     // tuning aid: [CTA][128] nanosecond stamps in slots 100.. (agcn_fused_debug_set), NULL in production
 };
-
-#define CT_STAMP(slot)                                                                  \
-  do {                                                                                  \
-    if (p.dbg && threadIdx.x == 0) {                                                    \
-      unsigned long long t__;                                                           \
-      asm volatile("mov.u64 %0, %%globaltimer;\n" : "=l"(t__));                         \
-      p.dbg[(long long)blockIdx.x * 128 + (slot)] = t__;                                \
-    }                                                                                   \
-  } while (0)
 
 struct Row {
   int grow;   // packed row or -1
@@ -120,7 +110,7 @@ __device__ __forceinline__ Row prologue(const CtArgs& p, int tile, int r, uint32
   const int tid = threadIdx.x, nthreads = blockDim.x;
   if (TILE) {
     // ONE warp fetches the tile's graph list: with every thread of 444 resident CTAs reading the same few cache lines of
-    // the plan tables, the first phase of the kernel took 5 us (tools/rows_timeline.py, cheb stamps)
+    // the plan tables, the first phase of the kernel took 5 us (per-CTA globaltimer timeline)
     if (tid < 32) {
       int gs = 0, ge = 0;
       if (tid == 0) {
@@ -317,9 +307,7 @@ __global__ void __launch_bounds__(TILE ? 256 : 320, TILE ? 3 : 1) cheb_tile_fwd_
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, wpr = rows >> 5;
   const int h = warp / wpr, r = (warp - h * wpr) * 32 + lane;
   const int F = p.F, K = p.K;
-  CT_STAMP(100);
   const Row me = prologue<TILE>(p, tile, r, s_glist, sL);
-  CT_STAMP(101);
   const bool vec = ((F & 3) == 0) && ((reinterpret_cast<uintptr_t>(p.X) & 15) == 0) &&
                    ((reinterpret_cast<uintptr_t>(p.T) & 15) == 0) && ((p.tslice & 3) == 0);
   // my row of the graph's matrix, or (transL) my column: (L^T V)_i = sum_j L[j][i] V_j
@@ -353,14 +341,11 @@ __global__ void __launch_bounds__(TILE ? 256 : 320, TILE ? 3 : 1) cheb_tile_fwd_
       }
       cp_async_commit();
     }
-    if (c == c_beg) CT_STAMP(102);
     cp_async_wait_all();
     __syncthreads();  // (first chunk: the L matrices and) the T_0 chunk of every row have landed
     if (c == c_beg) {
-      CT_STAMP(103);
       mask = nonzero_mask<MW>(lrow, lstep, me.n);
       masked = prefer_masked<MW>(mask, me.n);
-      CT_STAMP(104);
     }
     float tm1[16], tm2[16];
     read_seg(buf0, r, h, tm1);
@@ -387,7 +372,6 @@ __global__ void __launch_bounds__(TILE ? 256 : 320, TILE ? 3 : 1) cheb_tile_fwd_
       }
 #pragma unroll
       for (int u = 0; u < 16; ++u) { tm2[u] = tm1[u]; tm1[u] = t[u]; }
-      if (c == c_beg) CT_STAMP(104 + s);
     }
     if (c + 1 < c_end) __syncthreads();  // the last step's reads are done before the next chunk lands in buf0
   }
@@ -455,8 +439,6 @@ __global__ void __launch_bounds__(TILE ? 256 : 320, TILE ? 3 : 1) cheb_tile_bwd_
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-static unsigned long long* g_dbg = nullptr;
-
 static size_t smem_bytes(int rows, int lfloats, bool tile) {
   return (size_t)2 * rows * CPITCH + (size_t)lfloats * 4 + (tile ? 128 * 32 + 16 : 0) + 64;
 }
@@ -473,7 +455,6 @@ static CtArgs base_args(const agcn_plan* plan, const float* L, int add_identity,
   a.order = plan->d_order; a.n_nodes = plan->d_n; a.node_off = plan->d_node_off; a.lap_off = plan->d_lap_off;
   a.chunks = (F + CH - 1) / CH;
   a.L = L; a.add_identity = add_identity; a.F = F; a.K = K;
-  a.dbg = g_dbg;
   return a;
 }
 
@@ -542,8 +523,6 @@ static int launch(const agcn_plan* plan, CtArgs a, bool forward, cudaStream_t st
 }
 
 }  // namespace ct
-
-void cheb_debug_set(void* d_buf) { ct::g_dbg = reinterpret_cast<unsigned long long*>(d_buf); }
 
 bool cheb_tiles_has_mid(const agcn_plan* plan) { return ct::mid_bucket(plan) != nullptr; }
 

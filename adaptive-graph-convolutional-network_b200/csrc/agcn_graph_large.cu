@@ -192,12 +192,6 @@ int grouped_rows_gemm(const agcn_plan* plan, int tiles, const float* Lmat, const
 
 // Tuning / debugging aid (include/agcn_sgcll.h): one row-tiled product over every graph above cheb_small_max,
 // impl 0 = dispatcher, 1 = SIMT, 2 = tensor cores, 3 = thin.
-static unsigned long long* g_grouped_dbg = nullptr;
-extern "C" int agcn_debug_grouped_timeline(void* d_buf) {
-  g_grouped_dbg = reinterpret_cast<unsigned long long*>(d_buf);
-  return AGCN_OK;
-}
-
 extern "C" int agcn_debug_grouped_product(const agcn_plan* plan, const float* d_L, const float* d_In, float* d_Out,
                                           int32_t F, int32_t transL, int32_t add_identity, float cmul, int32_t impl,
                                           void* stream) {
@@ -208,7 +202,6 @@ extern "C" int agcn_debug_grouped_product(const agcn_plan* plan, const float* d_
   GroupedArgs g = base_args(plan);
   g.L = d_L; g.add_identity = add_identity; g.transL = transL;
   g.In = d_In; g.Sub = nullptr; g.Add = nullptr; g.Out = d_Out; g.Out2 = nullptr; g.cmul = cmul; g.F = F;
-  g.dbg = g_grouped_dbg;
   const int tiles = plan->large_tiles;
   if (tiles == 0) return AGCN_OK;
   switch (impl) {

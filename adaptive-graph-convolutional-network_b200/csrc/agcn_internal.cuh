@@ -74,16 +74,6 @@ struct Bucket {
   int limit;  // upper size limit of the bucket (every graph of the bucket has n <= limit)
 };
 
-// A/B tuning switches (AGCN_DISABLE_TCGEN05, AGCN_DISABLE_FUSED, AGCN_BIG_TC, AGCN_CHEB_SMALL_MAX) exist only in builds
-// made with -DAGCN_AB_SWITCHES (tools/gpu_check.sh); the shipped library has ONE code path per shape and reads no
-// environment variables.
-#ifdef AGCN_AB_SWITCHES
-#include <cstdlib>
-inline const char* ab_env(const char* name) { return getenv(name); }
-#else
-inline const char* ab_env(const char*) { return nullptr; }
-#endif
-
 void set_error(const std::string& msg);
 int cuda_fail(cudaError_t e, const char* what, const char* file, int line);
 extern std::atomic<uint64_t> g_launches;
@@ -114,7 +104,7 @@ extern std::atomic<uint64_t> g_launches;
 struct agcn_plan {
   int32_t B = 0, Nmax = 0, max_n = 0;
   int32_t uniform_n = 0;   // n when every graph of the batch has the same size (then node_off[g] = g n, lap_off[g] = g n^2), else 0
-  int32_t cheb_small_max = AGCN_CHEB_SMALL_MAX;  // overridable with the environment variable of the same name
+  int32_t cheb_small_max = AGCN_CHEB_SMALL_MAX;  // agcn_plan_create lowers it to AGCN_FUSE_MAX_N when mid-size graphs dominate the batch
   int64_t R = 0;   // total nodes
   int64_t LL = 0;  // total n^2
   std::vector<int32_t> n, node_off, order;
@@ -321,7 +311,6 @@ struct GroupedArgs {
   int F;
   const float* RowScale;  // optional: Out += RowScale[row] * ScaleIn[row, c]
   const float* ScaleIn;
-  unsigned long long* dbg;  // tuning aid: timeline of the first CTA of grouped_tc_kernel (NULL in production)
   int force_uniform;        // tests: take bt::grouped_tcu_kernel whenever the batch is eligible, whatever the grid size
 };
 int grouped_launch(const agcn_plan* plan, int tiles, const GroupedArgs& g, cudaStream_t st);
@@ -341,10 +330,7 @@ int grouped_thin(int tiles, const GroupedArgs& g, cudaStream_t st);
 
 // ---------------------------------------------------------------- tile path of a layer: parameter operands and shape
 // rules (agcn_layer_operands.cu); recurrences in agcn_cheb_tile.cu, contraction in agcn_pre_tile.cu
-void fused_profile_enable(int on);
-int fused_profile_read(float* ms_sum, int* launches);
 void prof_enable(int on);
-void fused_debug_set(void* d_buf);  // per-CTA timeline buffer [CTAs][128] uint64 of the NEXT contraction / recurrence launches, or NULL
 bool fused_fwd_supported(const agcn_plan* plan, int F, int Fo, int K);
 bool fused_bwd_supported(const agcn_plan* plan, int F, int Fo, int K);
 size_t fused_w_floats(int Nv, int Kv, int Z);  // floats of one pre-split parameter operand

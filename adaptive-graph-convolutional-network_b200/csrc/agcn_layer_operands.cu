@@ -40,28 +40,14 @@ static int pad32(int x) { return (x + 31) & ~31; }
 // ------------------------------------------------------------------------------------------------
 // host API
 // ------------------------------------------------------------------------------------------------
-void rows_debug_set(void* d_buf);
-void cheb_debug_set(void* d_buf);
-// per-CTA timeline buffer [CTAs][128] uint64 of the NEXT launches of the contraction (slots 0..) and of the recurrence
-// tiles (slots 100..), or NULL
-void fused_debug_set(void* d_buf) {
-  rows_debug_set(d_buf);
-  cheb_debug_set(d_buf);
-}
-
-bool fused_enabled() {
-  static const bool off = ab_env("AGCN_DISABLE_FUSED") != nullptr || ab_env("AGCN_DISABLE_TCGEN05") != nullptr;
-  return !off;
-}
-
 // forward: one accumulator of pad16(Fo) <= 128 columns
 bool fused_fwd_supported(const agcn_plan* plan, int F, int Fo, int K) {
-  return fused_enabled() && plan->ft_tiles > 0 && K >= 2 && Fo >= 1 && Fo <= 128 && F >= 1;
+  return plan->ft_tiles > 0 && K >= 2 && Fo >= 1 && Fo <= 128 && F >= 1;
 }
 
 // backward: K accumulators of pad16(F) columns within the 512 TMEM columns
 bool fused_bwd_supported(const agcn_plan* plan, int F, int Fo, int K) {
-  if (!fused_enabled() || plan->ft_tiles <= 0 || K < 2 || F > 128) return false;
+  if (plan->ft_tiles <= 0 || K < 2 || F > 128) return false;
   const int N = ft::pad16(F), stride = N <= 32 ? 32 : (N <= 64 ? 64 : 128);
   return K * stride <= 512;
 }

@@ -1,7 +1,6 @@
 // Batch topology ("plan") and layout conversion between the reference's zero-padded wire layout
 // (models/tf_modules/graph_topology.py:84-135) and the packed HBM layout of this library.
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 #include <numeric>
@@ -88,7 +87,7 @@ __global__ void pack_lap_kernel(const float* __restrict__ padded, float* __restr
 
 // Padded -> packed over the REAL rows only (the direction every training step takes).  When the padded array is a pinned
 // host buffer read in place over PCIe, the kernel lives for the PCIe transfer time beside the previous training step.
-// Three measurements of round 2 (tools/pack_time.py, tools/pack_sweep.sh, tools/e2e_host_split.py) shaped it:
+// Three measurements of round 2 (tools/pack_time.py, a pack-grid sweep, tools/e2e_host_split.py) shaped it:
 //  1. A zero-copy read crosses PCIe per L2 sector group: unaligned scalar row reads decay to 32-byte requests and the
 //     link's outstanding-read tags saturate at ~18 GB/s whatever the number of threads; whole aligned 128-byte lines
 //     (eight lanes x float4, elements outside the segment dropped) reach 40 GB/s.
@@ -217,13 +216,12 @@ __global__ void __launch_bounds__(1024) pack_rows_kernel(const float* __restrict
   }
 }
 
-// grid of the pack kernels (finding 3 above; A/B builds: AGCN_PACK_CTAS / AGCN_PACK_THREADS override)
+// grid of the pack kernels (finding 3 above)
 constexpr int PACK_CTAS = 2, PACK_THREADS = 1024;
 static void pack_shape(int64_t warp_items, unsigned* ctas, unsigned* threads) {
-  static const int c = ab_env("AGCN_PACK_CTAS") ? atoi(ab_env("AGCN_PACK_CTAS")) : PACK_CTAS;
-  static const int t = ab_env("AGCN_PACK_THREADS") ? atoi(ab_env("AGCN_PACK_THREADS")) : PACK_THREADS;
-  *threads = (unsigned)t;
-  *ctas = (unsigned)std::max<int64_t>(1, std::min<int64_t>((std::max<int64_t>(1, warp_items) * 32 + t - 1) / t, c));
+  *threads = (unsigned)PACK_THREADS;
+  *ctas = (unsigned)std::max<int64_t>(
+      1, std::min<int64_t>((std::max<int64_t>(1, warp_items) * 32 + PACK_THREADS - 1) / PACK_THREADS, PACK_CTAS));
 }
 
 static void launch_pack(const agcn_plan* plan, const float* padded, float* packed, int F, int lap, cudaStream_t st) {
@@ -482,7 +480,6 @@ int agcn_plan_create(const int32_t* n_nodes_host, int32_t B, int32_t Nmax, void*
     for (int i = pos; i < B && p->n[p->order[i]] > AGCN_FUSE_MAX_N; ++i) ++mid;
     if (mid >= AGCN_MID_TILED_MIN) p->cheb_small_max = AGCN_FUSE_MAX_N;
   }
-  if (const char* e = ab_env("AGCN_CHEB_SMALL_MAX")) p->cheb_small_max = std::min(AGCN_SMALL_MAX, std::max(16, atoi(e)));
   for (int i = 0; i < B && p->n[p->order[i]] > p->cheb_small_max; ++i) {
     const int g = p->order[i];
     if (i <= p->large_count) p->big_tile_start.push_back((int32_t)p->tile_graph.size());

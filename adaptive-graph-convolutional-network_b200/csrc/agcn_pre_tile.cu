@@ -405,7 +405,7 @@ pre_tile_kernel(const __grid_constant__ CUtensorMap tmBhi, const __grid_constant
 // the backward direction) and write them into an operand slot in TENSOR MEMORY (tcgen05.st; the MMAs take A from TMEM):
 //  * a tf32 MMA with both operands in shared memory reads 8 KB per 64 cycles at N = 128 -- all of the SM's 128 B/clk --
 //    so the workers' own loads / stores and the TMA writes of the next tiles fought the tensor core for the same port
-//    (rows_timeline: 1.0 us to split and store one 16 KB item, 1.4 us per item against 0.4 us of MMA work);
+//    (per-CTA globaltimer timeline: 1.0 us to split and store one 16 KB item, 1.4 us per item against 0.4 us of MMA work);
 //  * with A in tensor memory the MMAs read only the parameter tile (64 B/clk) and the workers never write shared memory,
 //    so no proxy fence at all.
 // Every dYpre chunk is split ONCE and multiplied with its K parameter tiles.  Requires Fin % 32 == 0, 16-byte aligned
@@ -427,17 +427,7 @@ struct RowsArgs {
   int act;
   float* Out;                  // forward: Y; backward: G [K][R][Fout]
   long long out_slice;
-  unsigned long long* dbg;     // tuning aid: [tiles][128] nanosecond stamps (agcn_fused_debug_set), NULL in production
 };
-
-#define RG_STAMP(slot)                                                                  \
-  do {                                                                                  \
-    if (p.dbg) {                                                                        \
-      unsigned long long t__;                                                           \
-      asm volatile("mov.u64 %0, %%globaltimer;\n" : "=l"(t__));                         \
-      p.dbg[(long long)blockIdx.x * 128 + (slot)] = t__;                                \
-    }                                                                                   \
-  } while (0)
 
 // D[tmem] (+)= A[tmem] * B[smem]   (A: lane = row, one 32-bit column per K element)
 __device__ __forceinline__ void umma_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
@@ -494,7 +484,6 @@ rows_gemm_kernel(const __grid_constant__ CUtensorMap tmBhi, const __grid_constan
   const int nb = FWD ? 1 : (split ? 1 : K);     // parameter tiles per item
 
   if (threadIdx.x == 0) {
-    RG_STAMP(0);
     for (int s = 0; s < 4; ++s) {
       mbar_init(&a_full[s], WORKERS / 32);
       mbar_init(&a_empty[s], 1);
@@ -521,7 +510,6 @@ rows_gemm_kernel(const __grid_constant__ CUtensorMap tmBhi, const __grid_constan
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  if (threadIdx.x == 0) RG_STAMP(1);
 
   if (warp == 0) {
     // ================= TMA producer of the parameter tiles =================
@@ -574,13 +562,11 @@ rows_gemm_kernel(const __grid_constant__ CUtensorMap tmBhi, const __grid_constan
       for (int i = 0; i < items; ++i) {
         const int aslot = i % NA;
         mbar_wait(&a_full[aslot], (uint32_t)((i / NA) & 1));
-        if (i < 12) RG_STAMP(40 + 3 * i);
         tc_fence_after();
         const uint32_t ta_hi = tmem_base + (uint32_t)(p.a_col0 + aslot * 2 * CH), ta_lo = ta_hi + CH;
         for (int j = 0; j < nb; ++j, ++bi) {
           const int slot = bi % NB;
           mbar_wait(&b_full[slot], (uint32_t)((bi / NB) & 1));
-          if (i < 12 && j == 0) RG_STAMP(41 + 3 * i);
           tc_fence_after();
           const uint32_t sw = b_ring + (uint32_t)(slot * 2 * w_bytes), sw_lo = sw + w_bytes;
           const uint32_t acc = tmem_base + (uint32_t)(FWD ? 0 : (z0 + j) * p.acc_stride);
@@ -595,7 +581,6 @@ rows_gemm_kernel(const __grid_constant__ CUtensorMap tmBhi, const __grid_constan
           umma_commit(&b_empty[slot]);
         }
         umma_commit(&a_empty[aslot]);
-        if (i < 12) RG_STAMP(42 + 3 * i);
       }
       umma_commit(out_bar);
     }
@@ -612,9 +597,7 @@ rows_gemm_kernel(const __grid_constant__ CUtensorMap tmBhi, const __grid_constan
       const int sslot = i % NS, aslot = i % NA;
       if (lane == 0) {
         mbar_wait(&s_full[sslot], (uint32_t)((i / NS) & 1));
-        if (wi == 0 && i < 12) RG_STAMP(4 + 3 * i);
         if (i >= NA) mbar_wait(&a_empty[aslot], (uint32_t)((i / NA - 1) & 1));
-        if (wi == 0 && i < 12) RG_STAMP(5 + 3 * i);
       }
       __syncwarp();
       const uint32_t st = s_ring + (uint32_t)(sslot * stage_bytes);
@@ -647,12 +630,10 @@ rows_gemm_kernel(const __grid_constant__ CUtensorMap tmBhi, const __grid_constan
       if (lane == 0) {
         mbar_arrive(&s_empty[sslot]);   // the staged tile is consumed (its values are in registers / tensor memory)
         mbar_arrive(&a_full[aslot]);
-        if (wi == 0 && i < 12) RG_STAMP(6 + 3 * i);
       }
     }
     // ---- drain
     if (lane == 0) mbar_wait(out_bar, 0);
-    if (wi == 0 && lane == 0) RG_STAMP(2);
     __syncwarp();
     tc_fence_after();
     const int Fout = p.Fout;
@@ -689,7 +670,6 @@ rows_gemm_kernel(const __grid_constant__ CUtensorMap tmBhi, const __grid_constan
   }
   tc_fence_before();
   __syncthreads();
-  if (threadIdx.x == 0) RG_STAMP(3);
   if (warp == 1) {
     switch (p.tmem_cols) {
       case 32: asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 32;\n" ::"r"(tmem_base) : "memory"); break;
@@ -743,9 +723,6 @@ static int make_map(CUtensorMap* map, const float* ptr, uint64_t rows, uint64_t 
 static int pad16(int x) { return (x + 15) & ~15; }
 static int pad32(int x) { return (x + 31) & ~31; }
 
-static void* g_rows_dbg = nullptr;
-static void* rows_debug_buffer() { return g_rows_dbg; }
-
 // fast path of the all-rows contraction: full 32-column chunks, 16-byte aligned rows, accumulators within TMEM
 static bool rows_fast(const PreArgs& a) {
   auto al = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
@@ -769,7 +746,6 @@ static int launch_rows(const agcn_plan* plan, const PreArgs& a, const CUtensorMa
   r.tmem_cols = tm;
   r.has_mask = (!a.forward && a.Mask) ? 1 : 0;
   r.bias = a.bias; r.act = a.act; r.Out = a.Out; r.out_slice = a.out_slice;
-  r.dbg = reinterpret_cast<unsigned long long*>(rows_debug_buffer());
   // raw row tiles: [R, Fin] views of the operand matrices, box = 32 columns x 128 rows (rows beyond the tensor: zeros)
   CUtensorMap min, maux;
   int rc;
@@ -852,8 +828,6 @@ static int launch(const agcn_plan* plan, int tile0, int ntiles, PreArgs& a, cons
 }
 
 }  // namespace pt
-
-void rows_debug_set(void* d_buf) { pt::g_rows_dbg = d_buf; }
 
 // Y = act(sum_s T_s W_s + b) over the 128-row ranges [tile0, tile0 + ntiles) of the plan's tile list, or (tile0 < 0) over
 // every packed row; wsplit = the pre-split W_s of fused_fwd_prep

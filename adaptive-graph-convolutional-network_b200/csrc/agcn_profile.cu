@@ -49,16 +49,14 @@ ProfScope::~ProfScope() {
 
 void prof_enable(int on) { g_prof_on.store(on ? 1 : 0); }
 
-// Drains the pending records.  only != NULL: sum of the records of that kernel name (the others are dropped).
-int prof_drain(const char* only, float* ms_sum, int* launches, std::string* table, std::string* timeline = nullptr) {
+// Drains the pending records into a per-kernel table and, if asked, a launch timeline.
+int prof_drain(std::string* table, std::string* timeline = nullptr) {
   std::vector<ProfRec> recs;
   {
     std::lock_guard<std::mutex> lock(g_prof_mu);
     recs.swap(g_prof_recs);
   }
   std::map<std::string, std::pair<int, double>> agg;
-  float total = 0.f;
-  int n = 0;
   if (timeline) timeline->clear();
   for (ProfRec& r : recs) {
     float ms = 0.f;
@@ -77,14 +75,8 @@ int prof_drain(const char* only, float* ms_sum, int* launches, std::string* tabl
     auto& a = agg[r.name];
     a.first += 1;
     a.second += ms;
-    if (only && std::string(only) == r.name) {
-      total += ms;
-      ++n;
-    }
   }
   for (ProfRec& d : recs) { cudaEventDestroy(d.e0); cudaEventDestroy(d.e1); }
-  if (ms_sum) *ms_sum = total;
-  if (launches) *launches = n;
   if (table) {
     table->clear();
     for (auto& kv : agg) *table += kv.first + "\t" + std::to_string(kv.second.first) + "\t" + std::to_string(kv.second.second) + "\n";
@@ -105,9 +97,6 @@ __global__ void __launch_bounds__(256) fma_probe_kernel(float* __restrict__ sink
   sink[(size_t)blockIdx.x * blockDim.x + threadIdx.x] = ((a0 + a1) + (a2 + a3)) + ((a4 + a5) + (a6 + a7));
 }
 
-void fused_profile_enable(int on) { prof_enable(on); }
-int fused_profile_read(float* ms_sum, int* launches) { return prof_drain("pt::rows_gemm_kernel(fwd)", ms_sum, launches, nullptr); }
-
 }  // namespace agcn
 
 extern "C" {
@@ -126,7 +115,7 @@ int agcn_probe_fp32_fma(float* d_sink, int32_t iters, void* stream) {
 
 int agcn_profile_timeline(char* buf, size_t cap, size_t* needed) {
   std::string table, timeline;
-  int rc = agcn::prof_drain(nullptr, nullptr, nullptr, &table, &timeline);
+  int rc = agcn::prof_drain(&table, &timeline);
   if (rc) return rc;
   if (needed) *needed = timeline.size() + 1;
   if (buf && cap) {
@@ -139,7 +128,7 @@ int agcn_profile_timeline(char* buf, size_t cap, size_t* needed) {
 
 int agcn_profile_read(char* buf, size_t cap, size_t* needed) {
   std::string table;
-  int rc = agcn::prof_drain(nullptr, nullptr, nullptr, &table);
+  int rc = agcn::prof_drain(&table);
   if (rc) return rc;
   if (needed) *needed = table.size() + 1;
   if (buf && cap) {

@@ -15,10 +15,8 @@
 // Used for Y = act(sum_k T_k W_k + b) (graphconv.py:238-247), G_k = dY W_k^T, XW = X M_L
 // (graphconv.py:164) and dX += dXW M_L^T.
 #include <cuda.h>
-#include <cstdio>
 
 #include <algorithm>
-#include <cstdlib>
 #include <mutex>
 
 #include "agcn_internal.cuh"
@@ -515,15 +513,6 @@ tc_gemm_tn_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
           lo_p[idx] = lo;
         }
       };
-#ifdef AGCN_TN_DEBUG
-      if (t == 0 && blockIdx.x == 0 && kb == 0) {
-        const float* fa = reinterpret_cast<const float*>(st);
-        const float* fb = reinterpret_cast<const float*>(st + 2 * SM::A_BYTES);
-        printf("TNDBG a_boxes %d b_boxes %d num_kb %d A: %f %f %f %f | row1 %f %f %f %f | B: %f %f %f %f row1 %f %f\n", a_boxes,
-               b_boxes, num_kb, fa[0], fa[1], fa[2], fa[3], fa[32], fa[33], fa[34], fa[35], fb[0], fb[1], fb[2], fb[3],
-               fb[32], fb[33]);
-      }
-#endif
       split(reinterpret_cast<float4*>(st), reinterpret_cast<float4*>(st + SM::A_BYTES), a_boxes * 256);
       split(reinterpret_cast<float4*>(st + 2 * SM::A_BYTES),
             reinterpret_cast<float4*>(st + 2 * SM::A_BYTES + SM::B_BYTES), b_boxes * 256);
@@ -550,11 +539,6 @@ tc_gemm_tn_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constan
             "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
           : "r"(taddr));
       asm volatile("tcgen05.wait::ld.sync.aligned;\n" ::: "memory");
-#ifdef AGCN_TN_DEBUG
-      if (blockIdx.x == 0 && c0 == 0 && lane < 2)
-        printf("TNDBG tmem q %d lane %d: %f %f %f %f\n", q, lane, __uint_as_float(v[0]), __uint_as_float(v[1]),
-               __uint_as_float(v[2]), __uint_as_float(v[3]));
-#endif
 #pragma unroll
       for (int u = 0; u < 8; ++u)
         *reinterpret_cast<float4*>(&stg[lane * 36 + 4 * u]) =
@@ -674,7 +658,6 @@ static int tc_npad(int N) { return N <= 64 ? 64 : (N + 127) / 128 * 128; }
 static int tc_kpitch(int Kd) { return (Kd + 3) & ~3; }
 
 bool tc_gemm_supported(const GemmArgs& a) {
-  if (ab_env("AGCN_DISABLE_TCGEN05")) return false;
   auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
   if (a.M < 1 || a.Kd < 32) return false;
   if (a.S > 1 && a.Kd % 4 != 0) return false;  // stacked slices share one tensor map
@@ -814,7 +797,6 @@ int tc_gemm(const GemmArgs& a, const float* scratch, cudaStream_t st) {
 namespace agcn {
 
 bool tc_gemm_tn_supported(const GemmTNArgs& a) {
-  if (ab_env("AGCN_DISABLE_TCGEN05") || ab_env("AGCN_DISABLE_TCGEN05_TN")) return false;
   auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
   if (a.M < 32 || a.Kd > 128 || a.Kd % 4 != 0 || a.N % 4 != 0) return false;
   if (a.lda0 % 4 != 0 || a.ldd % 4 != 0 || !al16(a.A0) || !al16(a.D)) return false;

@@ -102,17 +102,11 @@ const int64_t* agcn_plan_lap_off_host(const agcn_plan* plan);  /* [B+1] host   *
 int agcn_fused_tiles_host(const int32_t* n_nodes_host, int32_t B, int32_t* gstart_out, int32_t gstart_cap,
                           int32_t* entries_out, int32_t entries_cap, int32_t* tiles_out, int32_t* n_entries_out);
 
-/* Measurement aid (no reference counterpart; bench.py's roofline): while enabled, every eager agcn_sgcll_forward on
- * the tile path brackets the launch of its tensor-core contraction with CUDA events on the launching stream;
- * agcn_fused_profile_read waits for them and returns the summed duration (ms) and the number of launches since
- * the last read.  Must be off during CUDA graph capture. */
-int agcn_fused_profile(int enable);
-int agcn_fused_profile_read(float* ms_sum, int* launches);
-
-/* The same for every main kernel of the library (bench.py's per-kernel roofline table): while enabled (and the stream
- * is not capturing) the host wrappers bracket each launch with CUDA events on its stream.  agcn_profile_read waits
- * for them, clears the records and writes one line per kernel, "name<TAB>launches<TAB>milliseconds\n", into buf
- * (NUL-terminated, truncated to cap); *needed receives the size the whole table takes. */
+/* Measurement aid (no reference counterpart; bench.py's per-kernel roofline table): while enabled (and the stream is
+ * not capturing) the host wrappers of the main kernels bracket each launch with CUDA events on its stream.
+ * agcn_profile_read waits for them, clears the records and writes one line per kernel,
+ * "name<TAB>launches<TAB>milliseconds\n", into buf (NUL-terminated, truncated to cap); *needed receives the size the
+ * whole table takes. */
 int agcn_profile_enable(int enable);
 int agcn_profile_read(char* buf, size_t cap, size_t* needed);
 /* The same records as a timeline instead of sums: one line per launch, "name<TAB>start_ms<TAB>end_ms\n", times relative
@@ -123,10 +117,6 @@ int agcn_profile_timeline(char* buf, size_t cap, size_t* needed);
  * 148 * 8 * 256 * 8 * 2 * iters FLOP; d_sink needs 148 * 8 * 256 floats.  The caller times it with CUDA events. */
 int agcn_probe_fp32_fma(float* d_sink, int32_t iters, void* stream);
 
-/* Tuning aid (no reference counterpart): d_buf = device buffer of tiles x 128 uint64; the following fused forward
- * launches record a per-tile timeline of nanosecond stamps into it.  NULL switches the recording off. */
-int agcn_fused_debug_set(void* d_buf);
-
 /* Tuning / debugging aid (no reference counterpart): Out = cmul * op(L_g) In over the rows of every graph with more
  * than AGCN_CHEB_SMALL_MAX nodes (the row-tiled path; other rows of Out are not written), op = L (+I) or L^T (+I);
  * impl 0 = the library's own choice, 1 = SIMT kernel, 2 = tcgen05 kernel (F % 4 == 0, F >= 16), 3 = streaming kernel
@@ -135,10 +125,6 @@ int agcn_fused_debug_set(void* d_buf);
 int agcn_debug_grouped_product(const agcn_plan* plan, const float* d_L /*packed*/, const float* d_In /*[R,F]*/,
                                float* d_Out /*[R,F]*/, int32_t F, int32_t transL, int32_t add_identity, float cmul,
                                int32_t impl, void* stream);
-
-/* d_buf = device buffer of 1024 uint64 (or NULL): the following agcn_debug_grouped_product calls with impl 2 record a
- * nanosecond timeline of their first CTA into it (tools/tc_timeline.py). */
-int agcn_debug_grouped_timeline(void* d_buf);
 
 /* ---- layout conversion (pad_data2sparse / pad_Lap2sparse, graph_topology.py:84-98;
  *      tf.slice at graphconv.py:153-154; tf.pad at graphconv.py:249-251) ------------------ */

@@ -431,10 +431,16 @@ def test_head_loss_and_gradients_match_oracle(Fh, Fm, Nt, kind):
         assert O.rel_err(a.grad.cpu(), b.grad) <= TOL, name
 
 
-@pytest.mark.parametrize("sizes,F", [([256, 256, 256], 64), ([384, 384], 160), ([256], 16), ([1024, 1024], 128)])
-def test_uniform_tensor_core_product(sizes, F):
-    """bt::grouped_tcu_kernel (TMA-staged L tiles, A operand in tensor memory, equal-size graphs) forced through the
-    debug entry, every op(L) variant, against a float64 product on the device."""
+_UNIFORM_SHAPES = [([256, 256, 256], 64), ([384, 384], 160), ([256], 16), ([1024, 1024], 128)]
+
+
+@pytest.mark.parametrize("sizes,F,impl", [(s, F, impl) for s, F in _UNIFORM_SHAPES for impl in (1, 2, 4)] +
+                         [([256, 256], 8, impl) for impl in (1, 3)])
+def test_uniform_tensor_core_product(sizes, F, impl):
+    """Each row-tiled product kernel on equal-size graphs, chosen through the debug entry: impl 1 = the SIMT kernel
+    (grouped_lap_gemm_kernel), 2 = bt::grouped_tc_kernel, 3 = the streaming kernel for F <= 8 (bt::grouped_thin_kernel),
+    4 = bt::grouped_tcu_kernel (TMA-staged L tiles, A operand in tensor memory) forced whatever the grid size.  Every
+    op(L) variant, against a float64 product on the device."""
     import ctypes
     import agcn_b200
     from agcn_b200 import _lib
@@ -457,11 +463,11 @@ def test_uniform_tensor_core_product(sizes, F):
                 ref[r0:r0 + n] = 2.0 * (Lg @ X[r0:r0 + n].double())
             out = torch.full((R, F), float("nan"), device=dev)
             _lib.check(_lib.lib().agcn_debug_grouped_product(batch.handle, _ptr(L), _ptr(X), _ptr(out), F, transL,
-                                                             add_identity, 2.0, 4, _stream_ptr()))
+                                                             add_identity, 2.0, impl, _stream_ptr()))
             torch.cuda.synchronize()
             assert torch.isfinite(out).all()
             err = float((out.double() - ref).abs().max() / ref.abs().max())
-            assert err <= 1e-5, (sizes, F, transL, add_identity, err)
+            assert err <= 1e-5, (sizes, F, impl, transL, add_identity, err)
 
 
 @pytest.mark.parametrize("metric_grad", ["reference", "full"])
