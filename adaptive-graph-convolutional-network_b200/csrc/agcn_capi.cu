@@ -9,24 +9,6 @@ using namespace agcn;
 
 namespace {
 
-// node-level GEMM: tensor cores when the operands are TMA-compatible, CUDA cores otherwise (F = 75)
-int node_gemm_tn(const GemmTNArgs& t, cudaStream_t st) {
-  if (tc_gemm_tn_supported(t)) return tc_gemm_tn(t, st);
-  return gemm_tn(t, st);
-}
-
-// presplit: the hi / lo copies of B in tc_scratch were already produced by tc_gemm_split_b (side stream)
-int node_gemm(const GemmArgs& g, float* tc_scratch, cudaStream_t st, bool presplit = false) {
-  if (tc_gemm_supported(g)) {
-    if (!presplit) {
-      int rc = tc_gemm_split_b(g, tc_scratch, st);
-      if (rc) return rc;
-    }
-    return tc_gemm(g, tc_scratch, st);
-  }
-  return gemm_rows(g, st);
-}
-
 // Y = act(sum_k T_k W_k + b)   graphconv.py:238-247, :118-123
 GemmArgs y_gemm_args(const agcn_sgcll_desc* d, int R, const float* X, const float* T, const float* weight,
                      const float* bias, float* Y) {
@@ -109,15 +91,11 @@ Work carve_work(const agcn_sgcll_desc* d, const agcn_plan* p, void* base) {
   w.dYp = c.take((size_t)p->R * d->Fo);
   w.G = c.take((size_t)d->K * p->R * d->F);
   w.V = c.take((size_t)(d->K > 1 ? d->K - 1 : 0) * p->R * d->Fo);  // V_k = T_k(L^T) dYpre of the recurrence-first backward
-  size_t tn = gemm_tn_partial_floats((int)p->R, d->F, d->Fo, d->K);
-  if (m.full) tn = std::max(tn, gemm_tn_partial_floats((int)p->R, d->F, d->F, 1));
-  {
-    GemmTNArgs t;
-    t.M = (int)p->R; t.Kd = d->F; t.N = d->Fo; t.S = d->K;
-    tn = std::max(tn, tc_gemm_tn_partial_floats(t));
-    t.N = d->F; t.S = 1;
-    tn = std::max(tn, tc_gemm_tn_partial_floats(t));
-  }
+  GemmTNArgs t;  // dweight, and dM_L with metric_grad = full
+  t.M = (int)p->R; t.Kd = d->F; t.N = d->Fo; t.S = d->K;
+  size_t tn = gemm_tn_auto_partial_floats(t);
+  t.N = d->F; t.S = 1;
+  if (m.full) tn = std::max(tn, gemm_tn_auto_partial_floats(t));
   w.tn_part = c.take(tn);
   w.act_part = c.take(act_bwd_partial_floats(p->R, d->Fo));
   w.dL = m.need_dL ? c.take((size_t)dl_parts(d, p) * dl_stride(p)) : nullptr;
@@ -408,7 +386,7 @@ int forward_impl(const agcn_sgcll_desc* desc, const agcn_plan* plan, const float
     g.A0 = d_X; g.lda0 = F;
     g.B = d_M_L; g.ldb = F;
     g.C = XW; g.ldc = F;
-    if ((rc = node_gemm(g, wk.tcM, st))) return rc;
+    if ((rc = gemm_auto(g, wk.tcM, st))) return rc;
   }
   GraphArgs ga;
   ga.plan = plan; ga.F = F; ga.K = K;
@@ -449,7 +427,7 @@ int forward_impl(const agcn_sgcll_desc* desc, const agcn_plan* plan, const float
   if ((rc = graph_chebyshev_fwd(ga, st))) return rc;  // graphconv.py:221-236
   if (y_tc || g_tc || fuse_b) AGCN_CUDA(cudaStreamWaitEvent(st, plan->ev_side_join, 0));
   // x = reshape(transpose(stack T)) . weight + bias, activation   graphconv.py:238-247, :118-123
-  if ((rc = node_gemm(gy, wk.tcY, st, /*presplit=*/true))) return rc;
+  if ((rc = gemm_auto(gy, wk.tcY, st, /*presplit=*/true))) return rc;
   return AGCN_OK;
 }
 
@@ -505,7 +483,7 @@ int backward_impl(const agcn_sgcll_desc* desc, const agcn_plan* plan, const floa
     GemmArgs g = g_gemm_args(desc, R, dYp, d_weight, (K == 1) ? d_dX : wk.G);
     GemmArgs probe = g_gemm_args(desc, R, d_Y, d_weight, wk.G);
     const bool presplit = (desc->flags & AGCN_SAVE_FOR_BACKWARD) && tc_gemm_supported(probe);
-    if ((rc = node_gemm(g, sv.tcG, st, presplit))) return rc;
+    if ((rc = gemm_auto(g, sv.tcG, st, presplit))) return rc;
   }
   GraphArgs ga;
   ga.plan = plan; ga.F = F; ga.K = K;
@@ -528,7 +506,7 @@ int backward_impl(const agcn_sgcll_desc* desc, const agcn_plan* plan, const floa
     t.A1 = sv.T; t.lda1 = F; t.sliceA1 = (int64_t)R * F;
     t.D = dYp; t.ldd = Fo;
     t.out = d_dweight; t.partial = wk.tn_part;
-    if ((rc = node_gemm_tn(t, plan->side))) return rc;
+    if ((rc = gemm_tn_auto(t, plan->side))) return rc;
   }
   AGCN_CUDA(cudaEventRecord(plan->ev_side_join, plan->side));
   if (vfirst) {
@@ -587,13 +565,13 @@ int backward_impl(const agcn_sgcll_desc* desc, const agcn_plan* plan, const floa
     t.A0 = d_X; t.lda0 = F;
     t.D = wk.dXW; t.ldd = F;
     t.out = d_dM_L; t.partial = wk.tn_part;
-    if ((rc = node_gemm_tn(t, st))) return rc;
+    if ((rc = gemm_tn_auto(t, st))) return rc;
     GemmArgs g;  // dX += dXW M_L^T
     g.M = R; g.N = F; g.Kd = F;
     g.A0 = wk.dXW; g.lda0 = F;
     g.B = d_M_L; g.ldb = F; g.transB = 1;
     g.C = d_dX; g.ldc = F; g.accumulate = 1;
-    if ((rc = node_gemm(g, wk.tcM, st))) return rc;
+    if ((rc = gemm_auto(g, wk.tcM, st))) return rc;
   } else {
     // tf.py_func has no gradient: M_L receives none (graphconv.py:211, SURVEY Q1)
     if ((rc = zero_async(d_dM_L, (size_t)F * F, st))) return rc;
@@ -606,11 +584,12 @@ int backward_impl(const agcn_sgcll_desc* desc, const agcn_plan* plan, const floa
 extern "C" {
 
 /* Building block exported for tests and tuning: out[(f*S + s)*N + c] = sum_r A_s[r, f] * D[r, c].
- * use_tensor_cores = 0 forces the CUDA-core kernel.  scratch: agcn_gemm_tn_scratch_bytes() bytes. */
+ * use_tensor_cores < 0 takes the library's engine, 1 forces tcgen05, 0 the CUDA cores.  scratch:
+ * agcn_gemm_tn_scratch_bytes() bytes. */
 size_t agcn_gemm_tn_scratch_bytes(int32_t M, int32_t Kd, int32_t N, int32_t S) {
   GemmTNArgs t;
   t.M = M; t.Kd = Kd; t.N = N; t.S = S;
-  return 4 * std::max(gemm_tn_partial_floats(M, Kd, N, S), tc_gemm_tn_partial_floats(t)) + 256;
+  return 4 * gemm_tn_auto_partial_floats(t) + 256;
 }
 
 int agcn_gemm_tn(const float* d_A0, const float* d_A1, const float* d_D, float* d_out, int32_t M, int32_t Kd,
@@ -622,14 +601,9 @@ int agcn_gemm_tn(const float* d_A0, const float* d_A1, const float* d_D, float* 
   t.A1 = d_A1; t.lda1 = Kd; t.sliceA1 = (int64_t)M * Kd;
   t.D = d_D; t.ldd = N;
   t.out = d_out; t.partial = reinterpret_cast<float*>(d_scratch);
-  if (use_tensor_cores) {
-    if (!tc_gemm_tn_supported(t)) {
-      set_error("gemm_tn: shape not supported by the tensor-core kernel");
-      return AGCN_ERR_INVALID;
-    }
-    return tc_gemm_tn(t, (cudaStream_t)stream);
-  }
-  return gemm_tn(t, (cudaStream_t)stream);
+  const cudaStream_t st = (cudaStream_t)stream;
+  if (use_tensor_cores < 0) return gemm_tn_auto(t, st);
+  return use_tensor_cores ? tc_gemm_tn(t, st) : gemm_tn(t, st);
 }
 
 /* Node-level linear map over the packed rows, the building block of the layers around SGC-LL that are plain
@@ -649,7 +623,7 @@ int agcn_node_gemm(const float* d_A, int32_t lda, const float* d_B, int32_t ldb,
   g.B = d_B; g.ldb = ldb; g.transB = transB;
   g.C = d_C; g.ldc = ldc;
   g.bias = d_bias; g.scale = d_scale; g.accumulate = accumulate; g.act = activation;
-  return node_gemm(g, reinterpret_cast<float*>(d_scratch), (cudaStream_t)stream);
+  return gemm_auto(g, reinterpret_cast<float*>(d_scratch), (cudaStream_t)stream);
 }
 
 int agcn_sgcll_host_scratch_bytes(const agcn_sgcll_desc* desc, const agcn_plan* plan, size_t* bytes) {

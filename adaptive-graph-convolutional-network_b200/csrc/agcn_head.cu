@@ -186,16 +186,34 @@ __global__ void sum_parts_kernel(const float* __restrict__ parts, int n, float* 
 
 namespace {
 
-// contraction over the rows: tensor cores when the shape allows it (>= 32 rows, TMA-compatible), CUDA cores otherwise
-int tn_any(const GemmTNArgs& t, cudaStream_t st) {
-  if (tc_gemm_tn_supported(t)) return tc_gemm_tn(t, st);
-  return gemm_tn(t, st);
-}
-size_t tn_any_partial(const GemmTNArgs& t) {
-  return std::max(tc_gemm_tn_partial_floats(t), gemm_tn_partial_floats(t.M, t.Kd, t.N, t.S));
+inline int pad4(int x) { return (x + 3) & ~3; }
+
+// dhead_W [Kd, N] = A^T D over `rows` rows, A [rows, Kd] and D with row pitch pad4(N): the tensor-core TN kernel takes
+// Kd <= 128 and N % 4 == 0, so the contraction runs 128 result rows at a time into Wpad [Kd, pad4(N)], whose N real
+// columns are then copied to dW.  tn_part holds head_weight_grad_partial_floats(rows, Kd, N) floats.
+size_t head_weight_grad_partial_floats(int rows, int Kd, int N) {
+  GemmTNArgs t;
+  t.M = rows; t.Kd = std::min(Kd, 128); t.N = pad4(N); t.S = 1;
+  return gemm_tn_auto_partial_floats(t);
 }
 
-inline int pad4(int x) { return (x + 3) & ~3; }
+int head_weight_grad(const float* A, int rows, int Kd, const float* D, int N, float* Wpad, float* tn_part, float* dW,
+                     cudaStream_t st) {
+  const int Np = pad4(N);
+  for (int f0 = 0; f0 < Kd; f0 += 128) {
+    GemmTNArgs t;
+    t.M = rows; t.Kd = std::min(128, Kd - f0); t.N = Np; t.S = 1;
+    t.A0 = A + f0; t.lda0 = Kd;
+    t.D = D; t.ldd = Np;
+    t.out = Wpad + (size_t)f0 * Np; t.partial = tn_part;
+    int rc = gemm_tn_auto(t, st);
+    if (rc) return rc;
+  }
+  const int64_t total = (int64_t)Kd * N;
+  copy_pitched_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(Wpad, Np, dW, N, Kd, N);
+  AGCN_LAUNCH_CHECK();
+  return AGCN_OK;
+}
 
 // The forward areas come first: they are agcn_head_predict's whole work area, and training adds its backward areas
 // behind them.
@@ -224,12 +242,9 @@ HeadWork carve_head(const agcn_plan* plan, int Fh, int Fm, int Nt, bool train, v
     w.dWh_pad = c.take((size_t)Fm * Ntp);
     w.tcC = c.take(tc_gemm_scratch_floats(Fm, Nt, 1, 1));   // head_W^T operand   (dmol  = dlog head_W^T)
     w.tcD = c.take(tc_gemm_scratch_floats(Fh, Fm, 1, 1));   // dense_W^T operand  (dhsum = dpre dense_W^T)
-    GemmTNArgs t;
-    t.M = (int)B; t.Kd = std::min(Fm, 128); t.N = Ntp; t.S = 1;
-    size_t tn = tn_any_partial(t);
-    t.Kd = Fh; t.N = Fm;
-    tn = std::max(tn, tn_any_partial(t));
-    w.tn_part = c.take(tn);
+    GemmTNArgs t;  // ddense_W
+    t.M = (int)B; t.Kd = Fh; t.N = Fm; t.S = 1;
+    w.tn_part = c.take(std::max(head_weight_grad_partial_floats((int)B, Fm, Nt), gemm_tn_auto_partial_floats(t)));
     w.splitk = c.take((size_t)8 * B * std::max(Fm, Fh));  // split-K partial sums of the two long contractions
   }
   w.bytes = c.bytes;
@@ -353,29 +368,16 @@ int head_run(const char* who, const agcn_plan* plan, const float* d_H, const flo
   AGCN_CUDA(cudaStreamWaitEvent(side, plan->ev_side_fork, 0));
   weighted_colsum_kernel<<<(Nt + 31) / 32, 256, 0, side>>>(w.dlog, Ntp, B, Nt, nullptr, gr->dhead_b);
   AGCN_LAUNCH_CHECK();
-  for (int f0 = 0; f0 < Fm; f0 += 128) {  // dhead_W = mol^T dlog, 128 rows of the result per contraction
-    GemmTNArgs t;
-    t.M = B; t.Kd = std::min(128, Fm - f0); t.N = Ntp; t.S = 1;
-    t.A0 = w.mol + f0; t.lda0 = Fm;
-    t.D = w.dlog; t.ldd = Ntp;
-    t.out = w.dWh_pad + (size_t)f0 * Ntp; t.partial = w.tn_part;
-    if ((rc = tn_any(t, side))) return rc;
-  }
-  {
-    const int64_t total = (int64_t)Fm * Nt;
-    copy_pitched_kernel<<<(unsigned)((total + 255) / 256), 256, 0, side>>>(w.dWh_pad, Ntp, gr->dhead_W, Nt, Fm, Nt);
-    AGCN_LAUNCH_CHECK();
-  }
+  if ((rc = head_weight_grad(w.mol, B, Fm, w.dlog, Nt, w.dWh_pad, w.tn_part, gr->dhead_W, side))) return rc;
 
   // main stream: dmol = dlog head_W^T, through tanh, ddense_b, dhsum, dH
-  auto gemm_any = [&](const GemmArgs& g, const float* scratch, bool tc) { return tc ? tc_gemm(g, scratch, st) : gemm_rows(g, st); };
-  if ((rc = gemm_any(g_dmol, w.tcC, tc_dmol))) return rc;
+  if ((rc = gemm_auto(g_dmol, w.tcC, st, /*presplit=*/true))) return rc;
   {
     const int64_t total = (int64_t)B * Fm;
     tanh_bwd_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(w.pre, w.dmol, total);  // dmol := dpre
     AGCN_LAUNCH_CHECK();
   }
-  if ((rc = gemm_any(g_dhs, w.tcD, tc_dhs))) return rc;
+  if ((rc = tc_dhs ? tc_gemm(g_dhs, w.tcD, st) : gemm_rows(g_dhs, st))) return rc;
   segment_broadcast_kernel<<<(B + 7) / 8, 256, 0, st>>>(w.dhsum, plan->d_node_off, B, Fh, gr->dH);
   AGCN_LAUNCH_CHECK();
   // dense parameter gradients (need dpre; the dhead_W contraction on the side stream is done with tn_part by now
@@ -390,7 +392,7 @@ int head_run(const char* who, const agcn_plan* plan, const float* d_H, const flo
     t.A0 = w.hsum; t.lda0 = Fh;
     t.D = w.dmol; t.ldd = Fm;
     t.out = gr->ddense_W; t.partial = w.tn_part;
-    if ((rc = tn_any(t, side))) return rc;
+    if ((rc = gemm_tn_auto(t, side))) return rc;
   }
   AGCN_CUDA(cudaEventRecord(plan->ev_side_join, side));
   AGCN_CUDA(cudaStreamWaitEvent(st, plan->ev_side_join, 0));
@@ -445,9 +447,7 @@ NodeHeadWork carve_node_head(const agcn_plan* plan, int Fh, int C, bool train, v
   if (train) {
     w.tcC = c.take(tc_gemm_scratch_floats(Fh, C, 1, 1));  // head_W^T    (dH = dlog head_W^T)
     w.dWh_pad = c.take((size_t)Fh * Cp);
-    GemmTNArgs t;
-    t.M = (int)R; t.Kd = std::min(Fh, 128); t.N = Cp; t.S = 1;
-    w.tn_part = c.take(tn_any_partial(t));
+    w.tn_part = c.take(head_weight_grad_partial_floats((int)R, Fh, C));
     w.colsum_part = c.take((size_t)colsum_parts(plan) * C);
   }
   w.bytes = c.bytes;
@@ -499,7 +499,7 @@ int node_head_run(const char* who, const agcn_plan* plan, const float* d_H, cons
   // logits (only the C real columns of dlog are written and read back: the pad columns feed nothing but the pad
   // columns of dWh_pad, which are not copied out), then the row softmax: d loss / d logits in place (training) or the
   // probabilities, and the per-row loss terms
-  if ((rc = tc_log ? tc_gemm(g_log, w.tcB, st) : gemm_rows(g_log, st))) return rc;
+  if ((rc = gemm_auto(g_log, w.tcB, st, /*presplit=*/true))) return rc;
   (train ? softmax_ce_kernel<true> : softmax_ce_kernel<false>)<<<(R + 7) / 8, 256, 0, st>>>(
       w.dlog, Cp, d_targets, d_weights, R, C, scale, d_probs, w.loss_part);
   AGCN_LAUNCH_CHECK();
@@ -515,22 +515,10 @@ int node_head_run(const char* who, const agcn_plan* plan, const float* d_H, cons
   colsum_part_kernel<<<colsum_parts(plan), 256, 0, side>>>(w.dlog, Cp, R, C, w.colsum_part);
   AGCN_LAUNCH_CHECK();
   if ((rc = colsum_reduce(w.colsum_part, colsum_parts(plan), C, d_dhead_b, side))) return rc;
-  for (int f0 = 0; f0 < Fh; f0 += 128) {  // dhead_W = H^T dlog, 128 rows of the result per contraction
-    GemmTNArgs t;
-    t.M = R; t.Kd = std::min(128, Fh - f0); t.N = Cp; t.S = 1;
-    t.A0 = d_H + f0; t.lda0 = Fh;
-    t.D = w.dlog; t.ldd = Cp;
-    t.out = w.dWh_pad + (size_t)f0 * Cp; t.partial = w.tn_part;
-    if ((rc = tn_any(t, side))) return rc;
-  }
-  {
-    const int64_t total = (int64_t)Fh * C;
-    copy_pitched_kernel<<<(unsigned)((total + 255) / 256), 256, 0, side>>>(w.dWh_pad, Cp, d_dhead_W, C, Fh, C);
-    AGCN_LAUNCH_CHECK();
-  }
+  if ((rc = head_weight_grad(d_H, R, Fh, w.dlog, C, w.dWh_pad, w.tn_part, d_dhead_W, side))) return rc;
   AGCN_CUDA(cudaEventRecord(plan->ev_side_join, side));
 
-  if ((rc = tc_dH ? tc_gemm(g_dH, w.tcC, st) : gemm_rows(g_dH, st))) return rc;
+  if ((rc = gemm_auto(g_dH, w.tcC, st, /*presplit=*/true))) return rc;
   AGCN_CUDA(cudaStreamWaitEvent(st, plan->ev_side_join, 0));
   return AGCN_OK;
 }

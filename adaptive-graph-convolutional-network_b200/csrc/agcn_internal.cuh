@@ -230,7 +230,14 @@ int gemm_tn(const GemmTNArgs& a, cudaStream_t st);
 // tcgen05 (3xTF32, MN-major operands) implementation of the same contraction (agcn_tc_gemm.cu)
 bool tc_gemm_tn_supported(const GemmTNArgs& a);
 size_t tc_gemm_tn_partial_floats(const GemmTNArgs& a);
-int tc_gemm_tn(const GemmTNArgs& a, cudaStream_t st);
+int tc_gemm_tn(const GemmTNArgs& a, cudaStream_t st);  // AGCN_ERR_INVALID for a shape tc_gemm_tn_supported rejects
+
+// The library's engine choice for the products above (agcn_node_gemm.cu): tcgen05 when tc_gemm_supported /
+// tc_gemm_tn_supported accept the operands, the CUDA cores otherwise.  gemm_auto splits B into tc_scratch
+// (tc_gemm_scratch_floats floats) first unless presplit says a tc_gemm_split_b of the same operand already ran.
+int gemm_auto(const GemmArgs& a, float* tc_scratch, cudaStream_t st, bool presplit = false);
+int gemm_tn_auto(const GemmTNArgs& a, cudaStream_t st);
+size_t gemm_tn_auto_partial_floats(const GemmTNArgs& a);  // scratch of a.partial for either engine
 
 // dYp = dY * act'(Y) (relu mask), colsum(dYp) -> dbias.  partial: act_bwd_partial_floats() floats.
 size_t act_bwd_partial_floats(int64_t R, int Fo);

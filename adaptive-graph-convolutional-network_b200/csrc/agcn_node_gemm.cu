@@ -7,6 +7,10 @@
 //   gemm_tn    : dW_k = T_k^T dY, dM_L = X^T dXW  contraction over the node dimension, deterministic
 //                two-stage reduction (no atomics)
 //   act_bwd_colsum : dYpre = dY * relu'(Y) and dbias = colsum(dYpre)
+//
+// gemm_auto / gemm_tn_auto pick between these kernels and their tcgen05 versions (agcn_tc_gemm.cu) for every caller.
+#include <algorithm>
+
 #include "agcn_internal.cuh"
 
 namespace agcn {
@@ -251,6 +255,25 @@ int gemm_tn(const GemmTNArgs& a, cudaStream_t st) {
   reduce_partials_kernel<<<(unsigned)((elems + 255) / 256), 256, 0, st>>>(a.partial, a.out, elems, splits);
   AGCN_LAUNCH_CHECK();
   return AGCN_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Engine of every node-level product: tensor cores when the operands are TMA-compatible, CUDA cores otherwise (F = 75)
+int gemm_auto(const GemmArgs& a, float* tc_scratch, cudaStream_t st, bool presplit) {
+  if (!tc_gemm_supported(a)) return gemm_rows(a, st);
+  if (!presplit) {
+    int rc = tc_gemm_split_b(a, tc_scratch, st);
+    if (rc) return rc;
+  }
+  return tc_gemm(a, tc_scratch, st);
+}
+
+int gemm_tn_auto(const GemmTNArgs& a, cudaStream_t st) {
+  return tc_gemm_tn_supported(a) ? tc_gemm_tn(a, st) : gemm_tn(a, st);
+}
+
+size_t gemm_tn_auto_partial_floats(const GemmTNArgs& a) {
+  return std::max(tc_gemm_tn_partial_floats(a), gemm_tn_partial_floats(a.M, a.Kd, a.N, a.S));
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -11,7 +11,7 @@
 //
 // A stack is a list of nodes (agcn_stack_create_nodes): SGC_LL layers, SGC_LL_Reslap layers whose L_prev is an earlier
 // Reslap layer's L_all (ResidualGraphMolResLap, tf_graphs.py:159-223), and BlockEnd nodes that close a residual block
-// (blockend.py:67-86, through agcn_node_gemm / agcn_gemm_tn as functional._NodeLinear calls them).
+// (blockend.py:67-86, through agcn_node_gemm and the TN contraction on the engines functional._NodeLinear gets).
 // agcn_stack_create is the list of SGC_LL layers.
 #include <algorithm>
 #include <cmath>
@@ -414,10 +414,12 @@ int agcn_stack_loss_grad(const agcn_stack* s, const agcn_plan* plan, const float
       act_grad_kernel<<<(unsigned)std::min<long long>((n + 255) / 256, 148 * 8), 256, 0, st>>>(
           dcur, w.H[l], w.dpre[l], n, d.activation == AGCN_ACT_RELU);
       AGCN_LAUNCH_CHECK();
-      // dW = H[src]^T dpre, on the kernel functional._NodeLinear picks for this shape
-      const int use_tc = (d.F <= 128 && d.F % 4 == 0 && d.Fo % 4 == 0 && R >= 32) ? 1 : 0;
-      rc = agcn_gemm_tn(w.H[nd.src], nullptr, w.dpre[l], G(l, 0), R, d.F, d.Fo, 1, w.layer_work, use_tc, stream);
-      if (rc) return rc;
+      GemmTNArgs t;  // dW = H[src]^T dpre, on the engine functional._NodeLinear gets from agcn_gemm_tn
+      t.M = R; t.Kd = d.F; t.N = d.Fo; t.S = 1;
+      t.A0 = w.H[nd.src]; t.lda0 = d.F;
+      t.D = w.dpre[l]; t.ldd = d.Fo;
+      t.out = G(l, 0); t.partial = static_cast<float*>(w.layer_work);
+      if ((rc = gemm_tn_auto(t, st))) return rc;
       dprev = w.dpre[l];
       if (s->res_user[l - 1] >= 0) {   // more is added to dH[l-1]: keep dpre itself for this BlockEnd's dX product
         AGCN_CUDA(cudaMemcpyAsync(dnext, dprev, (size_t)R * d.Fo * sizeof(float), cudaMemcpyDeviceToDevice, st));

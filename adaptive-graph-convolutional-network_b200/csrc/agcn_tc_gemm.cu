@@ -830,6 +830,10 @@ __global__ void reduce_chunks_kernel(const float* __restrict__ partial, float* _
 
 int tc_gemm_tn(const GemmTNArgs& a, cudaStream_t st) {
   using namespace tc;
+  if (!tc_gemm_tn_supported(a)) {
+    set_error("gemm_tn: shape not supported by the tensor-core kernel");
+    return AGCN_ERR_INVALID;
+  }
   int chunks, per;
   tn_chunks(a, &chunks, &per);
   CUtensorMap mA0, mA1, mD;

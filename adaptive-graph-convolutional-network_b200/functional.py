@@ -365,11 +365,11 @@ class _NodeLinear(torch.autograd.Function):
                 dWu = torch.empty_like(W)         # A^T dpre (contraction over the rows)
                 tn = torch.empty(lib.agcn_gemm_tn_scratch_bytes(M, Kd, N, 1), dtype=torch.uint8, device=dev)
                 # d beta = <dpre, A W> = <A^T dpre, W> is a sum with heavy cancellation: when it is wanted, the
-                # contraction runs in plain fp32 FMAs (tensor-core accumulation truncates) and the dot in double
+                # contraction runs in plain fp32 FMAs (tensor-core accumulation truncates) and the dot in double;
+                # otherwise on the library's engine (-1), the one agcn_stack_loss_grad uses for BlockEnd
                 want_dscale = has_scale and ctx.needs_input_grad[3]
-                use_tc = 1 if (Kd <= 128 and Kd % 4 == 0 and N % 4 == 0 and M >= 32 and not want_dscale) else 0
-                _lib.check(lib.agcn_gemm_tn(_ptr(A), None, _ptr(dpre), _ptr(dWu), M, Kd, N, 1, _ptr(tn), use_tc,
-                                            _stream_ptr(dev)))
+                _lib.check(lib.agcn_gemm_tn(_ptr(A), None, _ptr(dpre), _ptr(dWu), M, Kd, N, 1, _ptr(tn),
+                                            0 if want_dscale else -1, _stream_ptr(dev)))
                 if want_dscale:
                     dscale = (dWu.double() * W.double()).sum().float().reshape(scale.shape)
                 dW = dWu * scale if has_scale else dWu

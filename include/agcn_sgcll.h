@@ -202,7 +202,9 @@ int agcn_sgcll_backward(const agcn_sgcll_desc* desc, const agcn_plan* plan, cons
 /* Building block of the backward pass, exported for unit tests and tuning (no reference counterpart: it is
  * the dW = T^T dY contraction that tf.gradients derives from graphconv.py:245-247):
  *   out[(f*S + s)*N + c] = sum_r A_s[r, f] * D[r, c],  A_0 = d_A0 [M,Kd], A_s = d_A1 + (s-1)*M*Kd, D [M,N].
- * use_tensor_cores: 1 = tcgen05 3xTF32 kernel (needs Kd <= 128, Kd % 4 == 0, N % 4 == 0), 0 = CUDA cores. */
+ * use_tensor_cores: < 0 = the library's choice, the one the layer, head and stack calls make for their contractions
+ * over the rows (tcgen05 when the shape allows it, CUDA cores otherwise); 1 = tcgen05 3xTF32 kernel (needs M >= 32,
+ * Kd <= 128, Kd % 4 == 0, N % 4 == 0, 16-byte aligned operands, else AGCN_ERR_INVALID); 0 = CUDA cores. */
 size_t agcn_gemm_tn_scratch_bytes(int32_t M, int32_t Kd, int32_t N, int32_t S);
 int agcn_gemm_tn(const float* d_A0, const float* d_A1, const float* d_D, float* d_out, int32_t M, int32_t Kd,
                  int32_t N, int32_t S, void* d_scratch, int32_t use_tensor_cores, void* stream);

@@ -6,7 +6,8 @@ agcn_node_gemm  C (+)= act(scale * A op(B) + bias) over M packed rows:
                                             A / B are 16-byte aligned;
                   gemm_rows, scalar loads   everything else (here: A offset by one float).
 agcn_gemm_tn    out[(f*S + s)*N + c] = sum_r A_s[r, f] D[r, c], tcgen05 (use_tensor_cores = 1) or CUDA cores (0), both
-                a chunked contraction over the rows followed by a fixed-order reduction of the chunks.
+                a chunked contraction over the rows followed by a fixed-order reduction of the chunks; -1 takes the
+                library's choice (tcgen05 for M >= 32, Kd <= 128, Kd and N multiples of 4, aligned operands).
 
 Shapes are the ones where tiles go wrong: M = 1 and M just off a 128-row tile, N above 128 and not a multiple of 128,
 Kd not a multiple of 4 on the tensor cores, row pitches larger than the width (lda > Kd, ldc > N), transB, S > 1 and
@@ -162,7 +163,7 @@ def _tn_case(M, Kd, N, S, use_tc, gen):
         outs.append(out)
     ref = torch.einsum("srf,rc->fsc", A.double().view(S, M, Kd), D.double()).reshape(-1)
     err = float((outs[0].double() - ref).abs().max() / ref.abs().max().clamp_min(1e-30))
-    return err, torch.equal(outs[0], outs[1])
+    return err, torch.equal(outs[0], outs[1]), outs[0]
 
 
 @pytest.mark.parametrize("use_tc", (1, 0), ids=("tcgen05", "cuda_cores"))
@@ -175,7 +176,7 @@ def test_gemm_tn_matches_fp64_and_is_deterministic(use_tc):
         for Kd in grid["Kd"]:
             for N in grid["N"]:
                 for S in (1, 3):
-                    err, same = _tn_case(M, Kd, N, S, use_tc, gen)
+                    err, same, _ = _tn_case(M, Kd, N, S, use_tc, gen)
                     worst = max(worst, err)
                     if not (err <= BUDGET and same):
                         bad.append((M, Kd, N, S, "%.2e" % err, "deterministic" if same else "NOT DETERMINISTIC"))
@@ -217,6 +218,14 @@ ENGINE_CASES = [
     (128, 64, 30, 1, False, 0),     # gemm_rows scalar loads: Kd % 4 != 0 below 32
 ]
 
+TN_ENGINE_CASES = [
+    # M, Kd, N, S, engine of use_tensor_cores = -1 (the library's choice)
+    (100, 36, 68, 3, "tcgen05"),
+    (100, 132, 68, 1, "cuda cores"),   # Kd > 128
+    (100, 36, 66, 1, "cuda cores"),    # N % 4 != 0
+    (31, 36, 68, 1, "cuda cores"),     # M < 32
+]
+
 
 def test_engines_are_the_ones_the_grid_is_labelled_with():
     lib = _lib().lib()
@@ -226,6 +235,16 @@ def test_engines_are_the_ones_the_grid_is_labelled_with():
         label = []
         names = _kernels(lambda: label.append(_node_case(M, N, Kd, transB, "plain", pitched, off, gen, scratch)[2]))
         assert _engine_of(names) == {label[0]}, (M, N, Kd, transB, pitched, off, label[0], names)
-    for use_tc, want in ((1, "tcgen05"), (0, "cuda cores")):
-        names = _kernels(lambda: _tn_case(100, 36, 68, 3, use_tc, gen))
-        assert _engine_of(names) == {want}, (use_tc, names)
+    # agcn_gemm_tn on each engine it takes; the library's choice must give the bits of the engine it names
+    for M, Kd, N, S, auto in TN_ENGINE_CASES:
+        outs = {}
+        for use_tc, want in ((1, "tcgen05"), (0, "cuda cores"), (-1, auto)):
+            run = lambda: outs.setdefault(use_tc, _tn_case(M, Kd, N, S, use_tc, torch.Generator().manual_seed(M + Kd))[2])
+            if use_tc == 1 and auto != "tcgen05":
+                with pytest.raises(_lib().AgcnError, match="not supported by the tensor-core kernel"):
+                    run()
+                continue
+            names = _kernels(run)
+            assert _engine_of(names) == {want}, (M, Kd, N, S, use_tc, names)
+        same = outs[1 if auto == "tcgen05" else 0]
+        assert torch.equal(outs[-1].view(torch.int32), same.view(torch.int32)), (M, Kd, N, S)
