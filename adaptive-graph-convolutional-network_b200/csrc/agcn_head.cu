@@ -22,33 +22,144 @@
 
 namespace agcn {
 
-// hsum[g, :] = sum of the rows of graph g          (one warp per graph; every row load of the warp is in flight at
-// once: lanes walk the graph's rows as one contiguous [n_g * F] range, fixed summation order per column)
-__global__ void segment_sum_kernel(const float* __restrict__ H, const int32_t* __restrict__ node_off, int B, int F,
-                                   float* __restrict__ hsum) {
-  const int g = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-  if (g >= B) return;
-  const int r0 = node_off[g], r1 = node_off[g + 1];
-  if (F % 32 == 0) {
-    // lane owns columns lane, lane + 32, ...: consecutive lanes read consecutive addresses of every row
-    for (int c = lane; c < F; c += 32) {
-      float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
-      int r = r0;
-      for (; r + 4 <= r1; r += 4) {
-        s0 += __ldg(H + (int64_t)r * F + c);
-        s1 += __ldg(H + (int64_t)(r + 1) * F + c);
-        s2 += __ldg(H + (int64_t)(r + 2) * F + c);
-        s3 += __ldg(H + (int64_t)(r + 3) * F + c);
-      }
-      for (; r < r1; ++r) s0 += __ldg(H + (int64_t)r * F + c);
-      hsum[(int64_t)g * F + c] = (s0 + s1) + (s2 + s3);
-    }
-    return;
-  }
-  for (int c = lane; c < F; c += 32) {
+constexpr int HEAD_GRAPHS = 4;  // graphs per CTA of head_fwd_kernel / head_bwd_kernel (B = 1024: 256 CTAs)
+
+// GraphGatherMol + DenseMol (commuted) + tanh for HEAD_GRAPHS graphs x 256 columns of Fm:
+//   hsum[g, :] = sum of the rows of graph g,  a = hsum[g, :] dense_W + n_g dense_b,  mol = tanh(a),
+//   dtanh = tanh'(a) = sech^2(a) evaluated as 4 e / (1 + e)^2, e = exp(-2 |a|): the sum over a molecule's atoms
+//   saturates the tanh, and 1 - mol^2 would then cancel to a handful of significant bits (errors of 1e-4 .. 1e-3
+//   relative in every gradient behind it).
+// The row sums run 64 columns of Fh at a time, one thread per (graph, column); for Fh % 32 == 0 each thread keeps four
+// partial sums over rows r0 + 4i + j (eight rows in flight), the rest go to the first, and the result is
+// (s0 + s1) + (s2 + s3).  The product runs one thread per column in fp32, four k at a time with the expression of
+// gemm_rows_kernel (groups aligned to k = 0, zero past Fh), so `pre` is what gemm_rows computes.  Every CTA sums its
+// graphs' rows; those of blockIdx.y == 0 write hsum (ddense_W = hsum^T dpre reads it).
+__global__ void __launch_bounds__(256) head_fwd_kernel(const float* __restrict__ H, const int32_t* __restrict__ node_off,
+                                                       const int32_t* __restrict__ n_nodes,
+                                                       const float* __restrict__ W, const float* __restrict__ b, int B,
+                                                       int Fh, int Fm, float* __restrict__ hsum,
+                                                       float* __restrict__ dtanh, float* __restrict__ mol) {
+  __shared__ float hs[HEAD_GRAPHS][64];
+  const int t = threadIdx.x, g0 = blockIdx.x * HEAD_GRAPHS, c = blockIdx.y * 256 + t;
+  const int sg = t >> 6, sc = t & 63, g = g0 + sg;
+  const int r0 = g < B ? node_off[g] : 0, r1 = g < B ? node_off[g + 1] : 0;
+  float acc[HEAD_GRAPHS];
+#pragma unroll
+  for (int i = 0; i < HEAD_GRAPHS; ++i) acc[i] = 0.f;
+  for (int k0 = 0; k0 < Fh; k0 += 64) {
+    const int col = k0 + sc;
     float s = 0.f;
-    for (int r = r0; r < r1; ++r) s += H[(int64_t)r * F + c];
-    hsum[(int64_t)g * F + c] = s;
+    if (col < Fh) {
+      const float* __restrict__ h = H + col;
+      if (Fh % 32 == 0) {
+        float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
+        int r = r0;
+        for (; r + 8 <= r1; r += 8) {
+          float v[8];
+#pragma unroll
+          for (int j = 0; j < 8; ++j) v[j] = __ldg(h + (int64_t)(r + j) * Fh);
+          s0 += v[0]; s1 += v[1]; s2 += v[2]; s3 += v[3];
+          s0 += v[4]; s1 += v[5]; s2 += v[6]; s3 += v[7];
+        }
+        if (r + 4 <= r1) {
+          s0 += __ldg(h + (int64_t)r * Fh);
+          s1 += __ldg(h + (int64_t)(r + 1) * Fh);
+          s2 += __ldg(h + (int64_t)(r + 2) * Fh);
+          s3 += __ldg(h + (int64_t)(r + 3) * Fh);
+          r += 4;
+        }
+        for (; r < r1; ++r) s0 += __ldg(h + (int64_t)r * Fh);
+        s = (s0 + s1) + (s2 + s3);
+      } else {
+        for (int r = r0; r < r1; ++r) s += __ldg(h + (int64_t)r * Fh);
+      }
+      if (g < B && blockIdx.y == 0) hsum[(int64_t)g * Fh + col] = s;
+    }
+    hs[sg][sc] = s;
+    __syncthreads();
+    if (c < Fm) {
+      const int kn = min(64, Fh - k0);   // hs[.][k] == 0 for k >= kn
+      const float* __restrict__ w = W + (int64_t)k0 * Fm + c;
+      for (int k = 0; k < kn; k += 4) {
+        const float b0 = __ldg(w + (int64_t)k * Fm);
+        const float b1 = k + 1 < kn ? __ldg(w + (int64_t)(k + 1) * Fm) : 0.f;
+        const float b2 = k + 2 < kn ? __ldg(w + (int64_t)(k + 2) * Fm) : 0.f;
+        const float b3 = k + 3 < kn ? __ldg(w + (int64_t)(k + 3) * Fm) : 0.f;
+#pragma unroll
+        for (int i = 0; i < HEAD_GRAPHS; ++i)
+          acc[i] += hs[i][k] * b0 + hs[i][k + 1] * b1 + hs[i][k + 2] * b2 + hs[i][k + 3] * b3;
+      }
+    }
+    __syncthreads();
+  }
+  if (c >= Fm) return;
+  const float bc = b[c];
+#pragma unroll
+  for (int i = 0; i < HEAD_GRAPHS; ++i) {
+    if (g0 + i >= B) break;
+    const int64_t e = (int64_t)(g0 + i) * Fm + c;
+    const float a = acc[i] + (float)n_nodes[g0 + i] * bc;
+    mol[e] = tanhf(a);
+    const float ex = expf(-2.f * fabsf(a));
+    dtanh[e] = 4.f * ex / ((1.f + ex) * (1.f + ex));
+  }
+}
+
+// The way back from d loss / d mol to dH for HEAD_GRAPHS graphs per CTA (dynamic shared memory: HEAD_GRAPHS x (Fm + Fh)
+// floats).  dmol arrives as `chunks` split-K partial sums chunk_stride floats apart (chunks == 1: dmol itself), added in
+// the order of reduce_chunks_kernel; then
+//   dpre = dmol tanh'(a)                       (written: ddense_W and ddense_b read it; dpre may alias dmol)
+//   dhsum[g, j] = sum_c dpre[g, c] dense_W[j, c]: one thread per (graph, j), fp32, four c at a time with the expression
+//                 of gemm_rows_kernel, so dhsum is what gemm_rows computes; dense_W passes through shared memory in
+//                 64 x 32 tiles read along its rows
+//   dH[r, :] = dhsum[g, :] for every row r of graph g
+// dH == NULL: dpre only (the large shapes of head_run take dhsum from the tensor cores).
+__global__ void __launch_bounds__(256) head_bwd_kernel(const float* dmol, int64_t chunk_stride, int chunks,
+                                                       const float* __restrict__ dtanh, const float* __restrict__ W,
+                                                       const int32_t* __restrict__ node_off, int B, int Fh, int Fm,
+                                                       float* dpre, float* __restrict__ dH) {
+  extern __shared__ float sp[];  // [HEAD_GRAPHS][Fm] dpre, then [HEAD_GRAPHS][Fh] dhsum
+  __shared__ float ws[64][33];   // dense_W[j0 + jj, c0 + cc]
+  float* dh = sp + HEAD_GRAPHS * Fm;
+  const int t = threadIdx.x, g0 = blockIdx.x * HEAD_GRAPHS, ng = min(HEAD_GRAPHS, B - g0);
+  for (int c = t; c < Fm; c += 256) {
+#pragma unroll
+    for (int i = 0; i < HEAD_GRAPHS; ++i) {
+      float v = 0.f;
+      if (i < ng) {
+        const int64_t e = (int64_t)(g0 + i) * Fm + c;
+        float s = 0.f;
+        for (int k = 0; k < chunks; ++k) s += dmol[k * chunk_stride + e];
+        v = s * dtanh[e];
+        dpre[e] = v;
+      }
+      sp[i * Fm + c] = v;
+    }
+  }
+  if (!dH) return;
+  const int i = t >> 6, jj = t & 63;   // 256 threads = HEAD_GRAPHS x 64
+  const float* p = sp + i * Fm;
+  for (int j0 = 0; j0 < Fh; j0 += 64) {
+    float acc = 0.f;
+    for (int c0 = 0; c0 < Fm; c0 += 32) {
+      __syncthreads();
+      for (int e = t; e < 64 * 32; e += 256) {
+        const int r = e >> 5, cc = e & 31;
+        ws[r][cc] = j0 + r < Fh && c0 + cc < Fm ? __ldg(W + (int64_t)(j0 + r) * Fm + c0 + cc) : 0.f;
+      }
+      __syncthreads();
+      const int cn = min(32, Fm - c0);   // a multiple of 4
+      for (int cc = 0; cc < cn; cc += 4)
+        acc += p[c0 + cc] * ws[jj][cc] + p[c0 + cc + 1] * ws[jj][cc + 1] + p[c0 + cc + 2] * ws[jj][cc + 2] +
+               p[c0 + cc + 3] * ws[jj][cc + 3];
+    }
+    if (j0 + jj < Fh) dh[i * Fh + j0 + jj] = acc;
+  }
+  __syncthreads();
+  for (int g = 0; g < ng; ++g) {
+    const int r0 = node_off[g0 + g], rows = node_off[g0 + g + 1] - r0;
+    float* __restrict__ out = dH + (int64_t)r0 * Fh;
+    for (int e = t; e < rows * Fh; e += 256) out[e] = dh[g * Fh + e % Fh];
   }
 }
 
@@ -65,27 +176,6 @@ __global__ void __launch_bounds__(1024) expand_labels_kernel(const uint8_t* __re
     targets[e] = make_float2(1.f - yv, yv);
     weights[e] = make_float2(wv, wv);
   }
-}
-
-// mol = tanh(a), a = pre + n_g b   (graphgather.py:77); `pre` is overwritten with tanh'(a) = sech^2(a) evaluated as
-// 4 e / (1 + e)^2, e = exp(-2 |a|): the sum over a molecule's atoms saturates the tanh, and 1 - mol^2 would then
-// cancel to a handful of significant bits (errors of 1e-4 .. 1e-3 relative in every gradient behind it)
-__global__ void gather_tanh_kernel(float* __restrict__ pre, const float* __restrict__ b,
-                                   const int32_t* __restrict__ n_nodes, int B, int Fm, float* __restrict__ mol) {
-  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (e >= (int64_t)B * Fm) return;
-  const int g = (int)(e / Fm), c = (int)(e % Fm);
-  const float a = pre[e] + (float)n_nodes[g] * b[c];
-  mol[e] = tanhf(a);
-  const float ex = expf(-2.f * fabsf(a));
-  pre[e] = 4.f * ex / ((1.f + ex) * (1.f + ex));
-}
-
-// dpre = dmol tanh'(a), in place over dmol
-__global__ void tanh_bwd_kernel(const float* __restrict__ dtanh, float* __restrict__ dmol, int64_t total) {
-  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (e >= total) return;
-  dmol[e] = dmol[e] * dtanh[e];
 }
 
 // out[c] = sum_r w_r M[r, c]  (w == NULL: plain column sums): 32 columns per CTA, rows over 8 warps, fixed order
@@ -256,15 +346,19 @@ struct HeadGrads {
   float *dH, *ddense_W, *ddense_b, *dhead_W, *dhead_b;
 };
 
-// Both head calls.  The forward runs the same products with the same tile configurations for training (grads set) and
-// prediction (grads NULL): `pre` on the CUDA cores, the logits on the tensor cores with the loss (or the probabilities)
-// in their epilogue, the single-task softmax in softmax_ce_kernel.  The evaluation loss is therefore bit-identical to
-// the training loss.  Prediction writes the probabilities (weighted L2: the values) to d_probs and the loss to d_loss
-// when targets are given; training writes the loss and every gradient.
+// Both head calls.  The forward runs the same kernels with the same tile configurations for training (grads set) and
+// prediction (grads NULL): gather, dense product and tanh in head_fwd_kernel, the logits on the tensor cores with the
+// loss (or the probabilities) in their epilogue, the single-task softmax in softmax_ce_kernel.  The evaluation loss is
+// therefore bit-identical to the training loss.  Prediction writes the probabilities (weighted L2: the values) to
+// d_probs and the loss to d_loss when targets are given; training writes the loss and every gradient.
+//
+// Training: the main stream runs dmol = dlog head_W^T and head_bwd_kernel, which ends at dH; the parameter gradients
+// run beside it on plan->head.  join_head: `st` waits for them before head_run returns.  Otherwise the caller must make
+// `st` wait for plan->ev_head_join before it reads the parameter gradients or ends a capture (agcn_stack_loss_grad).
 int head_run(const char* who, const agcn_plan* plan, const float* d_H, const float* d_dense_W, const float* d_dense_b,
              const float* d_head_W, const float* d_head_b, const float* d_targets, const float* d_weights, float scale,
              int32_t loss_kind, int32_t Fh, int32_t Fm, int32_t Nt, float* d_probs, float* d_loss, const HeadGrads* gr,
-             void* d_work, size_t work_bytes, cudaStream_t st) {
+             void* d_work, size_t work_bytes, bool join_head, cudaStream_t st) {
   const std::string at = std::string(who) + ": ";
   AGCN_REQUIRE(loss_kind != AGCN_PER_NODE_SOFTMAX_CE,
                at + "AGCN_PER_NODE_SOFTMAX_CE is the per-node head: call agcn_node_head_loss_grad / agcn_node_head_predict");
@@ -287,13 +381,9 @@ int head_run(const char* who, const agcn_plan* plan, const float* d_H, const flo
     return AGCN_ERR_WORKSPACE;
   }
   const int B = plan->B, Ntp = pad4(Nt);
-  cudaStream_t side = plan->side;
+  cudaStream_t side = plan->side, hs = plan->head;
 
-  GemmArgs g_pre, g_log;
-  g_pre.M = B; g_pre.N = Fm; g_pre.Kd = Fh;
-  g_pre.A0 = w.hsum; g_pre.lda0 = Fh;
-  g_pre.B = d_dense_W; g_pre.ldb = Fm;
-  g_pre.C = w.pre; g_pre.ldc = Fm;
+  GemmArgs g_log;
   g_log.M = B; g_log.N = Nt; g_log.Kd = Fm;
   g_log.A0 = w.mol; g_log.lda0 = Fm;
   g_log.B = d_head_W; g_log.ldb = Nt;
@@ -311,17 +401,19 @@ int head_run(const char* who, const agcn_plan* plan, const float* d_H, const flo
     }
   }
   AGCN_REQUIRE(tc_gemm_supported(g_log), at + "operands are not TMA-compatible (alignment)");
-  GemmArgs g_dmol, g_dhs;
+  GemmArgs g_dmol;  // split-K partials are left for head_bwd_kernel to add
   g_dmol.M = B; g_dmol.N = Fm; g_dmol.Kd = Nt;
   g_dmol.A0 = w.dlog; g_dmol.lda0 = Ntp;
   g_dmol.B = d_head_W; g_dmol.ldb = Nt; g_dmol.transB = 1;  // head_W is [Fm, Nt] = [N, Kd]
-  g_dmol.C = w.dmol; g_dmol.ldc = Fm; g_dmol.split_k_partial = w.splitk;
+  g_dmol.C = w.dmol; g_dmol.ldc = Fm; g_dmol.split_k_partial = w.splitk; g_dmol.split_k_raw = 1;
+  GemmArgs g_dhs;
   g_dhs.M = B; g_dhs.N = Fh; g_dhs.Kd = Fm;
   g_dhs.A0 = w.dmol; g_dhs.lda0 = Fm;
   g_dhs.B = d_dense_W; g_dhs.ldb = Fm; g_dhs.transB = 1;    // dense_W is [Fh, Fm] = [N, Kd]
   g_dhs.C = w.dhsum; g_dhs.ldc = Fh; g_dhs.split_k_partial = w.splitk;
-  // dhsum = dpre dense_W^T is [B, Fm] x [Fm, Fh] with Fh = 64: eight 128-row tiles of eight k-blocks each -- a latency chain
-  // of 30 us on 8 SMs on the tensor-core kernel, 12 us spread over every SM on the CUDA cores (33 MFLOP)
+  // dhsum = dpre dense_W^T runs inside head_bwd_kernel, on the CUDA cores, up to 2^26 multiply-adds: every CTA reads all
+  // of dense_W, which the large products pay for (B = 4096, Fh = 128, Fm = 512: 637 against 558 us per head call on
+  // the tensor cores); those keep the tcgen05 product and a broadcast into dH
   const bool tc_dmol = train && tc_gemm_supported(g_dmol),
              tc_dhs = train && tc_gemm_supported(g_dhs) && (int64_t)B * Fh * Fm > (1ll << 26);
 
@@ -336,16 +428,15 @@ int head_run(const char* who, const agcn_plan* plan, const float* d_H, const flo
 
   // GraphGatherMol + DenseMol (commuted) + tanh.  `pre` feeds a tanh that the sum over a molecule's atoms saturates:
   // tanh'(a) = sech^2(a) has relative sensitivity 2 |da|, so the absolute error of this [B, Fh] x [Fh, Fm] product (a
-  // few MFLOP) decides the accuracy of every gradient behind it.  Plain fp32 FMAs (gemm_rows) keep it at fp32 rounding
-  // level; 3xTF32 is ~4x coarser.
-  segment_sum_kernel<<<(B + 7) / 8, 256, 0, st>>>(d_H, plan->d_node_off, B, Fh, w.hsum);
-  AGCN_LAUNCH_CHECK();
-  if ((rc = gemm_rows(g_pre, st))) return rc;
+  // few MFLOP) decides the accuracy of every gradient behind it.  Plain fp32 FMAs keep it at fp32 rounding level;
+  // 3xTF32 is ~4x coarser.  w.pre receives tanh'(a).
   {
-    const int64_t total = (int64_t)B * Fm;
-    gather_tanh_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(w.pre, d_dense_b, plan->d_n, B, Fm, w.mol);
-    AGCN_LAUNCH_CHECK();
+    const dim3 grid((unsigned)((B + HEAD_GRAPHS - 1) / HEAD_GRAPHS), (unsigned)((Fm + 255) / 256));
+    ProfScope prof("head_fwd_kernel", st);
+    head_fwd_kernel<<<grid, 256, 0, st>>>(d_H, plan->d_node_off, plan->d_n, d_dense_W, d_dense_b, B, Fh, Fm, w.hsum,
+                                          w.pre, w.mol);
   }
+  AGCN_LAUNCH_CHECK();
   // logits + loss epilogue: C receives d loss / d logits (training), the probabilities (prediction) or, for the
   // single-task head, the logits; the loss its per-warp partial sums
   AGCN_CUDA(cudaStreamWaitEvent(st, plan->ev_side_join, 0));
@@ -363,28 +454,35 @@ int head_run(const char* who, const agcn_plan* plan, const float* d_H, const flo
   }
   if (!train) return AGCN_OK;
 
-  // parameter gradients of the heads on the side stream, beside the chain back to dH
-  AGCN_CUDA(cudaEventRecord(plan->ev_side_fork, st));
-  AGCN_CUDA(cudaStreamWaitEvent(side, plan->ev_side_fork, 0));
-  weighted_colsum_kernel<<<(Nt + 31) / 32, 256, 0, side>>>(w.dlog, Ntp, B, Nt, nullptr, gr->dhead_b);
+  // the head's parameter gradients on plan->head, beside the chain back to dH on the main stream
+  AGCN_CUDA(cudaEventRecord(plan->ev_head_fork, st));
+  AGCN_CUDA(cudaStreamWaitEvent(hs, plan->ev_head_fork, 0));
+  weighted_colsum_kernel<<<(Nt + 31) / 32, 256, 0, hs>>>(w.dlog, Ntp, B, Nt, nullptr, gr->dhead_b);
   AGCN_LAUNCH_CHECK();
-  if ((rc = head_weight_grad(w.mol, B, Fm, w.dlog, Nt, w.dWh_pad, w.tn_part, gr->dhead_W, side))) return rc;
+  if ((rc = head_weight_grad(w.mol, B, Fm, w.dlog, Nt, w.dWh_pad, w.tn_part, gr->dhead_W, hs))) return rc;
 
-  // main stream: dmol = dlog head_W^T, through tanh, ddense_b, dhsum, dH
+  // main stream: dmol = dlog head_W^T, then dpre and dH in head_bwd_kernel (w.dmol := dpre)
   if ((rc = gemm_auto(g_dmol, w.tcC, st, /*presplit=*/true))) return rc;
   {
-    const int64_t total = (int64_t)B * Fm;
-    tanh_bwd_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(w.pre, w.dmol, total);  // dmol := dpre
+    const int chunks = tc_dmol ? tc_gemm_ksplit(g_dmol) : 1;
+    const size_t smem = (size_t)HEAD_GRAPHS * (Fm + Fh) * sizeof(float);
+    if (smem > 32 * 1024)
+      AGCN_CUDA(cudaFuncSetAttribute(head_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ProfScope prof("head_bwd_kernel", st);
+    head_bwd_kernel<<<(unsigned)((B + HEAD_GRAPHS - 1) / HEAD_GRAPHS), 256, smem, st>>>(
+        chunks > 1 ? w.splitk : w.dmol, (int64_t)B * Fm, chunks, w.pre, d_dense_W, plan->d_node_off, B, Fh, Fm, w.dmol,
+        tc_dhs ? nullptr : gr->dH);
+  }
+  AGCN_LAUNCH_CHECK();
+  if (tc_dhs) {
+    if ((rc = tc_gemm(g_dhs, w.tcD, st))) return rc;
+    segment_broadcast_kernel<<<(B + 7) / 8, 256, 0, st>>>(w.dhsum, plan->d_node_off, B, Fh, gr->dH);
     AGCN_LAUNCH_CHECK();
   }
-  if ((rc = tc_dhs ? tc_gemm(g_dhs, w.tcD, st) : gemm_rows(g_dhs, st))) return rc;
-  segment_broadcast_kernel<<<(B + 7) / 8, 256, 0, st>>>(w.dhsum, plan->d_node_off, B, Fh, gr->dH);
-  AGCN_LAUNCH_CHECK();
-  // dense parameter gradients (need dpre; the dhead_W contraction on the side stream is done with tn_part by now
-  // only if we wait for it, so they follow it on the side stream)
-  AGCN_CUDA(cudaEventRecord(plan->ev_fork, st));
-  AGCN_CUDA(cudaStreamWaitEvent(side, plan->ev_fork, 0));
-  weighted_colsum_kernel<<<(Fm + 31) / 32, 256, 0, side>>>(w.dmol, Fm, B, Fm, plan->d_n, gr->ddense_b);
+  // dense parameter gradients from dpre, behind dhead_W on plan->head (they share tn_part)
+  AGCN_CUDA(cudaEventRecord(plan->ev_head_fork, st));
+  AGCN_CUDA(cudaStreamWaitEvent(hs, plan->ev_head_fork, 0));
+  weighted_colsum_kernel<<<(Fm + 31) / 32, 256, 0, hs>>>(w.dmol, Fm, B, Fm, plan->d_n, gr->ddense_b);
   AGCN_LAUNCH_CHECK();
   {
     GemmTNArgs t;  // ddense_W = hsum^T dpre
@@ -392,10 +490,10 @@ int head_run(const char* who, const agcn_plan* plan, const float* d_H, const flo
     t.A0 = w.hsum; t.lda0 = Fh;
     t.D = w.dmol; t.ldd = Fm;
     t.out = gr->ddense_W; t.partial = w.tn_part;
-    if ((rc = gemm_tn_auto(t, side))) return rc;
+    if ((rc = gemm_tn_auto(t, hs))) return rc;
   }
-  AGCN_CUDA(cudaEventRecord(plan->ev_side_join, side));
-  AGCN_CUDA(cudaStreamWaitEvent(st, plan->ev_side_join, 0));
+  AGCN_CUDA(cudaEventRecord(plan->ev_head_join, hs));
+  if (join_head) AGCN_CUDA(cudaStreamWaitEvent(st, plan->ev_head_join, 0));
   return AGCN_OK;
 }
 
@@ -524,6 +622,20 @@ int node_head_run(const char* who, const agcn_plan* plan, const float* d_H, cons
 }
 
 }  // namespace
+
+int head_loss_grad(const agcn_plan* plan, const float* d_H, const float* d_dense_W, const float* d_dense_b,
+                   const float* d_head_W, const float* d_head_b, const float* d_targets, const float* d_weights,
+                   float scale, int32_t loss_kind, int32_t Fh, int32_t Fm, int32_t Nt, float* d_loss, float* d_dH,
+                   float* d_ddense_W, float* d_ddense_b, float* d_dhead_W, float* d_dhead_b, void* d_work,
+                   size_t work_bytes, bool join_head, cudaStream_t st) {
+  AGCN_REQUIRE(plan && d_H && d_dense_W && d_dense_b && d_head_W && d_head_b && d_targets && d_weights && d_loss &&
+                   d_dH && d_ddense_W && d_ddense_b && d_dhead_W && d_dhead_b && d_work,
+               "head_loss_grad: null pointer");
+  const HeadGrads gr{d_dH, d_ddense_W, d_ddense_b, d_dhead_W, d_dhead_b};
+  return head_run("head_loss_grad", plan, d_H, d_dense_W, d_dense_b, d_head_W, d_head_b, d_targets, d_weights, scale,
+                  loss_kind, Fh, Fm, Nt, nullptr, d_loss, &gr, d_work, work_bytes, join_head, st);
+}
+
 }  // namespace agcn
 
 using namespace agcn;
@@ -564,12 +676,9 @@ int agcn_head_loss_grad_ex(const agcn_plan* plan, const float* d_H, const float*
                            float scale, int32_t loss_kind, int32_t Fh, int32_t Fm, int32_t Nt, float* d_loss,
                            float* d_dH, float* d_ddense_W, float* d_ddense_b, float* d_dhead_W, float* d_dhead_b,
                            void* d_work, size_t work_bytes, void* stream) {
-  AGCN_REQUIRE(plan && d_H && d_dense_W && d_dense_b && d_head_W && d_head_b && d_targets && d_weights && d_loss &&
-                   d_dH && d_ddense_W && d_ddense_b && d_dhead_W && d_dhead_b && d_work,
-               "head_loss_grad: null pointer");
-  const HeadGrads gr{d_dH, d_ddense_W, d_ddense_b, d_dhead_W, d_dhead_b};
-  return head_run("head_loss_grad", plan, d_H, d_dense_W, d_dense_b, d_head_W, d_head_b, d_targets, d_weights, scale,
-                  loss_kind, Fh, Fm, Nt, nullptr, d_loss, &gr, d_work, work_bytes, (cudaStream_t)stream);
+  return head_loss_grad(plan, d_H, d_dense_W, d_dense_b, d_head_W, d_head_b, d_targets, d_weights, scale, loss_kind, Fh,
+                        Fm, Nt, d_loss, d_dH, d_ddense_W, d_ddense_b, d_dhead_W, d_dhead_b, d_work, work_bytes,
+                        /*join_head=*/true, (cudaStream_t)stream);
 }
 
 int agcn_head_predict_workspace_bytes(const agcn_plan* plan, int32_t Fh, int32_t Fm, int32_t Nt, size_t* bytes) {
@@ -587,7 +696,7 @@ int agcn_head_predict(const agcn_plan* plan, const float* d_H, const float* d_de
   AGCN_REQUIRE(plan && d_H && d_dense_W && d_dense_b && d_head_W && d_head_b && d_probs && d_work,
                "head_predict: null pointer");
   return head_run("head_predict", plan, d_H, d_dense_W, d_dense_b, d_head_W, d_head_b, d_targets, d_weights, scale,
-                  loss_kind, Fh, Fm, Nt, d_probs, d_loss, nullptr, d_work, work_bytes, (cudaStream_t)stream);
+                  loss_kind, Fh, Fm, Nt, d_probs, d_loss, nullptr, d_work, work_bytes, true, (cudaStream_t)stream);
 }
 
 int agcn_node_head_workspace_bytes(const agcn_plan* plan, int32_t Fh, int32_t C, size_t* bytes) {

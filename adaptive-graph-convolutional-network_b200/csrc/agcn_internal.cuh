@@ -148,6 +148,10 @@ struct agcn_plan {
   // runs beside the fused launch of the small-graph tiles
   cudaStream_t big = nullptr;
   cudaEvent_t ev_big_fork = nullptr, ev_big_join = nullptr;
+  // the graph head's parameter-gradient chain (agcn_head.cu): nothing else runs on it, so the stack can leave that chain
+  // running beside the layer backward passes and join it once at the end
+  cudaStream_t head = nullptr;
+  cudaEvent_t ev_head_fork = nullptr, ev_head_join = nullptr;
   // life cycle (agcn_plan.cu): streams / events / staging come from process-wide pools, the device block is
   // stream-ordered; ev_ready marks the upload of the tables on create_stream
   cudaEvent_t ev_ready = nullptr;
@@ -200,8 +204,13 @@ struct GemmArgs {
   // tensor-core kernel only: scratch of 8 * M * N floats; when given, long contractions with few output tiles are
   // split along K (plain outputs only: no bias / activation / accumulate / loss epilogue, ldc == N, Z == 1)
   float* split_k_partial = nullptr;
+  // with split_k_partial: leave the tc_gemm_ksplit(a) raw partial sums there for the caller to add (chunk k at
+  // split_k_partial + k * M * ldc, added in the order k = 0, 1, ... as tc_gemm's own reduction does); C is not written
+  // unless tc_gemm_ksplit(a) == 1
+  int split_k_raw = 0;
 };
 int tc_gemm_loss_parts(const GemmArgs& a);  // number of partial loss sums tc_gemm writes
+int tc_gemm_ksplit(const GemmArgs& a);      // number of split-K chunks tc_gemm runs (1: C is written directly)
 int gemm_rows(const GemmArgs& a, cudaStream_t st);
 // tcgen05 (3xTF32) implementation of the same contraction for TMA-compatible shapes (agcn_tc_gemm.cu)
 bool tc_gemm_supported(const GemmArgs& a);
@@ -392,6 +401,14 @@ struct Arena {
   template <typename T = float>
   T* take(size_t count) { return static_cast<T*>(area(count * sizeof(T))); }
 };
+
+// agcn_head_loss_grad_ex (agcn_head.cu).  join_head = false leaves the parameter-gradient chain on plan->head unjoined:
+// `st` must wait for plan->ev_head_join before anything reads those gradients, and before a capture of `st` ends.
+int head_loss_grad(const agcn_plan* plan, const float* d_H, const float* d_dense_W, const float* d_dense_b,
+                   const float* d_head_W, const float* d_head_b, const float* d_targets, const float* d_weights,
+                   float scale, int32_t loss_kind, int32_t Fh, int32_t Fm, int32_t Nt, float* d_loss, float* d_dH,
+                   float* d_ddense_W, float* d_ddense_b, float* d_dhead_W, float* d_dhead_b, void* d_work,
+                   size_t work_bytes, bool join_head, cudaStream_t st);
 
 int zero_async(float* dst, size_t floats, cudaStream_t st);  // zero fill by a kernel (never the copy engine)
 int plan_use(const agcn_plan* plan, cudaStream_t st);  // call first in every entry point that enqueues work

@@ -314,9 +314,10 @@ int zero_async(float* dst, size_t floats, cudaStream_t st) {
 // (reused only after the copy that read them has completed) and the device block is stream-ordered
 // (cudaMallocAsync / cudaFreeAsync).
 struct PlanRes {
-  cudaStream_t aux[3] = {nullptr, nullptr, nullptr}, side = nullptr, big = nullptr;
+  cudaStream_t aux[3] = {nullptr, nullptr, nullptr}, side = nullptr, big = nullptr, head = nullptr;
   cudaEvent_t ev_fork = nullptr, ev_join[3] = {nullptr, nullptr, nullptr}, ev_side_fork = nullptr, ev_side_join = nullptr,
-              ev_big_fork = nullptr, ev_big_join = nullptr, ev_ready = nullptr;
+              ev_big_fork = nullptr, ev_big_join = nullptr, ev_head_fork = nullptr, ev_head_join = nullptr,
+              ev_ready = nullptr;
   int device = -1;
 };
 struct Staging {
@@ -361,6 +362,9 @@ static cudaError_t acquire_res(PlanRes* out) {
   }
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&r.ev_big_fork, cudaEventDisableTiming);
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&r.ev_big_join, cudaEventDisableTiming);
+  if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&r.head, cudaStreamNonBlocking);
+  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&r.ev_head_fork, cudaEventDisableTiming);
+  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&r.ev_head_join, cudaEventDisableTiming);
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&r.ev_ready, cudaEventDisableTiming);
   *out = r;
   return e;
@@ -548,6 +552,7 @@ int agcn_plan_create(const int32_t* n_nodes_host, int32_t B, int32_t Nmax, void*
   for (int i = 0; i < 3; ++i) { p->aux[i] = res.aux[i]; p->ev_join[i] = res.ev_join[i]; }
   p->ev_fork = res.ev_fork; p->side = res.side; p->ev_side_fork = res.ev_side_fork; p->ev_side_join = res.ev_side_join;
   p->big = res.big; p->ev_big_fork = res.ev_big_fork; p->ev_big_join = res.ev_big_join; p->ev_ready = res.ev_ready;
+  p->head = res.head; p->ev_head_fork = res.ev_head_fork; p->ev_head_join = res.ev_head_join;
   p->res_device = res.device;
   p->staging_host = stg.host; p->staging_bytes = stg.bytes; p->staging_done = stg.done;
   p->create_stream = st;
@@ -608,6 +613,7 @@ int agcn_plan_destroy(agcn_plan* p) {
     for (int i = 0; i < 3; ++i) { r.aux[i] = p->aux[i]; r.ev_join[i] = p->ev_join[i]; }
     r.ev_fork = p->ev_fork; r.side = p->side; r.ev_side_fork = p->ev_side_fork; r.ev_side_join = p->ev_side_join;
     r.big = p->big; r.ev_big_fork = p->ev_big_fork; r.ev_big_join = p->ev_big_join; r.ev_ready = p->ev_ready;
+    r.head = p->head; r.ev_head_fork = p->ev_head_fork; r.ev_head_join = p->ev_head_join;
     r.device = p->res_device;
     release_res(r);
   }

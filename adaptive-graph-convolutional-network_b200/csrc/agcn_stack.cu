@@ -389,15 +389,18 @@ int agcn_stack_loss_grad(const agcn_stack* s, const agcn_plan* plan, const float
   // ---- DenseMol + GraphGatherMol + logits + loss, with every gradient of that part
   // (or the per-node head: logits + loss of every node)
   const agcn_sgcll_desc& last = s->nodes[nl - 1].desc;
+  // The graph head's parameter gradients run on plan->head.  Without notify they stay there beside the layer backward
+  // passes and are joined at the end; a notify caller gets them joined first, since it starts their all-reduce now.
+  const bool defer_head = !node_head(s) && !notify;
   if (node_head(s))
     rc = agcn_node_head_loss_grad(plan, w.H[nl - 1], d_params + ho[2], d_params + ho[3], d_targets, d_weights, scale,
                                   last.Fo, s->Nt, d_loss, w.dA, d_grads + ho[2], d_grads + ho[3], w.head_work,
                                   w.head_work_bytes, stream);
   else
-    rc = agcn_head_loss_grad_ex(plan, w.H[nl - 1], d_params + ho[0], d_params + ho[1], d_params + ho[2],
-                                d_params + ho[3], d_targets, d_weights, scale, s->loss_kind, last.Fo, s->Fm, s->Nt,
-                                d_loss, w.dA, d_grads + ho[0], d_grads + ho[1], d_grads + ho[2], d_grads + ho[3],
-                                w.head_work, w.head_work_bytes, stream);
+    rc = head_loss_grad(plan, w.H[nl - 1], d_params + ho[0], d_params + ho[1], d_params + ho[2], d_params + ho[3],
+                        d_targets, d_weights, scale, s->loss_kind, last.Fo, s->Fm, s->Nt, d_loss, w.dA,
+                        d_grads + ho[0], d_grads + ho[1], d_grads + ho[2], d_grads + ho[3], w.head_work,
+                        w.head_work_bytes, /*join_head=*/!defer_head, st);
   if (rc) return rc;
   if (notify) notify(notify_user, nl, stream);
   // ---- backward, last node first; the first layer's input has no gradient unless the metric is differentiable.
@@ -446,6 +449,7 @@ int agcn_stack_loss_grad(const agcn_stack* s, const agcn_plan* plan, const float
     }
     dcur = dprev;
   }
+  if (defer_head) AGCN_CUDA(cudaStreamWaitEvent(st, plan->ev_head_join, 0));
   return AGCN_OK;
 }
 

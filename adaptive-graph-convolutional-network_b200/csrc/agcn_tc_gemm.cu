@@ -684,6 +684,27 @@ int tc_gemm_loss_parts(const GemmArgs& a) {
   return 4 * ((a.M + tc::BM - 1) / tc::BM) * a.Z * (Npad / BN);
 }
 
+// split-K for long contractions with few output tiles (plain outputs only): chunk ks of the contraction writes its raw
+// partial sums to split_k_partial + ks * M * ldc, and reduce_chunks_kernel adds them in the order ks = 0, 1, ...
+static void tc_gemm_split(const GemmArgs& a, int* ksplit, int* kb_per_split) {
+  using namespace tc;
+  const int Npad = tc_npad(a.N), BN = (Npad <= 64 || tc_gemm_narrow2(a)) ? 64 : 128;
+  const int total_kb = a.S * ((a.Kd + BK - 1) / BK);
+  const int out_tiles = ((a.M + BM - 1) / BM) * a.Z * (Npad / BN);
+  int k = 1;
+  if (a.split_k_partial && !a.bias && !a.scale && a.act == AGCN_ACT_LINEAR && !a.accumulate && !a.bce_y && !a.prob &&
+      a.ldc == a.N && a.Z == 1 && total_kb >= 16 && out_tiles < 74)
+    k = std::min(std::min(8, total_kb / 4), std::max(1, 148 / out_tiles));
+  *kb_per_split = (total_kb + k - 1) / k;
+  *ksplit = (total_kb + *kb_per_split - 1) / *kb_per_split;
+}
+
+int tc_gemm_ksplit(const GemmArgs& a) {
+  int ksplit, per;
+  tc_gemm_split(a, &ksplit, &per);
+  return ksplit;
+}
+
 size_t tc_gemm_scratch_floats(int N, int Kd, int S, int Z) { return 2 * (size_t)Z * S * tc_npad(N) * tc_kpitch(Kd); }
 
 // Rearranges the parameter operand B to [slice][Npad][Kd] (K-major) and splits it into hi / lo TF32 halves.
@@ -753,17 +774,8 @@ int tc_gemm(const GemmArgs& a, const float* scratch, cudaStream_t st) {
   Args p;
   p.M = a.M; p.N = a.N; p.Kd = a.Kd; p.S = a.S;
   p.kb_per_slice = (a.Kd + BK - 1) / BK;
-  const int total_kb = a.S * p.kb_per_slice;
-  // split-K for long contractions with few output tiles (plain outputs only): partial sums + one reduction
-  const int out_tiles = ((a.M + BM - 1) / BM) * a.Z * (Npad / BN);
-  int ksplit = 1;
-  if (a.split_k_partial && !a.bias && !a.scale && a.act == AGCN_ACT_LINEAR && !a.accumulate && !a.bce_y && !a.prob &&
-      a.ldc == a.N && a.Z == 1 && total_kb >= 16 && out_tiles < 74)
-    ksplit = std::min(std::min(8, total_kb / 4), std::max(1, 148 / out_tiles));
-  p.ksplit = ksplit;
-  p.kb_per_split = (total_kb + ksplit - 1) / ksplit;
-  p.ksplit = (total_kb + p.kb_per_split - 1) / p.kb_per_split;
-  ksplit = p.ksplit;
+  tc_gemm_split(a, &p.ksplit, &p.kb_per_split);
+  const int ksplit = p.ksplit;
   p.rows_slice1 = rows_slice1;
   p.b_rows_slice = Npad;
   p.C = a.C; p.ldc = a.ldc; p.sliceC = a.sliceC;
@@ -784,7 +796,7 @@ int tc_gemm(const GemmArgs& a, const float* scratch, cudaStream_t st) {
   else
     launch_tc_gemm<false, false>(narrow2, BN, grid, mA0, mA1, mBhi, mBlo, p, st);
   AGCN_LAUNCH_CHECK();
-  if (ksplit > 1) {
+  if (ksplit > 1 && !a.split_k_raw) {
     const long long elems = (long long)a.M * a.ldc;
     reduce_chunks_kernel<<<(unsigned)((elems + 255) / 256), 256, 0, st>>>(a.split_k_partial, a.C, elems, ksplit);
     AGCN_LAUNCH_CHECK();
